@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W              (this repo's CUDA path)
     python bench.py --impl reference --gpus N --steps K ...    (reference CPU path)
+    python bench.py ... --dump-outputs DIR      (also save the last timed step's outputs)
 
 One *step* = one pass of the hot path over one batch: `mgd_encode_targets` on B
 images' ground-truth boxes (B x 3 grids of y_true written) followed by
@@ -79,7 +80,15 @@ def parse():
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"],
                     help="strong: --strong-batch images in total, split over the ranks, gather on the clock")
     ap.add_argument("--strong-batch", type=int, default=4096)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed step returned in its last call to DIR/<name>.npy "
+                         "(rank 0's outputs only when several ranks run)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl b200)")
+    return args
 
 
 def measured_peak():
@@ -334,6 +343,43 @@ def _time_gpu(fn, steps, warmup, barrier):
     return e0.elapsed_time(e1)
 
 
+DUMP_BYTES = 63 * 10 ** 6         # array bytes: under 64 MB on disk, .npy headers included
+DUMP_Y_IMAGES = 16
+
+
+def dump_outputs(out_dir, det, y_true):
+    """--dump-outputs: the detection tensors and y_true of the timed step's last call, as
+    float32 / float64 .npy files of at most DUMP_BYTES in all, so that two builds can be
+    compared output for output.  y_true is DUMP_Y_IMAGES images drawn with a fixed seed (a
+    batch is gigabytes); the detections are every image's, or a seeded sample of images when
+    they do not fit.  `<part>_images.npy` holds the batch indices each part was taken from."""
+    import numpy as np
+    import torch
+    rng = np.random.default_rng(0)
+
+    def pick(n, k):
+        return np.sort(rng.choice(n, k, replace=False)) if k < n else np.arange(n)
+
+    n_y = int(y_true[0].shape[0])
+    y_img = pick(n_y, min(n_y, DUMP_Y_IMAGES))
+    sel = torch.from_numpy(y_img).to(y_true[0].device)
+    arrays = {f"y_true_{int(y.shape[1])}": y.index_select(0, sel).cpu().numpy() for y in y_true}
+    arrays["y_true_images"] = y_img.astype(np.float64)
+    left = DUMP_BYTES - sum(a.nbytes for a in arrays.values())
+    # integer outputs go out as float64, which holds every int32 exactly
+    keys = ("boxes_xyxy", "scores", "classes", "counts")
+    n_det = int(det["counts"].shape[0])
+    per_image = 8 + sum(det[k][0].numel() * 8 for k in keys)
+    d_img = pick(n_det, min(n_det, left // per_image))
+    sel = torch.from_numpy(d_img).to(det["counts"].device)
+    for k in keys:
+        arrays[k] = det[k].index_select(0, sel).cpu().numpy().astype(np.float64)
+    arrays["detections_images"] = d_img.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_b200(args):
     import numpy as np
     import torch
@@ -437,6 +483,10 @@ def run_b200(args):
         barrier()
         prof = engine.profile_end()
     engine.poll_status(local)
+    n_step_images = (hi_s - lo_s) if strong else B
+    if args.dump_outputs and rank == 0:
+        # before the measurements below overwrite y_out
+        dump_outputs(args.dump_outputs, out, [y[:n_step_images] for y in y_out])
     ms = ev0.elapsed_time(ev1)
     ms_max = max_over_ranks(ms)
     total_images = (Bs if strong else B * world) * args.steps
@@ -489,7 +539,6 @@ def run_b200(args):
     # ---- rooflines (per-launch CUDA events on the launching stream) ----------------------------
     peak, peak_src = measured_peak()
     kernels = {}
-    n_step_images = (hi_s - lo_s) if strong else B
     for kind, nbytes in (("encode_fill", BYTES_ENCODE), ("decode_compact", BYTES_DECODE)):
         tot_ms, launches = prof[kind]
         if launches:

@@ -8,6 +8,10 @@ exist, the CUDA path (``tests/test_gpu_golden.py``).  NumPy runs with its AVX
 dispatch disabled (``ref_loader.pin_numpy_env``) so ``argsort`` ties and the float32
 transcendentals are the portable libm ones.
 
+``tests/golden/live_*.npz`` are not written here: they hold digests of the reference's outputs
+on the inputs of the live-reference tests and are rewritten by those tests
+(``golden_util.Recorded``, ``MGD_RECORD_REFERENCE_OUTPUTS=1``).
+
 Fixtures are kept small: y_true is stored sparsely (positive cells only), head
 outputs are quantised to float16-representable values so they store in half the
 space while every consumer sees the identical float32 tensor.
