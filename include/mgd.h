@@ -286,6 +286,75 @@ MGD_API int mgd_match_detections(const double *det_boxes, const double *det_scor
                          int memory, int device, void *stream, int flags);
 
 /*
+ * Streaming mAP on the device.  Replaces the rest of calculate_map (multigriddet/evaluation/
+ * metrics.py:541-815) after the matcher: the per-(class, threshold) precision / recall /
+ * AP arithmetic (compute_precision_recall :221-246, compute_average_precision :249-300) and
+ * the re-matches of the area-filtered per-scale APs (:745-800), fed batch by batch with the
+ * padded tensors mgd_decode_nms emits, without building the reference's lists of dicts.
+ *
+ * A "view" is one matcher run over all updates: MGD_MAP_VIEW_CORNER and MGD_MAP_VIEW_CENTRE
+ * match every detection with the cached (corner IoU) or un-cached (centre-format IoU) matcher
+ * of mgd_match_detections; MGD_MAP_VIEW_S / _M / _L match with the centre matcher only the
+ * detections and ground truth whose (x2-x1)*(y2-y1) lies in [-inf, 1024), [1024, 9216) or
+ * [9216, inf) -- the per-scale sub-calls of calculate_map.  `views` in the config is the set
+ * of views to match (bit 1 << view); the others stay empty.
+ *
+ *   mgd_map_record_bytes  bytes of device memory per padded detection slot of `records`
+ *   mgd_map_update        matches one batch and writes one record per padded slot at
+ *                         records + slot_offset * mgd_map_record_bytes(); slot_offset is the
+ *                         sum of batch * max_dets over the earlier updates, so a record's
+ *                         position is the detection's global index (image-major, slot order).
+ *                         Adds the ground-truth counts of every view to gt_hist
+ *                         (MGD_MAP_VIEWS, num_classes) int64, which the caller zeroes once.
+ *                         det_boxes (batch, max_dets, 4) f64 xyxy, det_scores (batch,
+ *                         max_dets) f64 -- FINITE values, det_classes (batch, max_dets) int32,
+ *                         det_counts (batch,) int32; gt_boxes (batch, max_gt, 4) f64,
+ *                         gt_classes (batch, max_gt) int32, gt_counts (batch,) int32.  A class id
+ *                         outside [0, num_classes) is reported as MGD_ERR_CLASS_RANGE through
+ *                         mgd_poll_status (MGD_FLAG_SYNC synchronises and reports it).
+ *   mgd_map_compute       sorts the first num_slots records (class ascending, score descending,
+ *                         equal scores: later detection first) and computes, per view and
+ *                         class, the AP at every threshold:
+ *                           ap_out          (MGD_MAP_VIEWS, C, T) f64, MGD_MAP_COCO: all-point
+ *                                           interpolation + trapezoid
+ *                           voc_points_out  (MGD_MAP_VIEWS, C, T, 11) f64, MGD_MAP_VOC: the max
+ *                                           precision at recall >= voc_recalls[k] (0 if none);
+ *                                           the AP is their mean
+ *                           det_hist_out    (MGD_MAP_VIEWS, C) int64 detections per view and class
+ *                         The trapezoid takes the recalls in the order np.argsort gives them
+ *                         with NumPy's generic (non-SIMD) introsort, which permutes runs of
+ *                         equal recall, as in the reference's own numbers.
+ *                         The entry left NULL is the one the method does not use.  A class
+ *                         without detections or without ground truth gets 0 here: the
+ *                         reference's rules for those cases are the caller's (they need the
+ *                         two histograms only).  Scratch comes from the calling thread's
+ *                         workspace (mgd_release_workspace).
+ * Device memory only; work is enqueued on `stream`.
+ */
+#define MGD_MAP_MAX_THRESHOLDS 32
+#define MGD_MAP_VOC_POINTS 11
+enum { MGD_MAP_COCO = 0, MGD_MAP_VOC = 1 };
+enum { MGD_MAP_VIEW_CORNER = 0, MGD_MAP_VIEW_CENTRE = 1, MGD_MAP_VIEW_S = 2, MGD_MAP_VIEW_M = 3,
+       MGD_MAP_VIEW_L = 4, MGD_MAP_VIEWS = 5 };
+typedef struct {
+    int num_classes;                  /* C >= 1                                            */
+    int num_thresholds;               /* T in [1, MGD_MAP_MAX_THRESHOLDS]                  */
+    int method;                       /* MGD_MAP_COCO or MGD_MAP_VOC                       */
+    int views;                        /* bit mask of the views to match, non-empty         */
+    double iou_thresholds[MGD_MAP_MAX_THRESHOLDS];
+    double voc_recalls[MGD_MAP_VOC_POINTS];   /* np.arange(0, 1.1, 0.1) as the host has it  */
+} mgd_map_config;
+MGD_API int mgd_map_record_bytes(void);
+MGD_API int mgd_map_update(const mgd_map_config *cfg, const double *det_boxes,
+                   const double *det_scores, const int *det_classes, const int *det_counts,
+                   int batch, int max_dets, const double *gt_boxes, const int *gt_classes,
+                   const int *gt_counts, int max_gt, long long slot_offset, void *records,
+                   long long *gt_hist, int device, void *stream, int flags);
+MGD_API int mgd_map_compute(const mgd_map_config *cfg, const void *records, long long num_slots,
+                    const long long *gt_hist, double *ap_out, double *voc_points_out,
+                    long long *det_hist_out, int device, void *stream, int flags);
+
+/*
  * Loss-side ignore mask.  Replaces MultiGridLoss._compute_ignore_mask and
  * _compute_iou_batch (multigriddet/losses/multigrid_loss.py:494-703, 445-492), called once
  * per layer from the loss (:316).  Forward only: the reference casts the mask from a

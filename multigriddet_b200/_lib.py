@@ -24,6 +24,10 @@ NMS_IOU, NMS_DIOU, NMS_SOFT, NMS_WBF = 0, 1, 2, 3
 IOU_CORNER, IOU_CENTRE = 0, 1
 BOXES_I32, BOXES_F64 = 0, 1
 
+MAP_MAX_THRESHOLDS, MAP_VOC_POINTS = 32, 11
+MAP_COCO, MAP_VOC = 0, 1
+MAP_VIEW_CORNER, MAP_VIEW_CENTRE, MAP_VIEW_S, MAP_VIEW_M, MAP_VIEW_L, MAP_VIEWS = range(6)
+
 OK, ERR_INVALID_ARGUMENT, ERR_CLASS_RANGE, ERR_CUDA, ERR_NO_DEVICE, ERR_UNSUPPORTED = range(6)
 
 
@@ -57,6 +61,18 @@ class PostConfig(ctypes.Structure):
     ]
 
 
+class MapConfig(ctypes.Structure):
+    """``mgd_map_config``"""
+    _fields_ = [
+        ("num_classes", ctypes.c_int),
+        ("num_thresholds", ctypes.c_int),
+        ("method", ctypes.c_int),
+        ("views", ctypes.c_int),
+        ("iou_thresholds", ctypes.c_double * MAP_MAX_THRESHOLDS),
+        ("voc_recalls", ctypes.c_double * MAP_VOC_POINTS),
+    ]
+
+
 class MgdError(RuntimeError):
     pass
 
@@ -75,7 +91,8 @@ EXPORTS = ("mgd_version", "mgd_last_error", "mgd_device_count", "mgd_encode_targ
            "mgd_host_free", "mgd_release_workspace", "mgd_reshape_boxes", "mgd_mosaic_merge_boxes",
            "mgd_ignore_mask", "mgd_encode_decode_nms", "mgd_letterbox_boxes",
            "mgd_encode_ignore_mask", "mgd_exchange_create", "mgd_exchange_connect",
-           "mgd_exchange_buffer", "mgd_exchange_timeouts", "mgd_exchange_destroy")
+           "mgd_exchange_buffer", "mgd_exchange_timeouts", "mgd_exchange_destroy",
+           "mgd_map_record_bytes", "mgd_map_update", "mgd_map_compute")
 
 IPC_HANDLE_BYTES = 64
 
@@ -197,6 +214,17 @@ def load():
     lib.mgd_exchange_timeouts.argtypes = [ctypes.c_void_p, ctypes.c_void_p, _IP]
     lib.mgd_exchange_destroy.restype = ctypes.c_int
     lib.mgd_exchange_destroy.argtypes = [ctypes.c_void_p]
+    lib.mgd_map_record_bytes.restype = ctypes.c_int
+    lib.mgd_map_record_bytes.argtypes = []
+    lib.mgd_map_update.restype = ctypes.c_int
+    lib.mgd_map_update.argtypes = [
+        ctypes.POINTER(MapConfig), ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
+        ctypes.c_int, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int,
+        ctypes.c_longlong, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_int]
+    lib.mgd_map_compute.restype = ctypes.c_int
+    lib.mgd_map_compute.argtypes = [
+        ctypes.POINTER(MapConfig), ctypes.c_void_p, ctypes.c_longlong, ctypes.c_void_p, ctypes.c_void_p,
+        ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_int]
     lib.mgd_profile_begin.restype = ctypes.c_int
     lib.mgd_profile_end.restype = ctypes.c_int
     lib.mgd_profile_end.argtypes = [_DP, _LLP]

@@ -14,7 +14,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libmgd.so")
-SOURCES = ("api.cu", "encode.cu", "decode.cu", "nms.cu", "match.cu", "boxes.cu", "loss.cu", "exchange.cu")
+SOURCES = ("api.cu", "encode.cu", "decode.cu", "nms.cu", "match.cu", "boxes.cu", "loss.cu", "exchange.cu", "map.cu")
 HEADERS = ("common.cuh", "decode_math.cuh", "libm_emul.h", "dlpack_abi.h", os.path.join("..", "..", "include", "mgd.h"))
 
 # -fmad=false: integer results (anchor, cell, keep set) depend on IEEE operations in

@@ -400,6 +400,7 @@ int status_to_error(int st)
     if (st & 2)
         return fail(MGD_ERR_INVALID_ARGUMENT,
                     "negative class id on a valid box (the reference would write a wrong channel)");
+    if (st & 4) return fail(MGD_ERR_CLASS_RANGE, "mAP update: class id outside [0, num_classes)");
     return MGD_OK;
 }
 
@@ -751,6 +752,10 @@ struct HostStreams {
     cudaEvent_t ev[2] = {nullptr, nullptr};
     Arena chunk[2];          // staging + scratch of the chunk in flight on s[i]
     Arena call;              // per-call tensors (boxes, output slab, status words)
+    // scratch of the mAP entry points (device-memory calls on the caller's stream): the next
+    // call, on whatever stream, first waits for map_done, recorded behind the previous one
+    Arena map;
+    cudaEvent_t map_done = nullptr;
     // page-locked bounce buffers for PAGEABLE caller memory: the driver's own pageable
     // path is one memcpy thread (~11 GB/s); several threads filling a page-locked chunk
     // while the previous chunk is on the link reach ~3x that
@@ -763,9 +768,10 @@ struct HostStreams {
     ~HostStreams()
     {
         if (!s[0] && !s[1] && chunk[0].blocks.empty() && chunk[1].blocks.empty() &&
-            call.blocks.empty() && !bounce[0] && !bounce[1]) return;
+            call.blocks.empty() && map.blocks.empty() && !map_done && !bounce[0] && !bounce[1]) return;
         for (int i = 0; i < 2; ++i) if (s[i]) cudaStreamSynchronize(s[i]);
-        chunk[0].release(); chunk[1].release(); call.release();
+        if (map_done) { cudaEventSynchronize(map_done); cudaEventDestroy(map_done); }
+        chunk[0].release(); chunk[1].release(); call.release(); map.release();
         for (int i = 0; i < 2; ++i) {
             if (bounce[i]) cudaFreeHost(bounce[i]);
             if (bounce_done[i]) cudaEventDestroy(bounce_done[i]);
@@ -1039,10 +1045,11 @@ int mgd_release_workspace(void)
     for (int d = 0; d < 64; ++d) {
         HostStreams& hs = t_streams[d];
         if (hs.chunk[0].blocks.empty() && hs.chunk[1].blocks.empty() && hs.call.blocks.empty() &&
-            !hs.bounce[0] && !hs.bounce[1]) continue;
+            hs.map.blocks.empty() && !hs.bounce[0] && !hs.bounce[1]) continue;
         if (cudaSetDevice(d) != cudaSuccess) { cudaGetLastError(); continue; }
         for (int i = 0; i < 2; ++i) if (hs.s[i]) cudaStreamSynchronize(hs.s[i]);
-        hs.chunk[0].release(); hs.chunk[1].release(); hs.call.release();
+        if (hs.map_done) cudaEventSynchronize(hs.map_done);
+        hs.chunk[0].release(); hs.chunk[1].release(); hs.call.release(); hs.map.release();
         for (int i = 0; i < 2; ++i) {
             if (hs.bounce[i]) cudaFreeHost(hs.bounce[i]);
             hs.bounce[i] = nullptr; hs.bounce_cap[i] = 0; hs.bounce_busy[i] = false;
@@ -1887,6 +1894,145 @@ int mgd_match_detections(const double* det_boxes, const double* det_scores, cons
     }
     CUDA_TRY(cudaFreeAsync(buf, st));
     if (!host && (flags & MGD_FLAG_SYNC)) CUDA_TRY(cudaStreamSynchronize(st));
+    return MGD_OK;
+}
+
+namespace {
+
+int check_map_config(const mgd_map_config* cfg)
+{
+    if (!cfg) return fail(MGD_ERR_INVALID_ARGUMENT, "cfg is NULL");
+    if (cfg->num_classes < 1)
+        return fail(MGD_ERR_INVALID_ARGUMENT, "num_classes must be >= 1, got %d", cfg->num_classes);
+    if (cfg->num_thresholds < 1 || cfg->num_thresholds > MGD_MAP_MAX_THRESHOLDS)
+        return fail(MGD_ERR_INVALID_ARGUMENT, "num_thresholds must be in [1, %d], got %d",
+                    MGD_MAP_MAX_THRESHOLDS, cfg->num_thresholds);
+    if (cfg->method != MGD_MAP_COCO && cfg->method != MGD_MAP_VOC)
+        return fail(MGD_ERR_INVALID_ARGUMENT, "method must be MGD_MAP_COCO or MGD_MAP_VOC, got %d", cfg->method);
+    if (cfg->views < 1 || cfg->views >= (1 << MGD_MAP_VIEWS))
+        return fail(MGD_ERR_INVALID_ARGUMENT, "views must be a non-empty mask of MGD_MAP_VIEW_* bits");
+    return MGD_OK;
+}
+
+// the calling thread's mAP scratch on `device`, ordered behind its previous use
+int map_workspace(int device, cudaStream_t st, Arena** out)
+{
+    HostStreams& hs = t_streams[device];
+    if (!hs.map_done) CUDA_TRY(cudaEventCreateWithFlags(&hs.map_done, cudaEventDisableTiming));
+    CUDA_TRY(cudaStreamWaitEvent(st, hs.map_done, 0));
+    hs.map.reset();
+    *out = &hs.map;
+    return MGD_OK;
+}
+
+int map_workspace_done(int device, cudaStream_t st)
+{
+    CUDA_TRY(cudaEventRecord(t_streams[device].map_done, st));
+    return MGD_OK;
+}
+
+}  // namespace
+
+int mgd_map_record_bytes(void)
+{
+    return (int)sizeof(MapRec);
+}
+
+int mgd_map_update(const mgd_map_config* cfg, const double* det_boxes, const double* det_scores,
+                   const int* det_classes, const int* det_counts, int batch, int max_dets,
+                   const double* gt_boxes, const int* gt_classes, const int* gt_counts, int max_gt,
+                   long long slot_offset, void* records, long long* gt_hist, int device, void* stream,
+                   int flags)
+{
+    nvtx_range nv_api("mgd_map_update");
+    int rc;
+    if ((rc = check_map_config(cfg))) return rc;
+    if (batch < 0 || max_dets < 0 || max_gt < 0 || slot_offset < 0)
+        return fail(MGD_ERR_INVALID_ARGUMENT, "batch, max_dets, max_gt and slot_offset must be >= 0");
+    if (slot_offset + (long long)batch * max_dets > 0x7fffffffll)
+        return fail(MGD_ERR_UNSUPPORTED, "more than 2^31 - 1 detection slots in one evaluation");
+    if (max_dets > 65535) return fail(MGD_ERR_UNSUPPORTED, "max_dets per image must be <= 65535");
+    if ((size_t)max_dets * 2 + (size_t)max_gt / 8 > 48 * 1024)
+        return fail(MGD_ERR_UNSUPPORTED, "max_dets / max_gt too large for one warp's shared memory");
+    if (batch > 0 && (!det_counts || !gt_counts || !gt_hist))
+        return fail(MGD_ERR_INVALID_ARGUMENT, "NULL tensor");
+    if ((long long)batch * max_dets > 0 && (!det_boxes || !det_scores || !det_classes || !records))
+        return fail(MGD_ERR_INVALID_ARGUMENT, "NULL detection tensor");
+    if ((long long)batch * max_gt > 0 && (!gt_boxes || !gt_classes))
+        return fail(MGD_ERR_INVALID_ARGUMENT, "NULL ground-truth tensor");
+    int num_sms;
+    DeviceScope dev_scope;
+    if ((rc = prepare_device(device, &num_sms, &dev_scope))) return rc;
+    if (batch == 0) return MGD_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    int* d_status;
+    if ((rc = deferred_status_word(device, &d_status))) return rc;
+    Arena* ws;
+    if ((rc = map_workspace(device, st, &ws))) return rc;
+    const size_t flags_bytes = (size_t)cfg->num_thresholds * batch * max_dets;
+    int* counters;
+    CUDA_TRY(ws->take(reinterpret_cast<void**>(&counters), MGD_MAP_VIEWS * sizeof(int)));
+    CUDA_TRY(cudaMemsetAsync(counters, 0, MGD_MAP_VIEWS * sizeof(int), st));
+    MapWriteArgs w;
+    memset(&w, 0, sizeof(w));
+    // one match_kernel walk per view: corner / centre IoU over everything, centre IoU per band
+    for (int v = 0; v < MGD_MAP_VIEWS; ++v) {
+        if (!((cfg->views >> v) & 1)) continue;
+        MatchArgs a;
+        memset(&a, 0, sizeof(a));
+        a.B = batch; a.M = max_dets; a.N = max_gt; a.T = cfg->num_thresholds;
+        for (int t = 0; t < a.T; ++t) a.thr[t] = cfg->iou_thresholds[t];
+        a.mode = v == MGD_MAP_VIEW_CORNER ? MGD_IOU_CORNER : MGD_IOU_CENTRE;
+        a.band = v >= MGD_MAP_VIEW_S ? 1 + v - MGD_MAP_VIEW_S : 0;
+        a.det_boxes = det_boxes; a.det_scores = det_scores; a.det_classes = det_classes;
+        a.det_counts = det_counts; a.gt_boxes = gt_boxes; a.gt_classes = gt_classes;
+        a.gt_counts = gt_counts;
+        unsigned char* tp;
+        CUDA_TRY(ws->take(reinterpret_cast<void**>(&tp), flags_bytes));
+        a.tp = tp;
+        a.next_image = counters + v;
+        if (flags_bytes) CUDA_TRY(launch_match(a, num_sms, st));
+        w.tp[v] = tp;
+    }
+    w.B = batch; w.M = max_dets; w.N = max_gt; w.T = cfg->num_thresholds; w.C = cfg->num_classes;
+    w.views = cfg->views;
+    w.det_boxes = det_boxes; w.det_scores = det_scores; w.det_classes = det_classes;
+    w.det_counts = det_counts; w.gt_boxes = gt_boxes; w.gt_classes = gt_classes; w.gt_counts = gt_counts;
+    w.recs = static_cast<MapRec*>(records) + slot_offset;
+    w.gt_hist = reinterpret_cast<unsigned long long*>(gt_hist);
+    w.status = d_status;
+    CUDA_TRY(launch_map_write(w, st));
+    if ((rc = map_workspace_done(device, st))) return rc;
+    if (flags & MGD_FLAG_SYNC) return mgd_poll_status(device, stream);
+    return MGD_OK;
+}
+
+int mgd_map_compute(const mgd_map_config* cfg, const void* records, long long num_slots,
+                    const long long* gt_hist, double* ap_out, double* voc_points_out,
+                    long long* det_hist_out, int device, void* stream, int flags)
+{
+    nvtx_range nv_api("mgd_map_compute");
+    int rc;
+    if ((rc = check_map_config(cfg))) return rc;
+    if (num_slots < 0 || num_slots > 0x7fffffffll)
+        return fail(MGD_ERR_INVALID_ARGUMENT, "num_slots must be in [0, 2^31 - 1]");
+    if ((num_slots > 0 && !records) || !gt_hist || !det_hist_out)
+        return fail(MGD_ERR_INVALID_ARGUMENT, "NULL tensor");
+    if (cfg->method == MGD_MAP_COCO ? !ap_out : !voc_points_out)
+        return fail(MGD_ERR_INVALID_ARGUMENT, "NULL output of the configured method");
+    int num_sms;
+    DeviceScope dev_scope;
+    if ((rc = prepare_device(device, &num_sms, &dev_scope))) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    Arena* ws;
+    if ((rc = map_workspace(device, st, &ws))) return rc;
+    void* scratch;
+    CUDA_TRY(ws->take(&scratch, map_compute_scratch_bytes(num_slots, cfg->num_thresholds)));
+    CUDA_TRY(launch_map_compute(*cfg, static_cast<const MapRec*>(records), num_slots,
+                                reinterpret_cast<const unsigned long long*>(gt_hist), ap_out, voc_points_out,
+                                reinterpret_cast<unsigned long long*>(det_hist_out), scratch, st));
+    if ((rc = map_workspace_done(device, st))) return rc;
+    if (flags & MGD_FLAG_SYNC) CUDA_TRY(cudaStreamSynchronize(st));
     return MGD_OK;
 }
 

@@ -138,13 +138,56 @@ struct MatchArgs {
     const double* gt_boxes;           // (B, N, 4)
     const int* gt_classes;            // (B, N)
     const int* gt_counts;             // (B,)
-    double thr[MGD_MAX_IOU_THRESHOLDS];
+    double thr[MGD_MAP_MAX_THRESHOLDS];   // T <= MGD_MAX_IOU_THRESHOLDS for mgd_match_detections
     int mode;                         // 0: corner IoU, candidate must beat 0 (cached matcher);
                                       // 1: centre-format IoU, first maximum (un-cached matcher)
+    int band;                         // 0: every box; 1 + b: only boxes in area band b
+                                      // (map_area_band): the others are left out of the walk
+                                      // like calculate_map's area filter (metrics.py:745-800)
     unsigned char* tp;                // (T, B, M)
     int* matched;                     // (T, B, M) or nullptr
     int* next_image;                  // work counter, zeroed by the caller
 };
+
+// Area band of an xyxy box for the per-scale APs: 0 = S (-inf, 1024), 1 = M [1024, 9216),
+// 2 = L [9216, inf), 3 = none (NaN area).  The area is (x2-x1)*(y2-y1) in float64
+// (metrics.py:_box_area) and the bounds are compared as _filter_by_area does.
+__device__ __forceinline__ int map_area_band(const double* b)
+{
+    const double area = __dmul_rn(__dsub_rn(b[2], b[0]), __dsub_rn(b[3], b[1]));
+    if (area < 1024.0) return 0;
+    if (area >= 1024.0 && area < 9216.0) return 1;
+    if (area >= 9216.0) return 2;
+    return 3;
+}
+
+// ---- streaming mAP (map.cu) ---------------------------------------------------------------
+// One record per padded detection slot, written by map_update and sorted by map_compute.
+struct __align__(8) MapRec {
+    double score;                     // as given (scores are finite)
+    int cls;                          // -1: padding slot (or a class id reported out of range)
+    int band;                         // map_area_band of the detection
+    unsigned bits[MGD_MAP_VIEWS];     // bit t: true positive at threshold t in that view
+    unsigned pad;
+};
+static_assert(sizeof(MapRec) == 40, "MapRec is the record format of mgd_map_record_bytes");
+
+struct MapWriteArgs {
+    int B, M, N, T, C, views;
+    const double* det_boxes; const double* det_scores; const int* det_classes; const int* det_counts;
+    const double* gt_boxes; const int* gt_classes; const int* gt_counts;
+    const unsigned char* tp[MGD_MAP_VIEWS];   // (T, B, M) flags of each matched view, else nullptr
+    MapRec* recs;                     // the update's first record
+    unsigned long long* gt_hist;      // (MGD_MAP_VIEWS, C)
+    int* status;                      // bit 2: class id outside [0, C)
+};
+cudaError_t launch_map_write(const MapWriteArgs& a, cudaStream_t stream);
+
+// scratch of map_compute (bytes), and the enqueue of sort + AP kernels
+size_t map_compute_scratch_bytes(long long n, int T);
+cudaError_t launch_map_compute(const mgd_map_config& cfg, const MapRec* recs, long long n,
+                               const unsigned long long* gt_hist, double* ap, double* voc,
+                               unsigned long long* det_hist, void* scratch, cudaStream_t stream);
 
 // ---- box-side pre-step of the encoder (reshape_boxes / merge_mosaic_bboxes) ---
 struct BoxOpArgs {

@@ -11,7 +11,9 @@
 // slot first, the order of a reversed stable argsort) and the 32 lanes scan the image's
 // ground-truth boxes.  Every IoU threshold is an independent walk over the same boxes.
 // float64 IoU in the reference's operation order (-fmad=false), so `iou >= threshold`
-// decides identically.
+// decides identically.  An optional area band (MatchArgs::band) restricts the walk to the
+// boxes calculate_map's per-scale filter keeps, which is the filtered lists' result: their
+// relative visiting order and ground-truth index order are those of the full lists.
 #include <math.h>
 #include "common.cuh"
 
@@ -47,6 +49,8 @@ __device__ __forceinline__ double iou_centre(const double* p, const double* g)
     return uni > 0.0 ? __ddiv_rn(inter, uni) : 0.0;
 }
 
+// kBand: a.band != 0 (a separate instantiation, so the plain matcher keeps its registers)
+template <bool kBand>
 __global__ void __launch_bounds__(kMatchWarps * 32)
 match_kernel(const __grid_constant__ MatchArgs a)
 {
@@ -85,12 +89,28 @@ match_kernel(const __grid_constant__ MatchArgs a)
 
         for (int t = 0; t < a.T; ++t) {
             const double thr = a.thr[t];
-            for (int w = lane; w < words; w += 32) taken[w] = 0u;
+            // ground truth outside the area band starts the walk as already claimed
+            for (int w = lane; w < words; w += 32) {
+                unsigned m = 0u;
+                if (kBand)
+                    for (int j = 32 * w; j < g && j < 32 * w + 32; ++j)
+                        if (map_area_band(gbox + 4 * j) != a.band - 1) m |= 1u << (j & 31);
+                taken[w] = m;
+            }
             __syncwarp();
             unsigned char* tp = a.tp + ((size_t)t * a.B + b) * a.M;
             int* who = a.matched ? a.matched + ((size_t)t * a.B + b) * a.M : nullptr;
             for (int k = 0; k < n; ++k) {
                 const int d = order[k];
+                // a detection outside the band is not in the filtered list: no claim, tp = 0;
+                // the visiting order of the others is unchanged
+                if (kBand && map_area_band(dbox + 4 * d) != a.band - 1) {
+                    if (lane == 0) {
+                        tp[d] = 0;
+                        if (who) who[d] = -1;
+                    }
+                    continue;
+                }
                 const int cls = dcl[d];
                 const double p[4] = {dbox[4 * d], dbox[4 * d + 1], dbox[4 * d + 2], dbox[4 * d + 3]};
                 double best = 0.0;
@@ -141,13 +161,14 @@ cudaError_t launch_match(const MatchArgs& a, int num_sms, cudaStream_t stream)
 {
     const size_t per_warp = ((size_t)a.M * 2 + (size_t)((a.N + 31) / 32) * 4 + 16 + 15) & ~(size_t)15;
     const size_t smem = per_warp * kMatchWarps;
-    cudaError_t e = cudaFuncSetAttribute(match_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    auto kernel = a.band ? match_kernel<true> : match_kernel<false>;
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     long long grid = ((long long)a.B + kMatchWarps - 1) / kMatchWarps;
     if (grid > (long long)num_sms * 8) grid = (long long)num_sms * 8;
     if (grid < 1) grid = 1;
     prof_mark_begin(PROF_OTHER, stream);
-    match_kernel<<<(unsigned)grid, kMatchWarps * 32, smem, stream>>>(a);
+    kernel<<<(unsigned)grid, kMatchWarps * 32, smem, stream>>>(a);
     prof_mark_end(PROF_OTHER, stream);
     return cudaGetLastError();
 }

@@ -488,6 +488,95 @@ def match_detections(det_boxes, det_scores, det_classes, det_counts, gt_boxes, g
     return (tp, who) if return_matched else tp
 
 
+_MAP_METHODS = {"coco": _lib.MAP_COCO, "voc": _lib.MAP_VOC}
+
+
+def map_config(num_classes, iou_thresholds, method="coco", views=(_lib.MAP_VIEW_CORNER,)) -> _lib.MapConfig:
+    """``mgd_map_config`` for ``map_update`` / ``map_compute``; raises ValueError on what the
+    library would refuse, before any device work."""
+    if method not in _MAP_METHODS:
+        raise ValueError(f"Unknown method: {method}")
+    thr = [float(t) for t in iou_thresholds]
+    if not 1 <= len(thr) <= _lib.MAP_MAX_THRESHOLDS:
+        raise ValueError(f"between 1 and {_lib.MAP_MAX_THRESHOLDS} IoU thresholds supported, got {len(thr)}")
+    if int(num_classes) < 1:
+        raise ValueError(f"num_classes must be >= 1, got {num_classes}")
+    if not views or any(not 0 <= v < _lib.MAP_VIEWS for v in views):
+        raise ValueError(f"views must be a non-empty subset of range({_lib.MAP_VIEWS})")
+    cfg = _lib.MapConfig()
+    cfg.num_classes = int(num_classes)
+    cfg.num_thresholds = len(thr)
+    cfg.method = _MAP_METHODS[method]
+    cfg.views = sum(1 << v for v in set(views))
+    for t, v in enumerate(thr):
+        cfg.iou_thresholds[t] = v
+    for k, x in enumerate(np.arange(0, 1.1, 0.1)):     # compute_average_precision's VOC recalls
+        cfg.voc_recalls[k] = float(x)
+    return cfg
+
+
+def map_record_bytes() -> int:
+    """Bytes of the record buffer per padded detection slot (``mgd_map_record_bytes``)."""
+    return int(_lib.load().mgd_map_record_bytes())
+
+
+def map_update(cfg, records, slot_offset, gt_hist, det_boxes, det_scores, det_classes, det_counts,
+               gt_boxes, gt_classes, gt_counts, sync=False):
+    """Match one batch and write its records at ``slot_offset`` of ``records`` (a CUDA byte
+    tensor), adding its ground-truth counts to ``gt_hist`` ((MAP_VIEWS, C) int64 CUDA tensor)
+    (``mgd_map_update``).  Torch CUDA tensors in ``match_detections``' layout; boxes may be
+    int32 (``decode_nms``' ``boxes_xyxy``).  Enqueued on the current stream; class-range errors
+    surface at the next ``poll_status`` unless ``sync``."""
+    import torch
+    lib = _lib.load()
+    dev = records.device
+    for name, t in (("det_boxes", det_boxes), ("det_scores", det_scores), ("det_classes", det_classes),
+                    ("det_counts", det_counts), ("gt_boxes", gt_boxes), ("gt_classes", gt_classes),
+                    ("gt_counts", gt_counts)):
+        if not (_is_torch(t) and t.device == dev):
+            raise ValueError(f"{name} must be a torch tensor on {dev}")
+    f64 = lambda x: x.to(torch.float64).contiguous()
+    i32 = lambda x: x.to(torch.int32).contiguous()
+    db, ds, dc, dn = f64(det_boxes), f64(det_scores), i32(det_classes), i32(det_counts)
+    gb, gc, gn = f64(gt_boxes), i32(gt_classes), i32(gt_counts)
+    if ds.dim() != 2 or tuple(db.shape) != (*ds.shape, 4) or dc.shape != ds.shape or tuple(dn.shape) != (ds.shape[0],):
+        raise ValueError("detections must be det_boxes (B, M, 4), det_scores / det_classes (B, M), det_counts (B,)")
+    B, M = int(ds.shape[0]), int(ds.shape[1])
+    if gc.dim() != 2 or gc.shape[0] != B or tuple(gb.shape) != (*gc.shape, 4) or tuple(gn.shape) != (B,):
+        raise ValueError("ground truth must be gt_boxes (B, N, 4), gt_classes (B, N), gt_counts (B,)")
+    N = int(gc.shape[1])
+    if records.dtype != torch.uint8 or records.numel() < (slot_offset + B * M) * map_record_bytes():
+        raise ValueError("records is not a uint8 tensor large enough for this update")
+    p = lambda x: ctypes.c_void_p(x.data_ptr()) if x.numel() else None
+    idx = dev.index or 0
+    rc = lib.mgd_map_update(ctypes.byref(cfg), p(db), p(ds), p(dc), p(dn), B, M, p(gb), p(gc), p(gn), N,
+                            int(slot_offset), p(records), p(gt_hist), idx,
+                            ctypes.c_void_p(_torch_stream(idx)), _lib.FLAG_SYNC if sync else 0)
+    _lib.raise_for_status(rc)
+
+
+def map_compute(cfg, records, num_slots, gt_hist):
+    """Sort the first ``num_slots`` records and compute every view's per-(class, threshold)
+    AP (``mgd_map_compute``).  Returns NumPy ``det_hist`` (MAP_VIEWS, C) int64 and ``ap``
+    (MAP_VIEWS, C, T) for 'coco' or ``voc`` (MAP_VIEWS, C, T, 11) for 'voc'; synchronises."""
+    import torch
+    lib = _lib.load()
+    dev = gt_hist.device
+    V, C, T = _lib.MAP_VIEWS, cfg.num_classes, cfg.num_thresholds
+    det_hist = torch.empty((V, C), dtype=torch.int64, device=dev)
+    coco = cfg.method == _lib.MAP_COCO
+    out = torch.empty((V, C, T) if coco else (V, C, T, _lib.MAP_VOC_POINTS), dtype=torch.float64, device=dev)
+    idx = dev.index or 0
+    rc = lib.mgd_map_compute(ctypes.byref(cfg),
+                             ctypes.c_void_p(records.data_ptr()) if records is not None and num_slots else None,
+                             int(num_slots), ctypes.c_void_p(gt_hist.data_ptr()),
+                             ctypes.c_void_p(out.data_ptr()) if coco else None,
+                             None if coco else ctypes.c_void_p(out.data_ptr()),
+                             ctypes.c_void_p(det_hist.data_ptr()), idx, ctypes.c_void_p(_torch_stream(idx)), 0)
+    _lib.raise_for_status(rc)
+    return {"det_hist": det_hist.cpu().numpy(), "ap" if coco else "voc": out.cpu().numpy()}
+
+
 def iou_matrix(boxes1, boxes2):
     """(n, m) float64 IoU matrix of xyxy boxes (``mgd_iou_matrix``), NumPy in / out."""
     lib = _lib.load()

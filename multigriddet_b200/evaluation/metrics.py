@@ -14,7 +14,7 @@ from typing import Any, Dict, List, Tuple
 
 import numpy as np
 
-from .. import engine
+from .. import _lib, engine
 
 COCO_THRESHOLDS = [0.5, 0.55, 0.6, 0.65, 0.7, 0.75, 0.8, 0.85, 0.9, 0.95]
 
@@ -153,13 +153,22 @@ def compute_average_precision(precisions: np.ndarray, recalls: np.ndarray, metho
     raise ValueError(f"Unknown method: {method}")
 
 
-def _class_ap(tp_row, pk: _Packed, class_id: int, method: str) -> float:
-    sel = pk.pred_classes == class_id
-    n_gt = int(np.sum(pk.gt_class_flat == class_id))
-    if not sel.any():
+def _special_ap(n_pred: int, n_gt: int):
+    """The AP of a class without predictions or without ground truth (metrics.py:303-385);
+    None when the class has both."""
+    if n_pred == 0:
         return 0.0 if n_gt > 0 else 1.0
     if n_gt == 0:
         return 0.0
+    return None
+
+
+def _class_ap(tp_row, pk: _Packed, class_id: int, method: str) -> float:
+    sel = pk.pred_classes == class_id
+    n_gt = int(np.sum(pk.gt_class_flat == class_id))
+    special = _special_ap(int(np.count_nonzero(sel)), n_gt)
+    if special is not None:
+        return special
     tp, fp, _ = _sorted_flags(tp_row[sel], pk.pred_scores[sel])
     return compute_average_precision(*compute_precision_recall(tp, fp, n_gt), method)
 
@@ -189,6 +198,76 @@ def _filter_by_area(predictions, ground_truths, min_area=None, max_area=None):
     return [p for p in predictions if keep(p)], [g for g in ground_truths if keep(g)]
 
 
+_SCALES = (("APS", None, 1024.0), ("APM", 1024.0, 9216.0), ("APL", 9216.0, None))
+
+
+class _DictSource:
+    """What ``_map_results`` reads, from the reference's lists of dicts."""
+
+    def __init__(self, predictions: List[Dict], ground_truths: List[Dict]):
+        self.predictions, self.ground_truths = predictions, ground_truths
+        self.num_predictions, self.num_ground_truths = len(predictions), len(ground_truths)
+
+    def classes(self):
+        return set(p["class"] for p in self.predictions) | set(g["class"] for g in self.ground_truths)
+
+    def scale(self, lo, hi) -> "_DictSource":
+        return _DictSource(*_filter_by_area(self.predictions, self.ground_truths, lo, hi))
+
+    def ap_table(self, iou_thresholds, matcher: str, method: str):
+        pk = _Packed(self.predictions, self.ground_truths)
+        tp = pk.flags(iou_thresholds, matcher) if iou_thresholds else None
+        return lambda class_id, t: _class_ap(tp[t], pk, class_id, method)
+
+
+def _map_results(src, num_classes, iou_thresholds, class_names, method, use_parallel, optimize_classes,
+                 cache_ious, compute_per_scale) -> Dict[str, Any]:
+    """calculate_map's result dict (metrics.py:541-815) from an AP source: the class set, the
+    matcher choice, the means over classes and thresholds and the per-scale rules.
+    ``src.ap_table(thresholds, matcher, method)(class_id, t)`` is the AP of one class at
+    threshold t; ``src.scale(lo, hi)`` is the source of the area-filtered sub-call."""
+    results = {"mAP": 0.0, "mAP50": 0.0, "mAP75": 0.0, "per_class": {}, "per_iou": {},
+               "num_predictions": src.num_predictions, "num_ground_truths": src.num_ground_truths}
+    if optimize_classes:
+        active = sorted(src.classes())
+    else:
+        active = list(range(num_classes))
+    if use_parallel and len(active) > 1 and cache_ious and src.num_predictions > 10000:
+        cache_ious = False
+    ap_of = src.ap_table(iou_thresholds, "corner" if cache_ious else "centre", method)
+    iou_aps = {thr: [] for thr in iou_thresholds}
+    class_aps = {}
+    for class_id in active:
+        name = class_names[class_id] if class_id < len(class_names) else f"class_{class_id}"
+        res = {}
+        for t, thr in enumerate(iou_thresholds):
+            ap = ap_of(class_id, t)
+            res[f"AP{thr:.2f}"] = ap
+            iou_aps[thr].append(ap)
+        res["AP"] = np.mean(list(res.values()))
+        class_aps[name] = res
+    results["per_class"] = class_aps
+    for thr in iou_thresholds:
+        if len(iou_aps[thr]) > 0:
+            results["per_iou"][f"mAP{thr:.2f}"] = np.mean(iou_aps[thr])
+    if 0.5 in iou_thresholds:
+        results["mAP50"] = results["per_iou"].get("mAP0.50", 0.0)
+    if 0.75 in iou_thresholds:
+        results["mAP75"] = results["per_iou"].get("mAP0.75", 0.0)
+    if len(iou_thresholds) > 0:
+        results["mAP"] = np.mean([results["per_iou"].get(f"mAP{thr:.2f}", 0.0) for thr in iou_thresholds])
+    for key, lo, hi in _SCALES:
+        results[key], results[key + "50"] = 0.0, 0.0
+        if compute_per_scale:
+            sub_src = src.scale(lo, hi)
+            if sub_src.num_ground_truths > 0:
+                sub = _map_results(sub_src, num_classes, iou_thresholds, class_names, method,
+                                   use_parallel=False, optimize_classes=optimize_classes,
+                                   cache_ious=False, compute_per_scale=False)
+                results[key], results[key + "50"] = sub["mAP"], sub.get("mAP50", 0.0)
+    return results
+
+
 def calculate_map(predictions: List[Dict], ground_truths: List[Dict], num_classes: int,
                   iou_thresholds: List[float] = None, class_names: List[str] = None,
                   method: str = "coco", use_parallel: bool = True, optimize_classes: bool = True,
@@ -205,44 +284,111 @@ def calculate_map(predictions: List[Dict], ground_truths: List[Dict], num_classe
         iou_thresholds = list(COCO_THRESHOLDS)
     if class_names is None:
         class_names = [f"class_{i}" for i in range(num_classes)]
-    results = {"mAP": 0.0, "mAP50": 0.0, "mAP75": 0.0, "per_class": {}, "per_iou": {},
-               "num_predictions": len(predictions), "num_ground_truths": len(ground_truths)}
-    if optimize_classes:
-        active = sorted(set(p["class"] for p in predictions) | set(g["class"] for g in ground_truths))
-    else:
-        active = list(range(num_classes))
-    if use_parallel and len(active) > 1 and cache_ious and len(predictions) > 10000:
-        cache_ious = False
-    pk = _Packed(predictions, ground_truths)
-    tp = pk.flags(iou_thresholds, "corner" if cache_ious else "centre") if iou_thresholds else None
-    iou_aps = {thr: [] for thr in iou_thresholds}
-    class_aps = {}
-    for class_id in active:
-        name = class_names[class_id] if class_id < len(class_names) else f"class_{class_id}"
-        res = {}
-        for t, thr in enumerate(iou_thresholds):
-            ap = _class_ap(tp[t], pk, class_id, method)
-            res[f"AP{thr:.2f}"] = ap
-            iou_aps[thr].append(ap)
-        res["AP"] = np.mean(list(res.values()))
-        class_aps[name] = res
-    results["per_class"] = class_aps
-    for thr in iou_thresholds:
-        if len(iou_aps[thr]) > 0:
-            results["per_iou"][f"mAP{thr:.2f}"] = np.mean(iou_aps[thr])
-    if 0.5 in iou_thresholds:
-        results["mAP50"] = results["per_iou"].get("mAP0.50", 0.0)
-    if 0.75 in iou_thresholds:
-        results["mAP75"] = results["per_iou"].get("mAP0.75", 0.0)
-    if len(iou_thresholds) > 0:
-        results["mAP"] = np.mean([results["per_iou"].get(f"mAP{thr:.2f}", 0.0) for thr in iou_thresholds])
-    for key, lo, hi in (("APS", None, 1024.0), ("APM", 1024.0, 9216.0), ("APL", 9216.0, None)):
-        results[key], results[key + "50"] = 0.0, 0.0
+    return _map_results(_DictSource(predictions, ground_truths), num_classes, iou_thresholds, class_names,
+                        method, use_parallel, optimize_classes, cache_ious, compute_per_scale)
+
+
+class _DeviceSource:
+    """What ``_map_results`` reads, from ``mgd_map_compute``'s per-view outputs.  ``view`` is
+    the view the detections and ground truth are counted in: one of the two full-set views,
+    or an area band's view (``band``), which is also the one its APs come from."""
+
+    _BANDS = {(None, 1024.0): _lib.MAP_VIEW_S, (1024.0, 9216.0): _lib.MAP_VIEW_M, (9216.0, None): _lib.MAP_VIEW_L}
+
+    def __init__(self, out, gt_hist, view: int, band: bool = False):
+        self.out, self.gt_hist, self.view, self.band = out, gt_hist, view, band
+        self._det, self._gt = out["det_hist"][view], gt_hist[view]
+        self.num_predictions, self.num_ground_truths = int(self._det.sum()), int(self._gt.sum())
+
+    def classes(self):
+        return set(np.flatnonzero((self._det > 0) | (self._gt > 0)).tolist())
+
+    def scale(self, lo, hi) -> "_DeviceSource":
+        return _DeviceSource(self.out, self.gt_hist, self._BANDS[(lo, hi)], band=True)
+
+    def ap_table(self, iou_thresholds, matcher: str, method: str):
+        v = self.view if self.band else (_lib.MAP_VIEW_CORNER if matcher == "corner" else _lib.MAP_VIEW_CENTRE)
+        det, gt = self.out["det_hist"][v], self.gt_hist[v]
+
+        def ap_of(class_id, t):
+            special = _special_ap(int(det[class_id]), int(gt[class_id]))
+            if special is not None:
+                return special
+            if method == "voc":
+                return np.mean(self.out["voc"][v, class_id, t])
+            ap = self.out["ap"][v, class_id, t]
+            # compute_average_precision: float(np.sum(...)), or interp[0] * r[0] for one record
+            return ap if det[class_id] == 1 else float(ap)
+        return ap_of
+
+
+class MapAccumulator:
+    """``calculate_map`` fed batch by batch with device tensors, without the lists of dicts.
+
+    ``update`` takes the padded per-image tensors ``match_detections`` takes (torch CUDA
+    tensors; ``det_boxes`` may be the int32 ``boxes_xyxy`` of ``engine.decode_nms``) and only
+    enqueues work on the current stream: it matches the batch with every matcher the
+    configuration can need and appends one record per padded detection slot
+    (``mgd_map_update``).  ``compute`` sorts the records and computes the APs on the device
+    (``mgd_map_compute``) and returns ``calculate_map``'s result dict for all updates so far,
+    the detections listed image by image in slot order.  The arguments are
+    ``calculate_map``'s.  Scores must be finite and class ids in [0, num_classes);
+    ``compute`` raises AssertionError for a class id outside that range.
+
+    The AP follows ``np.argsort`` of the recalls as NumPy's generic introsort orders equal
+    ones, which is how the reference's numbers were produced (NumPy without its SIMD sort
+    dispatch, the pin of ``oracle/ref_loader.py``).  Where NumPy dispatches its argsort to
+    AVX-512 or AVX2 it orders those ties differently, and ``calculate_map`` itself then gives
+    different numbers from one CPU to another.
+    """
+
+    def __init__(self, num_classes: int, iou_thresholds: List[float] = None, class_names: List[str] = None,
+                 method: str = "coco", use_parallel: bool = True, optimize_classes: bool = True,
+                 cache_ious: bool = True, compute_per_scale: bool = True, device=None):
+        if iou_thresholds is None:
+            iou_thresholds = list(COCO_THRESHOLDS)
+        if class_names is None:
+            class_names = [f"class_{i}" for i in range(num_classes)]
+        # the matcher of the full set is chosen at compute() (it depends on the prediction
+        # count): with cache_ious and use_parallel both are matched
+        views = [_lib.MAP_VIEW_CORNER] if cache_ious else [_lib.MAP_VIEW_CENTRE]
+        if cache_ious and use_parallel:
+            views.append(_lib.MAP_VIEW_CENTRE)
         if compute_per_scale:
-            sp, sg = _filter_by_area(predictions, ground_truths, lo, hi)
-            if len(sg) > 0:
-                sub = calculate_map(sp, sg, num_classes, iou_thresholds, class_names, method,
-                                    use_parallel=False, optimize_classes=optimize_classes,
-                                    cache_ious=False, compute_per_scale=False)
-                results[key], results[key + "50"] = sub["mAP"], sub.get("mAP50", 0.0)
-    return results
+            views += [_lib.MAP_VIEW_S, _lib.MAP_VIEW_M, _lib.MAP_VIEW_L]
+        self._cfg = engine.map_config(num_classes, iou_thresholds, method, views)
+        self._args = (int(num_classes), list(iou_thresholds), list(class_names), method, use_parallel,
+                      optimize_classes, cache_ious, compute_per_scale)
+        import torch
+        self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+        self._record_bytes = engine.map_record_bytes()
+        self.reset()
+
+    def reset(self) -> None:
+        """Forget every update."""
+        import torch
+        self._records = torch.empty((0,), dtype=torch.uint8, device=self.device)
+        self._slots = 0
+        self._gt_hist = torch.zeros((_lib.MAP_VIEWS, self._cfg.num_classes), dtype=torch.int64, device=self.device)
+
+    def update(self, det_boxes, det_scores, det_classes, det_counts, gt_boxes, gt_classes, gt_counts) -> None:
+        """Add one batch: det_boxes (B, M, 4) xyxy, det_scores (B, M), det_classes (B, M),
+        det_counts (B,), gt_boxes (B, N, 4) xyxy, gt_classes (B, N), gt_counts (B,)."""
+        import torch
+        slots = int(det_scores.shape[0]) * int(det_scores.shape[1])
+        need = (self._slots + slots) * self._record_bytes
+        if need > self._records.numel():              # grow by doubling, on the stream
+            grown = torch.empty((max(need, 2 * self._records.numel()),), dtype=torch.uint8, device=self.device)
+            used = self._slots * self._record_bytes
+            grown[:used].copy_(self._records[:used])
+            self._records = grown
+        engine.map_update(self._cfg, self._records, self._slots, self._gt_hist, det_boxes, det_scores,
+                          det_classes, det_counts, gt_boxes, gt_classes, gt_counts)
+        self._slots += slots
+
+    def compute(self) -> Dict[str, Any]:
+        """``calculate_map``'s result dict over every update since construction or ``reset``."""
+        out = engine.map_compute(self._cfg, self._records, self._slots, self._gt_hist)
+        engine.poll_status(self.device.index or 0)
+        full = _lib.MAP_VIEW_CORNER if self._args[6] else _lib.MAP_VIEW_CENTRE    # a view always matched
+        return _map_results(_DeviceSource(out, self._gt_hist.cpu().numpy(), full), *self._args)
