@@ -355,6 +355,44 @@ MGD_API int mgd_map_compute(const mgd_map_config *cfg, const void *records, long
                     long long *det_hist_out, int device, void *stream, int flags);
 
 /*
+ * Sharded streaming mAP.  Each of `world` ranks runs mgd_map_update on its own shard of every
+ * global batch; the APs of a class are then computed on the one rank that owns it.  The result
+ * equals mgd_map_compute over the whole data, which orders equal scores of a class later
+ * detection first in global image order, so every record carries its GLOBAL slot: for local
+ * slot j of update u on rank r it is G_u + lo_r * M_u + (j - L_u), where G_u is the sum of
+ * n_total * max_dets over the earlier updates, lo_r the rank's first image of the update
+ * (contiguous shards), M_u its max_dets and L_u the rank's slot_offset of the update.
+ *
+ *   mgd_map_partition       takes the first num_slots records of this rank and the update
+ *                           segments (num_segments, 2) int64 (L_u, G_u + lo_r * M_u) with L_u
+ *                           ascending (updates without local images may be left out); drops
+ *                           padding slots; stamps each record's global slot into the record;
+ *                           writes the records grouped by destination rank owner[class]
+ *                           (owner (C,) int32, values in [0, world)), each group in local order,
+ *                           to out_records (room for num_slots records), and the records per
+ *                           destination to out_counts (world,) int64.  global_slots is the
+ *                           sum of n_total * max_dets over all updates (<= 2^32, else
+ *                           MGD_ERR_UNSUPPORTED); world <= 256.  An owner entry outside
+ *                           [0, world) is reported as MGD_ERR_INVALID_ARGUMENT through
+ *                           mgd_poll_status.
+ *   mgd_map_compute_merged  mgd_map_compute over the records a rank received (any order):
+ *                           sorted by class ascending, score descending, global slot descending,
+ *                           with gt_hist the SUM of every rank's ground-truth counts.  Only the
+ *                           (view, class) pairs with owner[class] == rank get their AP and
+ *                           det_hist; the others get exact zeros, so the element-wise sum of the
+ *                           ranks' ap_out / voc_points_out / det_hist_out is mgd_map_compute's.
+ * Device memory only; work is enqueued on `stream`; scratch as for mgd_map_compute.
+ */
+MGD_API int mgd_map_partition(const mgd_map_config *cfg, const void *records, long long num_slots,
+                      const long long *segments, int num_segments, long long global_slots,
+                      const int *owner, int world, void *out_records, long long *out_counts,
+                      int device, void *stream, int flags);
+MGD_API int mgd_map_compute_merged(const mgd_map_config *cfg, const void *records,
+                      long long num_records, const long long *gt_hist, const int *owner, int rank,
+                      double *ap_out, double *voc_points_out, long long *det_hist_out,
+                      int device, void *stream, int flags);
+
+/*
  * Loss-side ignore mask.  Replaces MultiGridLoss._compute_ignore_mask and
  * _compute_iou_batch (multigriddet/losses/multigrid_loss.py:494-703, 445-492), called once
  * per layer from the loss (:316).  Forward only: the reference casts the mask from a

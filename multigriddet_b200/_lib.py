@@ -92,7 +92,8 @@ EXPORTS = ("mgd_version", "mgd_last_error", "mgd_device_count", "mgd_encode_targ
            "mgd_ignore_mask", "mgd_encode_decode_nms", "mgd_letterbox_boxes",
            "mgd_encode_ignore_mask", "mgd_exchange_create", "mgd_exchange_connect",
            "mgd_exchange_buffer", "mgd_exchange_timeouts", "mgd_exchange_destroy",
-           "mgd_map_record_bytes", "mgd_map_update", "mgd_map_compute")
+           "mgd_map_record_bytes", "mgd_map_update", "mgd_map_compute", "mgd_map_partition",
+           "mgd_map_compute_merged")
 
 IPC_HANDLE_BYTES = 64
 
@@ -225,6 +226,16 @@ def load():
     lib.mgd_map_compute.argtypes = [
         ctypes.POINTER(MapConfig), ctypes.c_void_p, ctypes.c_longlong, ctypes.c_void_p, ctypes.c_void_p,
         ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_int]
+    lib.mgd_map_partition.restype = ctypes.c_int
+    lib.mgd_map_partition.argtypes = [
+        ctypes.POINTER(MapConfig), ctypes.c_void_p, ctypes.c_longlong, ctypes.c_void_p, ctypes.c_int,
+        ctypes.c_longlong, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int,
+        ctypes.c_void_p, ctypes.c_int]
+    lib.mgd_map_compute_merged.restype = ctypes.c_int
+    lib.mgd_map_compute_merged.argtypes = [
+        ctypes.POINTER(MapConfig), ctypes.c_void_p, ctypes.c_longlong, ctypes.c_void_p, ctypes.c_void_p,
+        ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p,
+        ctypes.c_int]
     lib.mgd_profile_begin.restype = ctypes.c_int
     lib.mgd_profile_end.restype = ctypes.c_int
     lib.mgd_profile_end.argtypes = [_DP, _LLP]

@@ -401,6 +401,7 @@ int status_to_error(int st)
         return fail(MGD_ERR_INVALID_ARGUMENT,
                     "negative class id on a valid box (the reference would write a wrong channel)");
     if (st & 4) return fail(MGD_ERR_CLASS_RANGE, "mAP update: class id outside [0, num_classes)");
+    if (st & 8) return fail(MGD_ERR_INVALID_ARGUMENT, "mAP partition: owner table entry outside [0, world)");
     return MGD_OK;
 }
 
@@ -2031,6 +2032,76 @@ int mgd_map_compute(const mgd_map_config* cfg, const void* records, long long nu
     CUDA_TRY(launch_map_compute(*cfg, static_cast<const MapRec*>(records), num_slots,
                                 reinterpret_cast<const unsigned long long*>(gt_hist), ap_out, voc_points_out,
                                 reinterpret_cast<unsigned long long*>(det_hist_out), scratch, st));
+    if ((rc = map_workspace_done(device, st))) return rc;
+    if (flags & MGD_FLAG_SYNC) CUDA_TRY(cudaStreamSynchronize(st));
+    return MGD_OK;
+}
+
+int mgd_map_partition(const mgd_map_config* cfg, const void* records, long long num_slots,
+                      const long long* segments, int num_segments, long long global_slots, const int* owner,
+                      int world, void* out_records, long long* out_counts, int device, void* stream, int flags)
+{
+    nvtx_range nv_api("mgd_map_partition");
+    int rc;
+    if ((rc = check_map_config(cfg))) return rc;
+    if (num_slots < 0 || num_slots > 0x7fffffffll)
+        return fail(MGD_ERR_INVALID_ARGUMENT, "num_slots must be in [0, 2^31 - 1]");
+    if (num_segments < 0 || (num_slots > 0 && num_segments < 1))
+        return fail(MGD_ERR_INVALID_ARGUMENT, "num_segments must be >= 1 when there are records");
+    if (global_slots < num_slots)
+        return fail(MGD_ERR_INVALID_ARGUMENT, "global_slots must be >= num_slots");
+    if (global_slots > (1ll << 32))
+        return fail(MGD_ERR_UNSUPPORTED, "more than 2^32 global detection slots in one evaluation");
+    if (world < 1) return fail(MGD_ERR_INVALID_ARGUMENT, "world must be >= 1, got %d", world);
+    if (world > 256) return fail(MGD_ERR_UNSUPPORTED, "world must be <= 256, got %d", world);
+    if (!owner || !out_counts) return fail(MGD_ERR_INVALID_ARGUMENT, "NULL tensor");
+    if (num_slots > 0 && (!records || !segments || !out_records))
+        return fail(MGD_ERR_INVALID_ARGUMENT, "NULL tensor");
+    int num_sms;
+    DeviceScope dev_scope;
+    if ((rc = prepare_device(device, &num_sms, &dev_scope))) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    MapPartitionArgs a;
+    a.recs = static_cast<const MapRec*>(records); a.n = num_slots; a.C = cfg->num_classes;
+    a.segs = segments; a.num_segs = num_segments; a.owner = owner; a.world = world;
+    a.out = static_cast<MapRec*>(out_records); a.counts = out_counts;
+    if ((rc = deferred_status_word(device, &a.status))) return rc;
+    Arena* ws;
+    if ((rc = map_workspace(device, st, &ws))) return rc;
+    void* scratch;
+    CUDA_TRY(ws->take(&scratch, map_partition_scratch_bytes(num_slots)));
+    CUDA_TRY(launch_map_partition(a, scratch, st));
+    if ((rc = map_workspace_done(device, st))) return rc;
+    if (flags & MGD_FLAG_SYNC) return mgd_poll_status(device, stream);
+    return MGD_OK;
+}
+
+int mgd_map_compute_merged(const mgd_map_config* cfg, const void* records, long long num_records,
+                           const long long* gt_hist, const int* owner, int rank, double* ap_out,
+                           double* voc_points_out, long long* det_hist_out, int device, void* stream, int flags)
+{
+    nvtx_range nv_api("mgd_map_compute_merged");
+    int rc;
+    if ((rc = check_map_config(cfg))) return rc;
+    if (num_records < 0 || num_records > 0x7fffffffll)
+        return fail(MGD_ERR_INVALID_ARGUMENT, "num_records must be in [0, 2^31 - 1]");
+    if ((num_records > 0 && !records) || !gt_hist || !owner || !det_hist_out)
+        return fail(MGD_ERR_INVALID_ARGUMENT, "NULL tensor");
+    if (cfg->method == MGD_MAP_COCO ? !ap_out : !voc_points_out)
+        return fail(MGD_ERR_INVALID_ARGUMENT, "NULL output of the configured method");
+    if (rank < 0) return fail(MGD_ERR_INVALID_ARGUMENT, "rank must be >= 0, got %d", rank);
+    int num_sms;
+    DeviceScope dev_scope;
+    if ((rc = prepare_device(device, &num_sms, &dev_scope))) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    Arena* ws;
+    if ((rc = map_workspace(device, st, &ws))) return rc;
+    void* scratch;
+    CUDA_TRY(ws->take(&scratch, map_compute_scratch_bytes(num_records, cfg->num_thresholds)));
+    CUDA_TRY(launch_map_compute_merged(*cfg, static_cast<const MapRec*>(records), num_records,
+                                       reinterpret_cast<const unsigned long long*>(gt_hist), owner, rank,
+                                       ap_out, voc_points_out, reinterpret_cast<unsigned long long*>(det_hist_out),
+                                       scratch, st));
     if ((rc = map_workspace_done(device, st))) return rc;
     if (flags & MGD_FLAG_SYNC) CUDA_TRY(cudaStreamSynchronize(st));
     return MGD_OK;

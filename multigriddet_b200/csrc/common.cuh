@@ -188,6 +188,28 @@ size_t map_compute_scratch_bytes(long long n, int T);
 cudaError_t launch_map_compute(const mgd_map_config& cfg, const MapRec* recs, long long n,
                                const unsigned long long* gt_hist, double* ap, double* voc,
                                unsigned long long* det_hist, void* scratch, cudaStream_t stream);
+// the same over records stamped by map_partition (ties broken by the global slot, descending);
+// only the classes `owner` gives to `rank` get APs, the others exact zeros
+cudaError_t launch_map_compute_merged(const mgd_map_config& cfg, const MapRec* recs, long long n,
+                                      const unsigned long long* gt_hist, const int* owner, int rank,
+                                      double* ap, double* voc, unsigned long long* det_hist, void* scratch,
+                                      cudaStream_t stream);
+
+// mgd_map_partition: the records grouped by the rank that owns their class, in local order,
+// padding dropped, each stamped with its global slot (MapRec::pad)
+struct MapPartitionArgs {
+    const MapRec* recs; long long n;  // the rank's first n records
+    int C;
+    const long long* segs;            // (num_segs, 2): first local slot of an update, its global slot
+    int num_segs;
+    const int* owner;                 // (C,) rank that owns each class
+    int world;                        // <= 256 (one radix digit)
+    MapRec* out;                      // (n,) records, rank by rank
+    long long* counts;                // (world,) records per rank
+    int* status;                      // bit 3: owner entry outside [0, world)
+};
+size_t map_partition_scratch_bytes(long long n);
+cudaError_t launch_map_partition(const MapPartitionArgs& a, void* scratch, cudaStream_t stream);
 
 // ---- box-side pre-step of the encoder (reshape_boxes / merge_mosaic_bboxes) ---
 struct BoxOpArgs {

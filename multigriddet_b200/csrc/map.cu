@@ -18,6 +18,12 @@
 //                         cum_tp, p and r in float64 in the reference's operation order, suffix
 //                         max of p (np.maximum.accumulate(p[::-1])[::-1]) and the trapezoid, or
 //                         the 11 VOC maxima
+// Sharded (mgd_map_partition / mgd_map_compute_merged): the tile kernels of the sort, with the
+// owner rank of each record's class as the digit, group a rank's records by destination and
+// stamp each with its global slot; the merged sort takes four more digits from that slot
+// (descending, so equal scores stay later detection first in global image order), and
+// map_ap_kernel walks only the classes the rank owns.
+//
 // compute_average_precision sorts the recalls with np.argsort (metrics.py:285) before the
 // trapezoid.  They are non-decreasing already, but the sort is NumPy's unstable introsort
 // (without SIMD dispatch, the NumPy the reference's numbers were produced with), which permutes
@@ -33,11 +39,13 @@ namespace {
 constexpr int kThreads = 256;
 constexpr int kTileItems = 8 * kThreads;     // sort tile: 8 sub-tiles of one item per thread
 constexpr int kDigits = 12;                  // 8 score bytes, then 4 class bytes (LSD order)
+constexpr int kSlotDigits = 4;               // merged sort: 4 global-slot bytes below the score
+constexpr int kMaxDigits = kDigits + kSlotDigits;
 
 struct MapPlan {
-    int active[kDigits];                     // pass runs (its digit is not the same for all keys)
-    int first[kDigits];                      // first pass: reads the input backwards
-    int src[kDigits], dst[kDigits];          // index buffers
+    int active[kMaxDigits];                  // pass runs (its digit is not the same for all keys)
+    int first[kMaxDigits];                   // first pass: reads the input (backwards without slot digits)
+    int src[kMaxDigits], dst[kMaxDigits];    // index buffers
     int final_buf;
 };
 
@@ -54,8 +62,13 @@ __device__ __forceinline__ unsigned long long score_key(double s)
 // padding slots sort behind every class
 __device__ __forceinline__ unsigned class_key(int cls, int C) { return cls < 0 ? (unsigned)C : (unsigned)cls; }
 
+// digit p of a record's key; S = kSlotDigits in the merged sort, whose least significant digits
+// are the global slot stamped into MapRec::pad, descending (later detection first)
+template <int S>
 __device__ __forceinline__ unsigned rec_digit(const MapRec& r, int p, int C)
 {
+    if (p < S) return (~r.pad >> (8 * p)) & 255u;
+    p -= S;
     if (p < 8) return (unsigned)(score_key(r.score) >> (8 * p)) & 255u;
     return (class_key(r.cls, C) >> (8 * (p - 8))) & 255u;
 }
@@ -139,11 +152,13 @@ __global__ void __launch_bounds__(kThreads) map_write_kernel(const __grid_consta
 }
 
 // ---- radix sort ------------------------------------------------------------------------------
-// histograms of all 12 digits in one pass (warp-aggregated: most digits are one value)
+// histograms of all 12 + S digits in one pass (warp-aggregated: most digits are one value)
+template <int S>
 __global__ void __launch_bounds__(kThreads) map_hist_kernel(const MapRec* recs, unsigned n, int C, unsigned* hist)
 {
-    __shared__ unsigned h[kDigits * 256];
-    for (int k = threadIdx.x; k < kDigits * 256; k += blockDim.x) h[k] = 0u;
+    constexpr int nd = kDigits + S;
+    __shared__ unsigned h[nd * 256];
+    for (int k = threadIdx.x; k < nd * 256; k += blockDim.x) h[k] = 0u;
     __syncthreads();
     const unsigned lane_lt = (1u << (threadIdx.x & 31)) - 1u;
     const unsigned stride = gridDim.x * blockDim.x;
@@ -151,24 +166,26 @@ __global__ void __launch_bounds__(kThreads) map_hist_kernel(const MapRec* recs, 
         const unsigned i = base + threadIdx.x;
         const bool valid = i < n;
         MapRec r;
-        if (valid) { r.score = recs[i].score; r.cls = recs[i].cls; }
-        for (int p = 0; p < kDigits; ++p) {
-            const unsigned d = valid ? rec_digit(r, p, C) : 256u;
+        if (valid) { r.score = recs[i].score; r.cls = recs[i].cls; if (S) r.pad = recs[i].pad; }
+        for (int p = 0; p < nd; ++p) {
+            const unsigned d = valid ? rec_digit<S>(r, p, C) : 256u;
             const unsigned peers = __match_any_sync(0xffffffffu, d);
             if (valid && (peers & lane_lt) == 0u) atomicAdd(&h[p * 256 + d], (unsigned)__popc(peers));
         }
     }
     __syncthreads();
-    for (int k = threadIdx.x; k < kDigits * 256; k += blockDim.x)
+    for (int k = threadIdx.x; k < nd * 256; k += blockDim.x)
         if (h[k]) atomicAdd(hist + k, h[k]);
 }
 
 // which passes run, and their buffers
+template <int S>
 __global__ void map_plan_kernel(const unsigned* hist, unsigned n, MapPlan* plan)
 {
-    __shared__ int active[kDigits];
+    constexpr int nd = kDigits + S;
+    __shared__ int active[nd];
     const int p = threadIdx.x;
-    if (p < kDigits) {
+    if (p < nd) {
         int a = 1;
         for (int d = 0; d < 256; ++d) if (hist[p * 256 + d] == n) a = 0;
         active[p] = a;
@@ -176,10 +193,10 @@ __global__ void map_plan_kernel(const unsigned* hist, unsigned n, MapPlan* plan)
     __syncthreads();
     if (threadIdx.x != 0) return;
     int any = 0;
-    for (int q = 0; q < kDigits; ++q) any |= active[q];
-    if (!any) active[kDigits - 1] = 1;      // all keys equal: one pass still reverses the input
+    for (int q = 0; q < nd; ++q) any |= active[q];
+    if (!any) active[nd - 1] = 1;           // all keys equal: one pass still reverses the input
     int cur = -1;
-    for (int q = 0; q < kDigits; ++q) {
+    for (int q = 0; q < nd; ++q) {
         plan->active[q] = active[q];
         plan->first[q] = active[q] && cur < 0;
         plan->src[q] = cur < 0 ? 0 : cur;
@@ -189,36 +206,94 @@ __global__ void map_plan_kernel(const unsigned* hist, unsigned n, MapPlan* plan)
     plan->final_buf = cur;
 }
 
+// the first pass reads the records backwards so that equal keys end up later index first; with
+// the global slot in the key (S > 0) no two keys are equal and it reads them in order
+template <int S>
 __device__ __forceinline__ unsigned pass_input(const MapPlan& pl, int p, const unsigned* bufs, unsigned n, unsigned i)
 {
-    return pl.first[p] ? n - 1u - i : bufs[(size_t)pl.src[p] * n + i];
+    return pl.first[p] ? (S ? i : n - 1u - i) : bufs[(size_t)pl.src[p] * n + i];
 }
 
+// The tile machinery below (per-tile digit counts, tile offsets, stable scatter) is shared by
+// the sort passes and by the rank partition of mgd_map_partition.  A Pass says whether it runs,
+// which item sits at input position i, the item's digit (256: the item is dropped) and where the
+// item goes once its output position is known.
+
+// one pass of the sort: items are record indices, the output is the pass's index buffer
+template <int S>
+struct SortPass {
+    const MapPlan* plan; int p; const MapRec* recs; unsigned n; int C; unsigned* bufs;
+    __device__ bool active() const { return plan->active[p]; }
+    __device__ unsigned item(unsigned i) const { return pass_input<S>(*plan, p, bufs, n, i); }
+    __device__ unsigned digit(unsigned it) const { return rec_digit<S>(recs[it], p, C); }
+    __device__ void put(unsigned pos, unsigned it) const { bufs[(size_t)plan->dst[p] * n + pos] = it; }
+};
+
+// the rank partition: items are record indices, the digit is the rank that owns the record's
+// class (padding slots are dropped), the output is the record with its global slot stamped in
+struct PartitionPass {
+    const MapRec* recs; int C; const int* owner; int world;
+    const long long* segs; int num_segs;          // (num_segs, 2): first local slot, its global slot
+    MapRec* out; int* status;
+    __device__ bool active() const { return true; }
+    __device__ unsigned item(unsigned i) const { return i; }
+    __device__ unsigned digit(unsigned it) const
+    {
+        const int c = recs[it].cls;
+        if (c < 0 || c >= C) return 256u;
+        const int o = owner[c];
+        if (o < 0 || o >= world) { atomicOr(status, 8); return 256u; }
+        return (unsigned)o;
+    }
+    __device__ void put(unsigned pos, unsigned it) const
+    {
+        int lo = 0, hi = num_segs - 1;                    // the last segment starting at or before it
+        while (lo < hi) {
+            const int mid = (lo + hi + 1) >> 1;
+            if (segs[2 * mid] <= (long long)it) lo = mid; else hi = mid - 1;
+        }
+        MapRec r = recs[it];
+        r.pad = (unsigned)(segs[2 * lo + 1] + ((long long)it - segs[2 * lo]));
+        out[pos] = r;
+    }
+};
+
 // digit counts per tile: tile_counts[tile][digit]
-__global__ void __launch_bounds__(kThreads) map_tile_count_kernel(const MapPlan* plan, int p, const MapRec* recs,
-                                                                   unsigned n, int C, const unsigned* bufs,
-                                                                   unsigned* tile_counts)
+template <class Pass>
+__global__ void __launch_bounds__(kThreads) map_tile_count_kernel(const Pass pass, unsigned n, unsigned* tile_counts)
 {
     __shared__ unsigned cnt[256];
-    if (!plan->active[p]) return;
+    if (!pass.active()) return;
     cnt[threadIdx.x] = 0u;
     __syncthreads();
-    const MapPlan& pl = *plan;
     for (int s = 0; s < kTileItems / kThreads; ++s) {
         const unsigned i = blockIdx.x * (unsigned)kTileItems + s * kThreads + threadIdx.x;
-        if (i < n) atomicAdd(&cnt[rec_digit(recs[pass_input(pl, p, bufs, n, i)], p, C)], 1u);
+        if (i < n) {
+            const unsigned d = pass.digit(pass.item(i));
+            if (d < 256u) atomicAdd(&cnt[d], 1u);
+        }
     }
     __syncthreads();
     tile_counts[(size_t)blockIdx.x * 256 + threadIdx.x] = cnt[threadIdx.x];
 }
 
-// tile counts -> first output position of each (tile, digit), in place
-__global__ void __launch_bounds__(kThreads) map_tile_offsets_kernel(const MapPlan* plan, int p, const unsigned* hist,
-                                                                     unsigned tiles, unsigned* tile_counts)
+// tile counts -> first output position of each (tile, digit), in place.  digit_totals: the
+// pass's histogram, or nullptr to sum it from the tile counts and store its first num_totals
+// entries to totals_out
+template <class Pass>
+__global__ void __launch_bounds__(kThreads) map_tile_offsets_kernel(const Pass pass, const unsigned* digit_totals,
+                                                                     unsigned tiles, unsigned* tile_counts,
+                                                                     long long* totals_out, int num_totals)
 {
-    if (!plan->active[p]) return;
+    if (!pass.active()) return;
     const unsigned d = threadIdx.x;
-    const unsigned h = hist[p * 256 + d];
+    unsigned h = 0u;
+    if (digit_totals) {
+        h = digit_totals[d];
+    } else {
+        for (unsigned t = 0; t < tiles; ++t) h += tile_counts[(size_t)t * 256 + d];
+        if ((int)d < num_totals) totals_out[d] = h;
+    }
     unsigned total;
     unsigned base = block_scan(h, AddU(), 0u, &total) - h;
     for (unsigned t = 0; t < tiles; ++t) {
@@ -230,28 +305,25 @@ __global__ void __launch_bounds__(kThreads) map_tile_offsets_kernel(const MapPla
 }
 
 // stable scatter of one tile: sub-tile by sub-tile, rank = earlier items of the same digit
-__global__ void __launch_bounds__(kThreads) map_scatter_kernel(const MapPlan* plan, int p, const MapRec* recs,
-                                                                unsigned n, int C, unsigned* bufs,
-                                                                const unsigned* tile_offsets)
+template <class Pass>
+__global__ void __launch_bounds__(kThreads) map_scatter_kernel(const Pass pass, unsigned n, const unsigned* tile_offsets)
 {
     __shared__ unsigned run[256];
     __shared__ unsigned wcnt[kThreads / 32][256];
-    if (!plan->active[p]) return;
-    const MapPlan& pl = *plan;
+    if (!pass.active()) return;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const unsigned lane_lt = (1u << lane) - 1u;
-    unsigned* dst = bufs + (size_t)pl.dst[p] * n;
     run[threadIdx.x] = tile_offsets[(size_t)blockIdx.x * 256 + threadIdx.x];
     for (int s = 0; s < kTileItems / kThreads; ++s) {
         for (int w = 0; w < kThreads / 32; ++w) wcnt[w][threadIdx.x] = 0u;
         __syncthreads();
         const unsigned i = blockIdx.x * (unsigned)kTileItems + s * kThreads + threadIdx.x;
         const bool valid = i < n;
-        const unsigned val = valid ? pass_input(pl, p, bufs, n, i) : 0u;
-        const unsigned d = valid ? rec_digit(recs[val], p, C) : 256u;
+        const unsigned it = valid ? pass.item(i) : 0u;
+        const unsigned d = valid ? pass.digit(it) : 256u;
         const unsigned peers = __match_any_sync(0xffffffffu, d);
         const unsigned rank = __popc(peers & lane_lt);
-        if (valid && rank == 0u) wcnt[warp][d] = __popc(peers);
+        if (d < 256u && rank == 0u) wcnt[warp][d] = __popc(peers);
         __syncthreads();
         unsigned sum = 0u;                                   // column of digit threadIdx.x
         for (int w = 0; w < kThreads / 32; ++w) {
@@ -260,7 +332,7 @@ __global__ void __launch_bounds__(kThreads) map_scatter_kernel(const MapPlan* pl
             sum += c;
         }
         __syncthreads();
-        if (valid) dst[run[d] + wcnt[warp][d] + rank] = val;
+        if (d < 256u) pass.put(run[d] + wcnt[warp][d] + rank, it);
         __syncthreads();
         run[threadIdx.x] += sum;
     }
@@ -362,6 +434,8 @@ struct ApArgs {
     double* ap;                       // (V, C, T) or nullptr
     double* voc;                      // (V, C, T, 11) or nullptr
     unsigned long long* det_hist;     // (V, C)
+    const int* owner;                 // (C,) merged compute: only classes with owner[c] == rank,
+    int rank;                         // the others get exact zeros; nullptr: every class
 };
 
 __global__ void __launch_bounds__(kThreads) map_ap_kernel(const __grid_constant__ ApArgs a)
@@ -371,7 +445,7 @@ __global__ void __launch_bounds__(kThreads) map_ap_kernel(const __grid_constant_
     __shared__ double carry[2];                             // interp and r of the later chunk's first record
     const int c = blockIdx.x, v = blockIdx.y, tid = threadIdx.x;
     const size_t vc = (size_t)v * a.C + c;
-    if (((a.views >> v) & 1) == 0 || a.n == 0u) {
+    if (((a.views >> v) & 1) == 0 || a.n == 0u || (a.owner && a.owner[c] != a.rank)) {
         if (tid == 0) a.det_hist[vc] = 0ull;
         for (int t = tid; t < a.T; t += kThreads) if (a.ap) a.ap[vc * a.T + t] = 0.0;
         for (int k = tid; k < a.T * MGD_MAP_VOC_POINTS; k += kThreads)
@@ -516,20 +590,26 @@ cudaError_t launch_map_write(const MapWriteArgs& a, cudaStream_t stream)
 size_t map_compute_scratch_bytes(long long n, int T)
 {
     const size_t tiles = (size_t)((n + kTileItems - 1) / kTileItems);
-    return align256(kDigits * 256 * 4) + align256(sizeof(MapPlan)) + align256(tiles * 256 * 4) +
+    return align256(kMaxDigits * 256 * 4) + align256(sizeof(MapPlan)) + align256(tiles * 256 * 4) +
            align256((size_t)n * 4 * 2) + align256((size_t)n * 4 * MGD_MAP_VIEWS) +
            (size_t)n * 8 * T * MGD_MAP_VIEWS;
 }
 
-cudaError_t launch_map_compute(const mgd_map_config& cfg, const MapRec* recs, long long n_,
-                               const unsigned long long* gt_hist, double* ap, double* voc,
-                               unsigned long long* det_hist, void* scratch, cudaStream_t stream)
+namespace {
+
+// S = 0: mgd_map_compute (equal keys later record first); S = kSlotDigits: the merged compute
+// over records stamped with their global slot, APs of the classes `owner` gives to `rank` only
+template <int S>
+cudaError_t map_compute_impl(const mgd_map_config& cfg, const MapRec* recs, long long n_,
+                             const unsigned long long* gt_hist, const int* owner, int rank, double* ap,
+                             double* voc, unsigned long long* det_hist, void* scratch, cudaStream_t stream)
 {
+    constexpr int nd = kDigits + S;
     const unsigned n = (unsigned)n_;
     const unsigned tiles = (unsigned)((n_ + kTileItems - 1) / kTileItems);
     char* s = static_cast<char*>(scratch);
     unsigned* hist = reinterpret_cast<unsigned*>(s);
-    s += align256(kDigits * 256 * 4);
+    s += align256(kMaxDigits * 256 * 4);
     MapPlan* plan = reinterpret_cast<MapPlan*>(s);
     s += align256(sizeof(MapPlan));
     unsigned* tile_counts = reinterpret_cast<unsigned*>(s);
@@ -542,15 +622,16 @@ cudaError_t launch_map_compute(const mgd_map_config& cfg, const MapRec* recs, lo
     cudaError_t e;
     prof_mark_begin(PROF_OTHER, stream);
     if (n > 0) {
-        if ((e = cudaMemsetAsync(hist, 0, kDigits * 256 * 4, stream)) != cudaSuccess) return e;
+        if ((e = cudaMemsetAsync(hist, 0, nd * 256 * 4, stream)) != cudaSuccess) return e;
         unsigned grid = (n + kThreads - 1) / kThreads;
         if (grid > 1184) grid = 1184;
-        map_hist_kernel<<<grid, kThreads, 0, stream>>>(recs, n, cfg.num_classes, hist);
-        map_plan_kernel<<<1, 32, 0, stream>>>(hist, n, plan);
-        for (int p = 0; p < kDigits; ++p) {
-            map_tile_count_kernel<<<tiles, kThreads, 0, stream>>>(plan, p, recs, n, cfg.num_classes, bufs, tile_counts);
-            map_tile_offsets_kernel<<<1, kThreads, 0, stream>>>(plan, p, hist, tiles, tile_counts);
-            map_scatter_kernel<<<tiles, kThreads, 0, stream>>>(plan, p, recs, n, cfg.num_classes, bufs, tile_counts);
+        map_hist_kernel<S><<<grid, kThreads, 0, stream>>>(recs, n, cfg.num_classes, hist);
+        map_plan_kernel<S><<<1, 32, 0, stream>>>(hist, n, plan);
+        for (int p = 0; p < nd; ++p) {
+            const SortPass<S> pass{plan, p, recs, n, cfg.num_classes, bufs};
+            map_tile_count_kernel<<<tiles, kThreads, 0, stream>>>(pass, n, tile_counts);
+            map_tile_offsets_kernel<<<1, kThreads, 0, stream>>>(pass, hist + p * 256, tiles, tile_counts, nullptr, 0);
+            map_scatter_kernel<<<tiles, kThreads, 0, stream>>>(pass, n, tile_counts);
         }
     }
     ApArgs a;
@@ -560,7 +641,46 @@ cudaError_t launch_map_compute(const mgd_map_config& cfg, const MapRec* recs, lo
     a.ap = cfg.method == MGD_MAP_COCO ? ap : nullptr;
     a.voc = cfg.method == MGD_MAP_VOC ? voc : nullptr;
     a.det_hist = det_hist;
+    a.owner = owner; a.rank = rank;
     map_ap_kernel<<<dim3((unsigned)cfg.num_classes, MGD_MAP_VIEWS), kThreads, 0, stream>>>(a);
+    prof_mark_end(PROF_OTHER, stream);
+    return cudaGetLastError();
+}
+
+}  // namespace
+
+cudaError_t launch_map_compute(const mgd_map_config& cfg, const MapRec* recs, long long n,
+                               const unsigned long long* gt_hist, double* ap, double* voc,
+                               unsigned long long* det_hist, void* scratch, cudaStream_t stream)
+{
+    return map_compute_impl<0>(cfg, recs, n, gt_hist, nullptr, 0, ap, voc, det_hist, scratch, stream);
+}
+
+cudaError_t launch_map_compute_merged(const mgd_map_config& cfg, const MapRec* recs, long long n,
+                                      const unsigned long long* gt_hist, const int* owner, int rank,
+                                      double* ap, double* voc, unsigned long long* det_hist, void* scratch,
+                                      cudaStream_t stream)
+{
+    return map_compute_impl<kSlotDigits>(cfg, recs, n, gt_hist, owner, rank, ap, voc, det_hist, scratch, stream);
+}
+
+size_t map_partition_scratch_bytes(long long n)
+{
+    return (size_t)((n + kTileItems - 1) / kTileItems) * 256 * 4;
+}
+
+cudaError_t launch_map_partition(const MapPartitionArgs& a, void* scratch, cudaStream_t stream)
+{
+    if (a.n == 0)
+        return cudaMemsetAsync(a.counts, 0, (size_t)a.world * sizeof(long long), stream);
+    const unsigned n = (unsigned)a.n;
+    const unsigned tiles = (unsigned)((a.n + kTileItems - 1) / kTileItems);
+    unsigned* tile_counts = static_cast<unsigned*>(scratch);
+    const PartitionPass pass{a.recs, a.C, a.owner, a.world, a.segs, a.num_segs, a.out, a.status};
+    prof_mark_begin(PROF_OTHER, stream);
+    map_tile_count_kernel<<<tiles, kThreads, 0, stream>>>(pass, n, tile_counts);
+    map_tile_offsets_kernel<<<1, kThreads, 0, stream>>>(pass, nullptr, tiles, tile_counts, a.counts, a.world);
+    map_scatter_kernel<<<tiles, kThreads, 0, stream>>>(pass, n, tile_counts);
     prof_mark_end(PROF_OTHER, stream);
     return cudaGetLastError();
 }

@@ -577,6 +577,89 @@ def map_compute(cfg, records, num_slots, gt_hist):
     return {"det_hist": det_hist.cpu().numpy(), "ap" if coco else "voc": out.cpu().numpy()}
 
 
+def _check_owner(owner, cfg, dev):
+    import torch
+    if not (_is_torch(owner) and owner.device == dev and owner.dtype == torch.int32 and owner.is_contiguous()
+            and tuple(owner.shape) == (cfg.num_classes,)):
+        raise ValueError(f"owner must be a contiguous int32 tensor of shape ({cfg.num_classes},) on {dev}")
+
+
+def map_partition(cfg, records, num_slots, segments, global_slots, owner, world):
+    """Group this rank's first ``num_slots`` records by the rank that owns their class, for the
+    sharded accumulator (``mgd_map_partition``).  ``segments``: (S, 2) int64 ``(L_u, G_u +
+    lo_r * M_u)`` per update with local images (a CUDA tensor or a sequence of pairs);
+    ``global_slots``: slots of all ranks over all updates; ``owner``: (C,) int32 CUDA tensor of
+    ranks in [0, world).  Padding slots are dropped and each record gets its global slot.
+    Returns the grouped records (a uint8 CUDA tensor with room for ``num_slots`` records) and
+    the records per destination rank, (world,) int64 on the device.  Enqueued on the current
+    stream; nothing synchronises."""
+    import torch
+    lib = _lib.load()
+    dev = records.device if _is_torch(records) else None
+    if not (_is_torch(records) and records.is_cuda and records.dtype == torch.uint8 and records.is_contiguous()):
+        raise ValueError("records must be a contiguous uint8 CUDA tensor")
+    num_slots, world = int(num_slots), int(world)
+    rb = map_record_bytes()
+    if num_slots < 0 or records.numel() < num_slots * rb:
+        raise ValueError(f"records holds {records.numel() // rb} records, num_slots is {num_slots}")
+    if world < 1:
+        raise ValueError(f"world must be >= 1, got {world}")
+    _check_owner(owner, cfg, dev)
+    if not _is_torch(segments):
+        segments = torch.tensor(np.asarray(segments, dtype=np.int64).reshape(-1, 2), device=dev)
+    if not (segments.device == dev and segments.dtype == torch.int64 and segments.is_contiguous()
+            and segments.dim() == 2 and segments.shape[1] == 2):
+        raise ValueError(f"segments must be a contiguous (S, 2) int64 tensor on {dev}")
+    if num_slots > 0 and segments.shape[0] == 0:
+        raise ValueError("segments is empty but there are records")
+    if int(global_slots) < num_slots:
+        raise ValueError(f"global_slots ({global_slots}) < num_slots ({num_slots})")
+    out = torch.empty((max(num_slots, 1) * rb,), dtype=torch.uint8, device=dev)
+    counts = torch.empty((world,), dtype=torch.int64, device=dev)
+    idx = dev.index or 0
+    p = lambda x: ctypes.c_void_p(x.data_ptr()) if x.numel() else None
+    rc = lib.mgd_map_partition(ctypes.byref(cfg), p(records) if num_slots else None, num_slots, p(segments),
+                               int(segments.shape[0]), int(global_slots), p(owner), world, p(out), p(counts),
+                               idx, ctypes.c_void_p(_torch_stream(idx)), 0)
+    _lib.raise_for_status(rc)
+    return out, counts
+
+
+def map_compute_merged(cfg, records, num_records, gt_hist, owner, rank):
+    """``map_compute`` over the records a rank received from ``map_partition`` of every rank
+    (``mgd_map_compute_merged``): ``gt_hist`` is the sum over the ranks, and only the classes
+    with ``owner[c] == rank`` get their APs and detection counts, the others exact zeros.
+    Returns CUDA tensors ``det_hist`` (MAP_VIEWS, C) int64 and ``ap`` (MAP_VIEWS, C, T) for
+    'coco' or ``voc`` (MAP_VIEWS, C, T, 11) for 'voc'.  Enqueued on the current stream."""
+    import torch
+    lib = _lib.load()
+    V, C, T = _lib.MAP_VIEWS, cfg.num_classes, cfg.num_thresholds
+    if not (_is_torch(gt_hist) and gt_hist.is_cuda and gt_hist.dtype == torch.int64 and gt_hist.is_contiguous()
+            and tuple(gt_hist.shape) == (V, C)):
+        raise ValueError(f"gt_hist must be a contiguous ({V}, {C}) int64 CUDA tensor")
+    dev = gt_hist.device
+    num_records = int(num_records)
+    if num_records < 0 or (num_records and not (
+            _is_torch(records) and records.device == dev and records.dtype == torch.uint8
+            and records.is_contiguous() and records.numel() >= num_records * map_record_bytes())):
+        raise ValueError(f"records must be a contiguous uint8 tensor on {dev} holding {num_records} records")
+    _check_owner(owner, cfg, dev)
+    if int(rank) < 0:
+        raise ValueError(f"rank must be >= 0, got {rank}")
+    det_hist = torch.empty((V, C), dtype=torch.int64, device=dev)
+    coco = cfg.method == _lib.MAP_COCO
+    out = torch.empty((V, C, T) if coco else (V, C, T, _lib.MAP_VOC_POINTS), dtype=torch.float64, device=dev)
+    idx = dev.index or 0
+    rc = lib.mgd_map_compute_merged(ctypes.byref(cfg), ctypes.c_void_p(records.data_ptr()) if num_records else None,
+                                    num_records, ctypes.c_void_p(gt_hist.data_ptr()),
+                                    ctypes.c_void_p(owner.data_ptr()), int(rank),
+                                    ctypes.c_void_p(out.data_ptr()) if coco else None,
+                                    None if coco else ctypes.c_void_p(out.data_ptr()),
+                                    ctypes.c_void_p(det_hist.data_ptr()), idx, ctypes.c_void_p(_torch_stream(idx)), 0)
+    _lib.raise_for_status(rc)
+    return {"det_hist": det_hist, "ap" if coco else "voc": out}
+
+
 def iou_matrix(boxes1, boxes2):
     """(n, m) float64 IoU matrix of xyxy boxes (``mgd_iou_matrix``), NumPy in / out."""
     lib = _lib.load()

@@ -392,3 +392,159 @@ class MapAccumulator:
         engine.poll_status(self.device.index or 0)
         full = _lib.MAP_VIEW_CORNER if self._args[6] else _lib.MAP_VIEW_CENTRE    # a view always matched
         return _map_results(_DeviceSource(out, self._gt_hist.cpu().numpy(), full), *self._args)
+
+
+def global_slot_segments(updates, rank: int, world_size: int):
+    """The sharded accumulator's global slots.  ``updates``: ``(n_total, max_dets)`` of every
+    update in order, the global batch of each split over the ranks by ``shard_bounds``.  Local
+    slot j of update u on ``rank`` is global slot ``G_u + lo * M_u + (j - L_u)``: ``G_u`` the
+    slots of all ranks over the earlier updates, ``lo`` the rank's first image, ``L_u`` its
+    local slot offset.  Returns the segments ``[(L_u, G_u + lo * M_u)]`` of the updates where
+    this rank has slots, and the global slot count."""
+    from ..sharding import shard_bounds
+    segments, local, glob = [], 0, 0
+    for n_total, m in updates:
+        lo, hi = shard_bounds(n_total, rank, world_size)
+        if (hi - lo) * m:
+            segments.append((local, glob + lo * m))
+        local += (hi - lo) * m
+        glob += n_total * m
+    return segments, glob
+
+
+def check_same_updates(updates, error=None, group=None) -> None:
+    """Collective over ``group`` (nothing to do without ``torch.distributed`` or at world size
+    1): raises ValueError on every rank if the ranks' ``(n_total, max_dets)`` update sequences
+    differ, and AssertionError on every rank if any rank passes an ``error`` (the class-range
+    report of its updates).  One ``all_gather_object``; no device is needed."""
+    from ..sharding import _dist
+    d = _dist()
+    if d is not None and d.get_world_size(group) > 1:
+        infos = [None] * d.get_world_size(group)
+        d.all_gather_object(infos, ([tuple(int(x) for x in u) for u in updates], error), group=group)
+        seqs = [seq for seq, _ in infos]
+        bad = [r for r, seq in enumerate(seqs) if seq != seqs[0]]
+        if bad:
+            raise ValueError(f"ranks {[0] + bad} made different update sequences (n_total, max_dets): "
+                             f"{len(seqs[0])} updates on rank 0, {[len(seqs[r]) for r in bad]} on the others")
+        errors = [(r, e) for r, (_, e) in enumerate(infos) if e]
+    else:
+        errors = [(0, error)] if error else []
+    if errors:
+        r, e = errors[0]
+        raise AssertionError(f"rank {r}: {e}")
+
+
+class ShardedMapAccumulator(MapAccumulator):
+    """``MapAccumulator`` over a batch sharded across the ranks of ``group`` (contiguous shards,
+    ``sharding.shard_bounds``), e.g. fed by ``ShardedGridPath.decode_nms(gather=False)``.
+
+    ``update`` takes this rank's shard of a global batch and, like ``MapAccumulator.update``,
+    only enqueues the matching on the current stream; it makes no collective call.  Every rank
+    makes the same sequence of updates.  ``compute`` is collective: each rank groups its
+    records by the rank that owns their class (class ``c`` belongs to rank ``c % world``;
+    ``mgd_map_partition``), the records are exchanged with ``all_to_all_single`` (device
+    tensors with NCCL, host memory with any other backend), each rank sorts what it received and
+    computes the APs of its own classes (``mgd_map_compute_merged``), and one all-reduce
+    assembles the tables.  Every rank returns the same dict, equal to ``MapAccumulator``'s over
+    the whole data: equal scores of a class are ordered later detection first in global image
+    order, because every record carries its global slot (``global_slot_segments``).  The
+    update sequences and the class-range status of all ranks are compared first, so a class id
+    out of range raises AssertionError on every rank.  Without ``torch.distributed`` or at world
+    size 1 the same partition and merged compute run without collectives."""
+
+    def __init__(self, num_classes: int, iou_thresholds: List[float] = None, class_names: List[str] = None,
+                 method: str = "coco", use_parallel: bool = True, optimize_classes: bool = True,
+                 cache_ious: bool = True, compute_per_scale: bool = True, device=None, group=None):
+        import torch
+        from ..sharding import _dist
+        d = _dist()
+        self.group = group
+        self.rank, self.world_size = (d.get_rank(group), d.get_world_size(group)) if d else (0, 1)
+        super().__init__(num_classes, iou_thresholds, class_names, method, use_parallel, optimize_classes,
+                         cache_ious, compute_per_scale, device)
+        self._owner = (torch.arange(int(num_classes), device=self.device) % self.world_size).to(torch.int32)
+
+    def reset(self) -> None:
+        """Forget every update (on this rank; every rank resets together)."""
+        super().reset()
+        self._updates = []
+
+    def update(self, det_boxes, det_scores, det_classes, det_counts, gt_boxes, gt_classes, gt_counts,
+               n_total: int = None) -> None:
+        """Add this rank's shard of a global batch of ``n_total`` images (default: the local batch
+        times the world size).  The shard must be the one ``shard_bounds(n_total)`` gives this
+        rank, possibly empty (a (0, M) / (0, N) batch), with the same M on every rank."""
+        from ..sharding import shard_bounds
+        n_local = int(det_scores.shape[0])
+        n_total = n_local * self.world_size if n_total is None else int(n_total)
+        lo, hi = shard_bounds(n_total, self.rank, self.world_size)
+        if hi - lo != n_local:
+            raise ValueError(f"rank {self.rank} holds {n_local} images, shard_bounds({n_total}) says {hi - lo}")
+        super().update(det_boxes, det_scores, det_classes, det_counts, gt_boxes, gt_classes, gt_counts)
+        self._updates.append((n_total, int(det_scores.shape[1])))
+
+    def _mark(self, phase: str) -> None:
+        """Called as each phase of ``compute`` has been enqueued ('check', 'partition', 'exchange',
+        'merged', 'reduce'); a hook for timing."""
+
+    def compute(self) -> Dict[str, Any]:
+        """``calculate_map``'s result dict over every rank's updates (collective)."""
+        import torch
+        error = None
+        try:
+            engine.poll_status(self.device.index or 0)
+        except AssertionError as e:
+            error = str(e)
+        check_same_updates(self._updates, error, self.group)
+        self._mark("check")
+        segments, global_slots = global_slot_segments(self._updates, self.rank, self.world_size)
+        send, counts = engine.map_partition(self._cfg, self._records, self._slots, segments, global_slots,
+                                            self._owner, self.world_size)
+        self._mark("partition")
+        if self.world_size == 1:
+            recs, n_recv, gt_hist = send, int(counts[0]), self._gt_hist
+        else:
+            recs, n_recv, gt_hist = self._exchange(send, counts)
+        self._mark("exchange")
+        out = engine.map_compute_merged(self._cfg, recs, n_recv, gt_hist, self._owner, self.rank)
+        self._mark("merged")
+        if self.world_size > 1:
+            out = self._all_reduce(out)
+        host = {k: v.cpu().numpy() for k, v in out.items()}
+        self._mark("reduce")
+        full = _lib.MAP_VIEW_CORNER if self._args[6] else _lib.MAP_VIEW_CENTRE
+        return _map_results(_DeviceSource(host, gt_hist.cpu().numpy(), full), *self._args)
+
+    def _wire(self):
+        """Where the collectives' tensors live: the device with NCCL, host memory otherwise."""
+        import torch
+        from ..sharding import _dist
+        return self.device if _dist().get_backend(self.group) == "nccl" else torch.device("cpu")
+
+    def _exchange(self, send, counts):
+        """Each rank's records to the ranks that own their classes; the summed ground truth."""
+        import torch
+        from ..sharding import _dist
+        d, g, rb, wire = _dist(), self.group, self._record_bytes, self._wire()
+        counts = counts.to(wire)
+        recv_counts = torch.empty_like(counts)
+        gt_hist = self._gt_hist.to(wire, copy=True)            # the local one stays: more updates may follow
+        d.all_to_all_single(recv_counts, counts, group=g)
+        d.all_reduce(gt_hist, group=g)
+        send_splits = [c * rb for c in counts.tolist()]
+        recv_splits = [c * rb for c in recv_counts.tolist()]
+        recs = torch.empty((sum(recv_splits),), dtype=torch.uint8, device=wire)
+        d.all_to_all_single(recs, send[:sum(send_splits)].to(wire), recv_splits, send_splits, group=g)
+        return recs.to(self.device), sum(recv_splits) // rb, gt_hist.to(self.device)
+
+    def _all_reduce(self, out):
+        """Sum the ranks' tables: each (view, class) is non-zero on its owner only, so the sums are
+        exact.  One float64 all-reduce; the detection counts travel as float64 (exact below 2^53)."""
+        import torch
+        from ..sharding import _dist
+        key = "ap" if "ap" in out else "voc"
+        det, n = out["det_hist"], out[key].numel()
+        flat = torch.cat([out[key].reshape(-1), det.reshape(-1).to(torch.float64)]).to(self._wire())
+        _dist().all_reduce(flat, group=self.group)
+        return {"det_hist": flat[n:].to(torch.int64).reshape(det.shape), key: flat[:n].reshape(out[key].shape)}
