@@ -393,6 +393,59 @@ MGD_API int mgd_map_compute_merged(const mgd_map_config *cfg, const void *record
                       int device, void *stream, int flags);
 
 /*
+ * Precision-recall curves and confidence operating points of the full-set views.
+ *
+ *   mgd_map_compute_pr         mgd_map_compute, and for every view in pr->views (MGD_MAP_VIEW_CORNER
+ *                              and / or MGD_MAP_VIEW_CENTRE, a subset of cfg->views) the curves and
+ *                              operating points below
+ *   mgd_map_compute_merged_pr  mgd_map_compute_merged, and the same for the classes owner[] gives
+ *                              `rank`; the other classes have empty curve segments and exact zeros in
+ *                              best_f1 / best_index / at_confidence, so the element-wise sum of the
+ *                              ranks' tables is the unsharded one
+ *
+ * Curves (CSR): the records of class c are [offsets[c], offsets[c + 1]) in the sort's order (score
+ * descending, equal scores later detection first), offsets[num_classes] records in all.  For
+ * record k of its class (0-based), at threshold t of view view_list[i] (the i-th set bit of views):
+ *   scores[offsets[c] + k]                    its score
+ *   precision[(i * T + t) * capacity + offsets[c] + k] = cum_tp / ((k + 1) + 1e-8)
+ *   recall   [(i * T + t) * capacity + offsets[c] + k] = cum_tp / (n_gt + 1e-8)
+ * in float64 in compute_precision_recall's (metrics.py:221-246) operation order.  A class without
+ * detections has an empty segment (the reference returns ([0.0], [0.0]) for it).
+ * Operating points, per (i, class, threshold); f1 = 2.0 * p * r / (p + r), 0 where p + r == 0:
+ *   best_f1 (V, C, T, 4)     (confidence = score[k], precision, recall, f1) at the first record k, in
+ *                            descending-score order, of maximum f1 among the records that end a
+ *                            run of equal scores (the only points a score >= confidence threshold
+ *                            can produce); zeros if that maximum is 0 or the class has no records
+ *   best_index (V, C, T)     that k, or -1 where best_f1 is zeros
+ *   at_confidence (V, C, T, Q, 3)  (precision, recall, f1) at record K - 1, K the class's records
+ *                            with score >= confidences[q]; zeros where K == 0.  NULL when Q == 0
+ * capacity must be >= num_slots (num_records for the merged form).  confidences is HOST memory
+ * (finite values, at most MGD_MAP_MAX_CONFIDENCES); every output is device memory.
+ */
+#define MGD_MAP_MAX_CONFIDENCES 32
+typedef struct {
+    int views;                        /* bit mask of MGD_MAP_VIEW_CORNER / _CENTRE, non-empty  */
+    int num_confidences;              /* Q in [0, MGD_MAP_MAX_CONFIDENCES]                     */
+    const double *confidences;        /* (Q,) host                                             */
+    long long capacity;               /* records per curve row of scores / precision / recall  */
+    long long *offsets;               /* (C + 1,) int64                                        */
+    double *scores;                   /* (capacity,)                                           */
+    double *precision;                /* (V, T, capacity), V = set bits of views               */
+    double *recall;                   /* (V, T, capacity)                                      */
+    double *best_f1;                  /* (V, C, T, 4)                                          */
+    long long *best_index;            /* (V, C, T)                                             */
+    double *at_confidence;            /* (V, C, T, Q, 3)                                       */
+} mgd_map_pr;
+MGD_API int mgd_map_compute_pr(const mgd_map_config *cfg, const void *records, long long num_slots,
+                      const long long *gt_hist, double *ap_out, double *voc_points_out,
+                      long long *det_hist_out, const mgd_map_pr *pr, int device, void *stream,
+                      int flags);
+MGD_API int mgd_map_compute_merged_pr(const mgd_map_config *cfg, const void *records,
+                      long long num_records, const long long *gt_hist, const int *owner, int rank,
+                      double *ap_out, double *voc_points_out, long long *det_hist_out,
+                      const mgd_map_pr *pr, int device, void *stream, int flags);
+
+/*
  * Loss-side ignore mask.  Replaces MultiGridLoss._compute_ignore_mask and
  * _compute_iou_batch (multigriddet/losses/multigrid_loss.py:494-703, 445-492), called once
  * per layer from the loss (:316).  Forward only: the reference casts the mask from a

@@ -25,6 +25,7 @@ IOU_CORNER, IOU_CENTRE = 0, 1
 BOXES_I32, BOXES_F64 = 0, 1
 
 MAP_MAX_THRESHOLDS, MAP_VOC_POINTS = 32, 11
+MAP_MAX_CONFIDENCES = 32
 MAP_COCO, MAP_VOC = 0, 1
 MAP_VIEW_CORNER, MAP_VIEW_CENTRE, MAP_VIEW_S, MAP_VIEW_M, MAP_VIEW_L, MAP_VIEWS = range(6)
 
@@ -73,6 +74,23 @@ class MapConfig(ctypes.Structure):
     ]
 
 
+class MapPr(ctypes.Structure):
+    """``mgd_map_pr``"""
+    _fields_ = [
+        ("views", ctypes.c_int),
+        ("num_confidences", ctypes.c_int),
+        ("confidences", ctypes.c_void_p),
+        ("capacity", ctypes.c_longlong),
+        ("offsets", ctypes.c_void_p),
+        ("scores", ctypes.c_void_p),
+        ("precision", ctypes.c_void_p),
+        ("recall", ctypes.c_void_p),
+        ("best_f1", ctypes.c_void_p),
+        ("best_index", ctypes.c_void_p),
+        ("at_confidence", ctypes.c_void_p),
+    ]
+
+
 class MgdError(RuntimeError):
     pass
 
@@ -93,7 +111,7 @@ EXPORTS = ("mgd_version", "mgd_last_error", "mgd_device_count", "mgd_encode_targ
            "mgd_encode_ignore_mask", "mgd_exchange_create", "mgd_exchange_connect",
            "mgd_exchange_buffer", "mgd_exchange_timeouts", "mgd_exchange_destroy",
            "mgd_map_record_bytes", "mgd_map_update", "mgd_map_compute", "mgd_map_partition",
-           "mgd_map_compute_merged")
+           "mgd_map_compute_merged", "mgd_map_compute_pr", "mgd_map_compute_merged_pr")
 
 IPC_HANDLE_BYTES = 64
 
@@ -236,6 +254,15 @@ def load():
         ctypes.POINTER(MapConfig), ctypes.c_void_p, ctypes.c_longlong, ctypes.c_void_p, ctypes.c_void_p,
         ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p,
         ctypes.c_int]
+    lib.mgd_map_compute_pr.restype = ctypes.c_int
+    lib.mgd_map_compute_pr.argtypes = [
+        ctypes.POINTER(MapConfig), ctypes.c_void_p, ctypes.c_longlong, ctypes.c_void_p, ctypes.c_void_p,
+        ctypes.c_void_p, ctypes.c_void_p, ctypes.POINTER(MapPr), ctypes.c_int, ctypes.c_void_p, ctypes.c_int]
+    lib.mgd_map_compute_merged_pr.restype = ctypes.c_int
+    lib.mgd_map_compute_merged_pr.argtypes = [
+        ctypes.POINTER(MapConfig), ctypes.c_void_p, ctypes.c_longlong, ctypes.c_void_p, ctypes.c_void_p,
+        ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.POINTER(MapPr), ctypes.c_int,
+        ctypes.c_void_p, ctypes.c_int]
     lib.mgd_profile_begin.restype = ctypes.c_int
     lib.mgd_profile_end.restype = ctypes.c_int
     lib.mgd_profile_end.argtypes = [_DP, _LLP]

@@ -2107,6 +2107,99 @@ int mgd_map_compute_merged(const mgd_map_config* cfg, const void* records, long 
     return MGD_OK;
 }
 
+namespace {
+
+// the curve / operating-point outputs of mgd_map_compute_pr and _merged_pr; n: records in
+int check_map_pr(const mgd_map_config* cfg, const mgd_map_pr* pr, long long n)
+{
+    const int full = (1 << MGD_MAP_VIEW_CORNER) | (1 << MGD_MAP_VIEW_CENTRE);
+    if (!pr) return fail(MGD_ERR_INVALID_ARGUMENT, "pr is NULL");
+    if (pr->views == 0 || (pr->views & ~full))
+        return fail(MGD_ERR_INVALID_ARGUMENT, "pr->views must be a non-empty mask of MGD_MAP_VIEW_CORNER / _CENTRE");
+    if (pr->views & ~cfg->views)
+        return fail(MGD_ERR_INVALID_ARGUMENT, "pr->views holds a view cfg->views does not match");
+    if (pr->num_confidences < 0 || pr->num_confidences > MGD_MAP_MAX_CONFIDENCES)
+        return fail(MGD_ERR_INVALID_ARGUMENT, "num_confidences must be in [0, %d], got %d",
+                    MGD_MAP_MAX_CONFIDENCES, pr->num_confidences);
+    if (pr->num_confidences > 0 && (!pr->confidences || !pr->at_confidence))
+        return fail(MGD_ERR_INVALID_ARGUMENT, "NULL confidences or at_confidence");
+    for (int q = 0; q < pr->num_confidences; ++q)
+        if (!isfinite(pr->confidences[q]))
+            return fail(MGD_ERR_INVALID_ARGUMENT, "confidences[%d] is not finite", q);
+    if (pr->capacity < n)
+        return fail(MGD_ERR_INVALID_ARGUMENT, "capacity (%lld) is below the record count (%lld)", pr->capacity, n);
+    if (!pr->offsets || !pr->best_f1 || !pr->best_index)
+        return fail(MGD_ERR_INVALID_ARGUMENT, "NULL operating-point output");
+    if (pr->capacity > 0 && (!pr->scores || !pr->precision || !pr->recall))
+        return fail(MGD_ERR_INVALID_ARGUMENT, "NULL curve output");
+    return MGD_OK;
+}
+
+}  // namespace
+
+int mgd_map_compute_pr(const mgd_map_config* cfg, const void* records, long long num_slots,
+                       const long long* gt_hist, double* ap_out, double* voc_points_out,
+                       long long* det_hist_out, const mgd_map_pr* pr, int device, void* stream, int flags)
+{
+    nvtx_range nv_api("mgd_map_compute_pr");
+    int rc;
+    if ((rc = check_map_config(cfg))) return rc;
+    if (num_slots < 0 || num_slots > 0x7fffffffll)
+        return fail(MGD_ERR_INVALID_ARGUMENT, "num_slots must be in [0, 2^31 - 1]");
+    if ((num_slots > 0 && !records) || !gt_hist || !det_hist_out)
+        return fail(MGD_ERR_INVALID_ARGUMENT, "NULL tensor");
+    if (cfg->method == MGD_MAP_COCO ? !ap_out : !voc_points_out)
+        return fail(MGD_ERR_INVALID_ARGUMENT, "NULL output of the configured method");
+    if ((rc = check_map_pr(cfg, pr, num_slots))) return rc;
+    int num_sms;
+    DeviceScope dev_scope;
+    if ((rc = prepare_device(device, &num_sms, &dev_scope))) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    Arena* ws;
+    if ((rc = map_workspace(device, st, &ws))) return rc;
+    void* scratch;
+    CUDA_TRY(ws->take(&scratch, map_compute_scratch_bytes(num_slots, cfg->num_thresholds)));
+    CUDA_TRY(launch_map_compute(*cfg, static_cast<const MapRec*>(records), num_slots,
+                                reinterpret_cast<const unsigned long long*>(gt_hist), ap_out, voc_points_out,
+                                reinterpret_cast<unsigned long long*>(det_hist_out), scratch, st, pr));
+    if ((rc = map_workspace_done(device, st))) return rc;
+    if (flags & MGD_FLAG_SYNC) CUDA_TRY(cudaStreamSynchronize(st));
+    return MGD_OK;
+}
+
+int mgd_map_compute_merged_pr(const mgd_map_config* cfg, const void* records, long long num_records,
+                              const long long* gt_hist, const int* owner, int rank, double* ap_out,
+                              double* voc_points_out, long long* det_hist_out, const mgd_map_pr* pr, int device,
+                              void* stream, int flags)
+{
+    nvtx_range nv_api("mgd_map_compute_merged_pr");
+    int rc;
+    if ((rc = check_map_config(cfg))) return rc;
+    if (num_records < 0 || num_records > 0x7fffffffll)
+        return fail(MGD_ERR_INVALID_ARGUMENT, "num_records must be in [0, 2^31 - 1]");
+    if ((num_records > 0 && !records) || !gt_hist || !owner || !det_hist_out)
+        return fail(MGD_ERR_INVALID_ARGUMENT, "NULL tensor");
+    if (cfg->method == MGD_MAP_COCO ? !ap_out : !voc_points_out)
+        return fail(MGD_ERR_INVALID_ARGUMENT, "NULL output of the configured method");
+    if (rank < 0) return fail(MGD_ERR_INVALID_ARGUMENT, "rank must be >= 0, got %d", rank);
+    if ((rc = check_map_pr(cfg, pr, num_records))) return rc;
+    int num_sms;
+    DeviceScope dev_scope;
+    if ((rc = prepare_device(device, &num_sms, &dev_scope))) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    Arena* ws;
+    if ((rc = map_workspace(device, st, &ws))) return rc;
+    void* scratch;
+    CUDA_TRY(ws->take(&scratch, map_compute_scratch_bytes(num_records, cfg->num_thresholds)));
+    CUDA_TRY(launch_map_compute_merged(*cfg, static_cast<const MapRec*>(records), num_records,
+                                       reinterpret_cast<const unsigned long long*>(gt_hist), owner, rank,
+                                       ap_out, voc_points_out, reinterpret_cast<unsigned long long*>(det_hist_out),
+                                       scratch, st, pr));
+    if ((rc = map_workspace_done(device, st))) return rc;
+    if (flags & MGD_FLAG_SYNC) CUDA_TRY(cudaStreamSynchronize(st));
+    return MGD_OK;
+}
+
 int mgd_ignore_mask(const mgd_head_config* cfg, const float* const* y_pred,
                     const float* const* y_true, int batch, double ignore_thresh, double eps,
                     float* const* ignore_mask, float* const* assigned_anchor_iou,

@@ -183,17 +183,19 @@ struct MapWriteArgs {
 };
 cudaError_t launch_map_write(const MapWriteArgs& a, cudaStream_t stream);
 
-// scratch of map_compute (bytes), and the enqueue of sort + AP kernels
+// scratch of map_compute (bytes), and the enqueue of sort + AP kernels; with `pr` (validated by
+// the caller) also the curves and operating points of mgd_map_compute_pr
 size_t map_compute_scratch_bytes(long long n, int T);
 cudaError_t launch_map_compute(const mgd_map_config& cfg, const MapRec* recs, long long n,
                                const unsigned long long* gt_hist, double* ap, double* voc,
-                               unsigned long long* det_hist, void* scratch, cudaStream_t stream);
+                               unsigned long long* det_hist, void* scratch, cudaStream_t stream,
+                               const mgd_map_pr* pr = nullptr);
 // the same over records stamped by map_partition (ties broken by the global slot, descending);
 // only the classes `owner` gives to `rank` get APs, the others exact zeros
 cudaError_t launch_map_compute_merged(const mgd_map_config& cfg, const MapRec* recs, long long n,
                                       const unsigned long long* gt_hist, const int* owner, int rank,
                                       double* ap, double* voc, unsigned long long* det_hist, void* scratch,
-                                      cudaStream_t stream);
+                                      cudaStream_t stream, const mgd_map_pr* pr = nullptr);
 
 // mgd_map_partition: the records grouped by the rank that owns their class, in local order,
 // padding dropped, each stamped with its global slot (MapRec::pad)

@@ -23,6 +23,9 @@
 // stamp each with its global slot; the merged sort takes four more digits from that slot
 // (descending, so equal scores stay later detection first in global image order), and
 // map_ap_kernel walks only the classes the rank owns.
+// map_pr_kernel (mgd_map_compute_pr / _merged_pr): one CTA per (class, threshold, full-set view)
+// over the same sorted order writes the precision-recall curve and the F1 / confidence
+// operating points; map_ap_kernel and its launch are unchanged.
 //
 // compute_average_precision sorts the recalls with np.argsort (metrics.py:285) before the
 // trapezoid.  They are non-decreasing already, but the sort is NumPy's unstable introsort
@@ -570,6 +573,124 @@ __global__ void __launch_bounds__(kThreads) map_ap_kernel(const __grid_constant_
     }
 }
 
+// ---- precision-recall curves and operating points -------------------------------------------
+struct PrArgs {
+    int C, T, Q;
+    int view[2];                      // view of output slot blockIdx.z (corner / centre)
+    double conf[MGD_MAP_MAX_CONFIDENCES];
+    const MapRec* recs;
+    unsigned n;
+    const MapPlan* plan;
+    const unsigned* bufs;
+    const unsigned long long* gt_hist;
+    const int* owner;                 // as in ApArgs: the others get exact zeros
+    int rank;
+    long long cap;                    // row length of precision / recall
+    long long* offsets;               // (C + 1,)
+    double* scores;                   // (cap,)
+    double* precision;                // (V, T, cap)
+    double* recall;                   // (V, T, cap)
+    double* best_f1;                  // (V, C, T, 4)
+    long long* best_index;            // (V, C, T)
+    double* at_conf;                  // (V, C, T, Q, 3)
+};
+
+__device__ __forceinline__ double f1_of(double p, double r) { return p + r == 0.0 ? 0.0 : 2.0 * p * r / (p + r); }
+
+// One CTA per (class, threshold, view): walks the class's segment of the sorted order forwards,
+// writes p and r at every record (the segment starts at offsets[c], so a record's sorted
+// position is its curve position), keeps the first maximum F1 among records that end a run of
+// equal scores, then finds each confidence's cut by binary search over the descending scores.
+__global__ void __launch_bounds__(kThreads) map_pr_kernel(const __grid_constant__ PrArgs a)
+{
+    __shared__ unsigned seg[2];
+    const int c = blockIdx.x, t = blockIdx.y, vi = blockIdx.z, v = a.view[vi], tid = threadIdx.x;
+    const size_t vct = ((size_t)vi * a.C + c) * a.T + t;
+    const unsigned* sorted = a.n ? a.bufs + (size_t)a.plan->final_buf * a.n : nullptr;
+    if (tid < 2) {                                          // class segment, as in map_ap_kernel
+        const unsigned want = (unsigned)c + tid;
+        unsigned lo = 0u, hi = a.n;
+        while (lo < hi) {
+            const unsigned mid = lo + (hi - lo) / 2;
+            if (class_key(a.recs[sorted[mid]].cls, a.C) < want) lo = mid + 1; else hi = mid;
+        }
+        seg[tid] = lo;
+    }
+    __syncthreads();
+    const unsigned s0 = seg[0], s1 = seg[1];                // empty for a class another rank owns
+    if (t == 0 && vi == 0 && tid == 0) {
+        a.offsets[c] = s0;
+        if (c == a.C - 1) a.offsets[a.C] = s1;
+    }
+    const size_t row = ((size_t)vi * a.T + t) * (size_t)a.cap;
+    const double r_den = (double)a.gt_hist[(size_t)v * a.C + c] + 1e-8;
+    unsigned carry = 0u, best_k = 0xffffffffu;
+    double best = 0.0;
+    for (unsigned base = s0; base < s1; base += kThreads) {
+        const unsigned i = base + tid;
+        const bool valid = i < s1;
+        unsigned f = 0u;
+        double s = 0.0;
+        if (valid) {
+            const MapRec& r = a.recs[sorted[i]];
+            f = (r.bits[v] >> t) & 1u;
+            s = r.score;
+        }
+        unsigned total;
+        const unsigned cum_tp = carry + block_scan(f, AddU(), 0u, &total);
+        if (valid) {
+            const unsigned k = i - s0;
+            // compute_precision_recall: cum_tp / (cum_tp + cum_fp + 1e-8), cum_tp / (num_gt + 1e-8)
+            const double p = (double)cum_tp / ((double)(k + 1u) + 1e-8);
+            const double r = (double)cum_tp / r_den;
+            a.precision[row + i] = p;
+            a.recall[row + i] = r;
+            if (t == 0 && vi == 0) a.scores[i] = s;
+            if (i + 1u == s1 || a.recs[sorted[i + 1u]].score != s) {     // a threshold can stop here
+                const double f1 = f1_of(p, r);
+                if (f1 > best) { best = f1; best_k = k; }   // k ascends per thread: the first maximum
+            }
+        }
+        carry += total;
+    }
+    double m;
+    block_scan(best, MaxD(), 0.0, &m);
+    double neg_k;                                           // the smallest k that reaches m, as -k
+    block_scan(m > 0.0 && best == m ? -(double)best_k : -4294967295.0, MaxD(), -4294967295.0, &neg_k);
+    const unsigned k_first = (unsigned)-neg_k;
+    // block_scan ended in __syncthreads: every p and r of the segment is visible to the CTA
+    if (tid == 0) {
+        double* o = a.best_f1 + vct * 4;
+        if (k_first == 0xffffffffu) {
+            o[0] = o[1] = o[2] = o[3] = 0.0;
+            a.best_index[vct] = (a.owner && a.owner[c] != a.rank) ? 0 : -1;
+        } else {
+            const unsigned i = s0 + k_first;
+            o[0] = a.recs[sorted[i]].score;
+            o[1] = a.precision[row + i];
+            o[2] = a.recall[row + i];
+            o[3] = m;
+            a.best_index[vct] = k_first;
+        }
+    }
+    for (int q = tid; q < a.Q; q += kThreads) {
+        unsigned lo = s0, hi = s1;                          // first record with score < conf[q]
+        while (lo < hi) {
+            const unsigned mid = lo + (hi - lo) / 2;
+            if (a.recs[sorted[mid]].score >= a.conf[q]) lo = mid + 1; else hi = mid;
+        }
+        double* o = a.at_conf + (vct * a.Q + q) * 3;
+        if (lo == s0) {
+            o[0] = o[1] = o[2] = 0.0;
+        } else {
+            const double p = a.precision[row + lo - 1], r = a.recall[row + lo - 1];
+            o[0] = p;
+            o[1] = r;
+            o[2] = f1_of(p, r);
+        }
+    }
+}
+
 size_t align256(size_t b) { return (b + 255) & ~(size_t)255; }
 
 }  // namespace
@@ -602,7 +723,8 @@ namespace {
 template <int S>
 cudaError_t map_compute_impl(const mgd_map_config& cfg, const MapRec* recs, long long n_,
                              const unsigned long long* gt_hist, const int* owner, int rank, double* ap,
-                             double* voc, unsigned long long* det_hist, void* scratch, cudaStream_t stream)
+                             double* voc, unsigned long long* det_hist, void* scratch, cudaStream_t stream,
+                             const mgd_map_pr* pr)
 {
     constexpr int nd = kDigits + S;
     const unsigned n = (unsigned)n_;
@@ -643,6 +765,21 @@ cudaError_t map_compute_impl(const mgd_map_config& cfg, const MapRec* recs, long
     a.det_hist = det_hist;
     a.owner = owner; a.rank = rank;
     map_ap_kernel<<<dim3((unsigned)cfg.num_classes, MGD_MAP_VIEWS), kThreads, 0, stream>>>(a);
+    if (pr) {
+        PrArgs q;
+        q.C = cfg.num_classes; q.T = cfg.num_thresholds; q.Q = pr->num_confidences;
+        int nv = 0;
+        for (int v = MGD_MAP_VIEW_CORNER; v <= MGD_MAP_VIEW_CENTRE; ++v)
+            if ((pr->views >> v) & 1) q.view[nv++] = v;
+        for (int k = 0; k < MGD_MAP_MAX_CONFIDENCES; ++k) q.conf[k] = k < q.Q ? pr->confidences[k] : 0.0;
+        q.recs = recs; q.n = n; q.plan = plan; q.bufs = bufs; q.gt_hist = gt_hist;
+        q.owner = owner; q.rank = rank;
+        q.cap = pr->capacity; q.offsets = pr->offsets; q.scores = pr->scores;
+        q.precision = pr->precision; q.recall = pr->recall;
+        q.best_f1 = pr->best_f1; q.best_index = pr->best_index; q.at_conf = pr->at_confidence;
+        map_pr_kernel<<<dim3((unsigned)cfg.num_classes, (unsigned)cfg.num_thresholds, (unsigned)nv), kThreads, 0,
+                        stream>>>(q);
+    }
     prof_mark_end(PROF_OTHER, stream);
     return cudaGetLastError();
 }
@@ -651,17 +788,19 @@ cudaError_t map_compute_impl(const mgd_map_config& cfg, const MapRec* recs, long
 
 cudaError_t launch_map_compute(const mgd_map_config& cfg, const MapRec* recs, long long n,
                                const unsigned long long* gt_hist, double* ap, double* voc,
-                               unsigned long long* det_hist, void* scratch, cudaStream_t stream)
+                               unsigned long long* det_hist, void* scratch, cudaStream_t stream,
+                               const mgd_map_pr* pr)
 {
-    return map_compute_impl<0>(cfg, recs, n, gt_hist, nullptr, 0, ap, voc, det_hist, scratch, stream);
+    return map_compute_impl<0>(cfg, recs, n, gt_hist, nullptr, 0, ap, voc, det_hist, scratch, stream, pr);
 }
 
 cudaError_t launch_map_compute_merged(const mgd_map_config& cfg, const MapRec* recs, long long n,
                                       const unsigned long long* gt_hist, const int* owner, int rank,
                                       double* ap, double* voc, unsigned long long* det_hist, void* scratch,
-                                      cudaStream_t stream)
+                                      cudaStream_t stream, const mgd_map_pr* pr)
 {
-    return map_compute_impl<kSlotDigits>(cfg, recs, n, gt_hist, owner, rank, ap, voc, det_hist, scratch, stream);
+    return map_compute_impl<kSlotDigits>(cfg, recs, n, gt_hist, owner, rank, ap, voc, det_hist, scratch, stream,
+                                         pr);
 }
 
 size_t map_partition_scratch_bytes(long long n)

@@ -660,6 +660,116 @@ def map_compute_merged(cfg, records, num_records, gt_hist, owner, rank):
     return {"det_hist": det_hist, "ap" if coco else "voc": out}
 
 
+_MAP_PR_TABLES = ("best_f1", "best_index", "at_confidence")
+
+
+def _map_pr_request(cfg, views, confidences, num_records, dev):
+    """Check a curve request and allocate its outputs: ``(mgd_map_pr, host confidences, CUDA
+    tensors)``; raises ValueError before any device work."""
+    import torch
+    views = sorted(set(int(v) for v in views))
+    if not views or any(v not in (_lib.MAP_VIEW_CORNER, _lib.MAP_VIEW_CENTRE) for v in views):
+        raise ValueError("curve views must be a non-empty subset of (MAP_VIEW_CORNER, MAP_VIEW_CENTRE)")
+    if any(not (cfg.views >> v) & 1 for v in views):
+        raise ValueError(f"curve views {views} are not all matched by the configuration")
+    conf = np.ascontiguousarray(np.asarray([] if confidences is None else confidences, dtype=np.float64).reshape(-1))
+    if len(conf) > _lib.MAP_MAX_CONFIDENCES:
+        raise ValueError(f"at most {_lib.MAP_MAX_CONFIDENCES} confidences supported, got {len(conf)}")
+    if not np.all(np.isfinite(conf)):
+        raise ValueError("confidences must be finite")
+    V, C, T, Q = len(views), cfg.num_classes, cfg.num_thresholds, len(conf)
+    cap = max(int(num_records), 1)
+    f64 = dict(dtype=torch.float64, device=dev)
+    out = {"views": views,
+           "offsets": torch.empty((C + 1,), dtype=torch.int64, device=dev),
+           "scores": torch.empty((cap,), **f64),
+           "precision": torch.empty((V, T, cap), **f64),
+           "recall": torch.empty((V, T, cap), **f64),
+           "best_f1": torch.empty((V, C, T, 4), **f64),
+           "best_index": torch.empty((V, C, T), dtype=torch.int64, device=dev),
+           "at_confidence": torch.empty((V, C, T, Q, 3), **f64)}
+    pr = _lib.MapPr()
+    pr.views = sum(1 << v for v in views)
+    pr.num_confidences = Q
+    pr.confidences = conf.ctypes.data if Q else None
+    pr.capacity = cap
+    for k in ("offsets", "scores", "precision", "recall", "best_f1", "best_index"):
+        setattr(pr, k, out[k].data_ptr())
+    pr.at_confidence = out["at_confidence"].data_ptr() if Q else None
+    return pr, conf, out
+
+
+def map_compute_pr(cfg, records, num_slots, gt_hist, views, confidences=None):
+    """``map_compute`` plus the precision-recall curves and operating points of the full-set
+    ``views`` (MAP_VIEW_CORNER and / or MAP_VIEW_CENTRE, matched by ``cfg``) in one call
+    (``mgd_map_compute_pr``); ``confidences``: up to 32 finite scores to evaluate p / r / F1 at.
+    Returns ``map_compute``'s dict (NumPy) with ``"pr"``: ``views`` (the list, in order), CUDA
+    tensors ``offsets`` (C+1,), ``scores`` (cap,), ``precision`` / ``recall`` (V, T, cap) -- the
+    first ``offsets[C]`` entries of a row are used -- and NumPy ``best_f1`` (V, C, T, 4),
+    ``best_index`` (V, C, T), ``at_confidence`` (V, C, T, Q, 3).  Synchronises."""
+    import torch
+    lib = _lib.load()
+    dev = gt_hist.device
+    V, C, T = _lib.MAP_VIEWS, cfg.num_classes, cfg.num_thresholds
+    num_slots = int(num_slots)
+    if num_slots < 0:
+        raise ValueError(f"num_slots must be >= 0, got {num_slots}")
+    pr, conf, tensors = _map_pr_request(cfg, views, confidences, num_slots, dev)
+    det_hist = torch.empty((V, C), dtype=torch.int64, device=dev)
+    coco = cfg.method == _lib.MAP_COCO
+    out = torch.empty((V, C, T) if coco else (V, C, T, _lib.MAP_VOC_POINTS), dtype=torch.float64, device=dev)
+    idx = dev.index or 0
+    rc = lib.mgd_map_compute_pr(ctypes.byref(cfg),
+                                ctypes.c_void_p(records.data_ptr()) if records is not None and num_slots else None,
+                                num_slots, ctypes.c_void_p(gt_hist.data_ptr()),
+                                ctypes.c_void_p(out.data_ptr()) if coco else None,
+                                None if coco else ctypes.c_void_p(out.data_ptr()),
+                                ctypes.c_void_p(det_hist.data_ptr()), ctypes.byref(pr), idx,
+                                ctypes.c_void_p(_torch_stream(idx)), 0)
+    _lib.raise_for_status(rc)
+    for k in _MAP_PR_TABLES:
+        tensors[k] = tensors[k].cpu().numpy()
+    return {"det_hist": det_hist.cpu().numpy(), "ap" if coco else "voc": out.cpu().numpy(), "pr": tensors}
+
+
+def map_compute_merged_pr(cfg, records, num_records, gt_hist, owner, rank, views, confidences=None):
+    """``map_compute_merged`` plus ``map_compute_pr``'s curves and operating points for the
+    classes with ``owner[c] == rank`` (``mgd_map_compute_merged_pr``): the other classes have
+    empty curve segments and exact zeros in ``best_f1`` / ``best_index`` / ``at_confidence``, so
+    summing the tables over the ranks assembles them.  Every output is a CUDA tensor; enqueued on
+    the current stream."""
+    import torch
+    lib = _lib.load()
+    V, C, T = _lib.MAP_VIEWS, cfg.num_classes, cfg.num_thresholds
+    if not (_is_torch(gt_hist) and gt_hist.is_cuda and gt_hist.dtype == torch.int64 and gt_hist.is_contiguous()
+            and tuple(gt_hist.shape) == (V, C)):
+        raise ValueError(f"gt_hist must be a contiguous ({V}, {C}) int64 CUDA tensor")
+    dev = gt_hist.device
+    num_records = int(num_records)
+    if num_records < 0 or (num_records and not (
+            _is_torch(records) and records.device == dev and records.dtype == torch.uint8
+            and records.is_contiguous() and records.numel() >= num_records * map_record_bytes())):
+        raise ValueError(f"records must be a contiguous uint8 tensor on {dev} holding {num_records} records")
+    _check_owner(owner, cfg, dev)
+    if int(rank) < 0:
+        raise ValueError(f"rank must be >= 0, got {rank}")
+    pr, conf, tensors = _map_pr_request(cfg, views, confidences, num_records, dev)
+    det_hist = torch.empty((V, C), dtype=torch.int64, device=dev)
+    coco = cfg.method == _lib.MAP_COCO
+    out = torch.empty((V, C, T) if coco else (V, C, T, _lib.MAP_VOC_POINTS), dtype=torch.float64, device=dev)
+    idx = dev.index or 0
+    rc = lib.mgd_map_compute_merged_pr(ctypes.byref(cfg),
+                                       ctypes.c_void_p(records.data_ptr()) if num_records else None,
+                                       num_records, ctypes.c_void_p(gt_hist.data_ptr()),
+                                       ctypes.c_void_p(owner.data_ptr()), int(rank),
+                                       ctypes.c_void_p(out.data_ptr()) if coco else None,
+                                       None if coco else ctypes.c_void_p(out.data_ptr()),
+                                       ctypes.c_void_p(det_hist.data_ptr()), ctypes.byref(pr), idx,
+                                       ctypes.c_void_p(_torch_stream(idx)), 0)
+    _lib.raise_for_status(rc)
+    return {"det_hist": det_hist, "ap" if coco else "voc": out, "pr": tensors}
+
+
 def iou_matrix(boxes1, boxes2):
     """(n, m) float64 IoU matrix of xyxy boxes (``mgd_iou_matrix``), NumPy in / out."""
     lib = _lib.load()

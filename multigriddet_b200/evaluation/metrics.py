@@ -308,6 +308,8 @@ class _DeviceSource:
 
     def ap_table(self, iou_thresholds, matcher: str, method: str):
         v = self.view if self.band else (_lib.MAP_VIEW_CORNER if matcher == "corner" else _lib.MAP_VIEW_CENTRE)
+        if not self.band:
+            self.matcher_view = v                         # the view of the main APs, for the curves
         det, gt = self.out["det_hist"][v], self.gt_hist[v]
 
         def ap_of(class_id, t):
@@ -320,6 +322,32 @@ class _DeviceSource:
             # compute_average_precision: float(np.sum(...)), or interp[0] * r[0] for one record
             return ap if det[class_id] == 1 else float(ap)
         return ap_of
+
+
+def _full_views(cfg):
+    """The full-set views a configuration matches (one or both of corner and centre)."""
+    return [v for v in (_lib.MAP_VIEW_CORNER, _lib.MAP_VIEW_CENTRE) if (cfg.views >> v) & 1]
+
+
+def _check_pr_args(precision_recall, confidences):
+    if confidences is not None and not precision_recall:
+        raise ValueError("confidences are evaluated with precision_recall=True only")
+
+
+def _precision_recall(pr, view, num_records, gt_hist, confidences) -> Dict[str, Any]:
+    """compute()'s "precision_recall" entry: the curves and tables of ``view`` out of the
+    compute's (``engine.map_compute_pr``) outputs, the curves trimmed to ``num_records`` and no
+    longer sharing memory with the other view's."""
+    import torch
+    vi = pr["views"].index(view)
+    own = lambda t: t.clone(memory_format=torch.contiguous_format)
+    res = {"matcher": "corner" if view == _lib.MAP_VIEW_CORNER else "centre",
+           "offsets": pr["offsets"], "scores": own(pr["scores"][:num_records]),
+           "precision": own(pr["precision"][vi, :, :num_records]), "recall": own(pr["recall"][vi, :, :num_records]),
+           "num_gt": np.array(gt_hist[view]), "best_f1": pr["best_f1"][vi], "best_index": pr["best_index"][vi]}
+    if confidences is not None:
+        res["at_confidence"] = pr["at_confidence"][vi]
+    return res
 
 
 class MapAccumulator:
@@ -386,12 +414,47 @@ class MapAccumulator:
                           det_classes, det_counts, gt_boxes, gt_classes, gt_counts)
         self._slots += slots
 
-    def compute(self) -> Dict[str, Any]:
-        """``calculate_map``'s result dict over every update since construction or ``reset``."""
+    def compute(self, precision_recall: bool = False, confidences=None) -> Dict[str, Any]:
+        """``calculate_map``'s result dict over every update since construction or ``reset``.
+
+        With ``precision_recall`` the same dict gains ``"precision_recall"``, computed in the same
+        library call (``mgd_map_compute_pr``) for the matcher ``calculate_map`` uses for its main
+        APs (``"matcher"``: 'corner' or 'centre'), per class ``c`` and threshold ``t``:
+
+        - ``offsets`` (C+1,), ``scores`` (n,), ``precision`` / ``recall`` (T, n): CUDA tensors.
+          The curve of class c is ``[offsets[c], offsets[c+1])``: its detections by descending
+          score (equal scores: later detection first), with ``compute_precision_recall``'s
+          values of the sorted TP / FP flags of ``match_predictions_to_gt(_cached)``, bit for bit.
+          A class without detections has an empty segment, not the reference's ``([0.0], [0.0])``.
+        - ``num_gt`` (C,): ground truth per class.
+        - ``best_f1`` (C, T, 4): (confidence, precision, recall, F1) at the first maximum of
+          ``F1 = 2 p r / (p + r)`` among the detections that end a run of equal scores -- the
+          points a ``score >= confidence`` filter can produce; zeros when that maximum is 0.
+          ``best_index`` (C, T): its position in the class's curve, -1 where ``best_f1`` is zeros.
+        - ``at_confidence`` (C, T, Q, 3), with ``confidences`` (up to 32 finite values): the
+          (precision, recall, F1) of the detections with ``score >= confidences[q]``, zeros where
+          none is left.  Equal to filtering the detections by that score and evaluating again.
+        """
+        _check_pr_args(precision_recall, confidences)
+        if precision_recall:
+            return self._compute_pr(confidences)
         out = engine.map_compute(self._cfg, self._records, self._slots, self._gt_hist)
         engine.poll_status(self.device.index or 0)
         full = _lib.MAP_VIEW_CORNER if self._args[6] else _lib.MAP_VIEW_CENTRE    # a view always matched
         return _map_results(_DeviceSource(out, self._gt_hist.cpu().numpy(), full), *self._args)
+
+    def _compute_pr(self, confidences) -> Dict[str, Any]:
+        # the matcher of the main APs is only known from the counts: curves of both full-set views
+        out = engine.map_compute_pr(self._cfg, self._records, self._slots, self._gt_hist, _full_views(self._cfg),
+                                    confidences)
+        engine.poll_status(self.device.index or 0)
+        full = _lib.MAP_VIEW_CORNER if self._args[6] else _lib.MAP_VIEW_CENTRE
+        gt = self._gt_hist.cpu().numpy()
+        src = _DeviceSource(out, gt, full)
+        res = _map_results(src, *self._args)
+        n = int(out["det_hist"][src.matcher_view].sum())
+        res["precision_recall"] = _precision_recall(out["pr"], src.matcher_view, n, gt, confidences)
+        return res
 
 
 def global_slot_segments(updates, rank: int, world_size: int):
@@ -488,9 +551,16 @@ class ShardedMapAccumulator(MapAccumulator):
         """Called as each phase of ``compute`` has been enqueued ('check', 'partition', 'exchange',
         'merged', 'reduce'); a hook for timing."""
 
-    def compute(self) -> Dict[str, Any]:
-        """``calculate_map``'s result dict over every rank's updates (collective)."""
+    def compute(self, precision_recall: bool = False, confidences=None) -> Dict[str, Any]:
+        """``calculate_map``'s result dict over every rank's updates (collective).
+
+        ``precision_recall`` / ``confidences`` as for ``MapAccumulator.compute``, in the same
+        collective calls: every rank holds the whole ``best_f1`` / ``best_index`` /
+        ``at_confidence`` tables (they join the one all-reduce), while the curves stay on the
+        rank that owns the class.  ``owned`` (C,) marks this rank's classes; the other classes
+        have empty curve segments here."""
         import torch
+        _check_pr_args(precision_recall, confidences)
         error = None
         try:
             engine.poll_status(self.device.index or 0)
@@ -507,14 +577,29 @@ class ShardedMapAccumulator(MapAccumulator):
         else:
             recs, n_recv, gt_hist = self._exchange(send, counts)
         self._mark("exchange")
-        out = engine.map_compute_merged(self._cfg, recs, n_recv, gt_hist, self._owner, self.rank)
+        if precision_recall:
+            out = engine.map_compute_merged_pr(self._cfg, recs, n_recv, gt_hist, self._owner, self.rank,
+                                               _full_views(self._cfg), confidences)
+        else:
+            out = engine.map_compute_merged(self._cfg, recs, n_recv, gt_hist, self._owner, self.rank)
         self._mark("merged")
         if self.world_size > 1:
             out = self._all_reduce(out)
+        pr = out.pop("pr", None)
         host = {k: v.cpu().numpy() for k, v in out.items()}
         self._mark("reduce")
         full = _lib.MAP_VIEW_CORNER if self._args[6] else _lib.MAP_VIEW_CENTRE
-        return _map_results(_DeviceSource(host, gt_hist.cpu().numpy(), full), *self._args)
+        gt = gt_hist.cpu().numpy()
+        src = _DeviceSource(host, gt, full)
+        res = _map_results(src, *self._args)
+        if pr is not None:
+            for k in engine._MAP_PR_TABLES:
+                pr[k] = pr[k].cpu().numpy()
+            owned = (self._owner == self.rank).cpu().numpy()
+            n = int(host["det_hist"][src.matcher_view][owned].sum())     # this rank's records
+            res["precision_recall"] = _precision_recall(pr, src.matcher_view, n, gt, confidences)
+            res["precision_recall"]["owned"] = owned
+        return res
 
     def _wire(self):
         """Where the collectives' tensors live: the device with NCCL, host memory otherwise."""
@@ -540,11 +625,20 @@ class ShardedMapAccumulator(MapAccumulator):
 
     def _all_reduce(self, out):
         """Sum the ranks' tables: each (view, class) is non-zero on its owner only, so the sums are
-        exact.  One float64 all-reduce; the detection counts travel as float64 (exact below 2^53)."""
+        exact.  One float64 all-reduce; the detection counts and best indices travel as float64
+        (exact below 2^53).  The curves are not sent."""
         import torch
         from ..sharding import _dist
         key = "ap" if "ap" in out else "voc"
-        det, n = out["det_hist"], out[key].numel()
-        flat = torch.cat([out[key].reshape(-1), det.reshape(-1).to(torch.float64)]).to(self._wire())
+        pr = out.get("pr")
+        tables = [out[key], out["det_hist"]] + ([pr[k] for k in engine._MAP_PR_TABLES] if pr else [])
+        flat = torch.cat([t.reshape(-1).to(torch.float64) for t in tables]).to(self._wire())
         _dist().all_reduce(flat, group=self.group)
-        return {"det_hist": flat[n:].to(torch.int64).reshape(det.shape), key: flat[:n].reshape(out[key].shape)}
+        summed, lo = [], 0
+        for t in tables:
+            summed.append(flat[lo:lo + t.numel()].to(t.dtype).reshape(t.shape))
+            lo += t.numel()
+        res = {key: summed[0], "det_hist": summed[1]}
+        if pr:
+            res["pr"] = dict(pr, **dict(zip(engine._MAP_PR_TABLES, summed[2:])))
+        return res
