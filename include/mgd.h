@@ -446,6 +446,45 @@ MGD_API int mgd_map_compute_merged_pr(const mgd_map_config *cfg, const void *rec
                       const mgd_map_pr *pr, int device, void *stream, int flags);
 
 /*
+ * Detection confusion matrix at chosen confidences.  Extends the matcher of mgd_match_detections
+ * (match_predictions_to_gt_cached / match_predictions_to_gt, multigriddet/evaluation/metrics.py:
+ * 147-218, 73-144) with a cross-class stage, per image, at one IoU threshold thr and for each
+ * confidence conf[q]:
+ *   kept     the first det_counts[b] detections with score >= conf[q] (padding is ignored);
+ *   stage 1  the reference's matcher on the kept set, unchanged (iou_mode as for
+ *            mgd_match_detections); each pair adds 1 to matrix[q, c, c];
+ *   stage 2  the kept detections stage 1 left unmatched, in the same order (score descending,
+ *            equal scores later slot first), each claim the unclaimed ground truth of ANY class
+ *            with the highest IoU (equal IoU: lowest ground-truth index) when it is >= thr; each
+ *            pair adds 1 to matrix[q, gt class, det class] and is never of one class;
+ *   then     each kept detection still unmatched adds 1 to matrix[q, C, det class] (a false
+ *            positive on background), each ground truth still unclaimed to matrix[q, gt class, C]
+ *            (a missed object).
+ * Rows are the true class, columns the detected class, index C background; [C, C] stays 0.  The
+ * diagonal is the matcher's TP count at that confidence, row g < C sums to the ground truth of
+ * class g and column d < C to the class-d detections with score >= conf[q].
+ *
+ *   inputs     mgd_map_update's layout: det_boxes (batch, max_dets, 4) f64, det_scores (batch,
+ *              max_dets) f64 -- FINITE values, det_classes (batch, max_dets) int32, det_counts
+ *              (batch,) int32; gt_boxes (batch, max_gt, 4) f64, gt_classes (batch, max_gt) int32,
+ *              gt_counts (batch,) int32; max_dets <= 65535
+ *   iou_threshold in (0, 1];  confidences: num_confidences HOST doubles, finite, 1 to
+ *              MGD_MAP_MAX_CONFIDENCES (pass -DBL_MAX to keep every detection)
+ *   matrix     (num_confidences, num_classes + 1, num_classes + 1) int64, device memory, added to
+ *              (the caller zeroes it once, then sums any number of updates into it)
+ * A class id outside [0, num_classes) on a real slot is reported as MGD_ERR_CLASS_RANGE through
+ * mgd_poll_status (MGD_FLAG_SYNC synchronises and reports it); cells with such an id are not
+ * counted.  Device memory only; work is enqueued on `stream`; scratch comes from the calling
+ * thread's workspace (mgd_release_workspace).
+ */
+MGD_API int mgd_confusion_update(const double *det_boxes, const double *det_scores,
+                      const int *det_classes, const int *det_counts, int batch, int max_dets,
+                      const double *gt_boxes, const int *gt_classes, const int *gt_counts, int max_gt,
+                      int num_classes, double iou_threshold, int iou_mode,
+                      const double *confidences, int num_confidences,
+                      long long *matrix, int device, void *stream, int flags);
+
+/*
  * Loss-side ignore mask.  Replaces MultiGridLoss._compute_ignore_mask and
  * _compute_iou_batch (multigriddet/losses/multigrid_loss.py:494-703, 445-492), called once
  * per layer from the loss (:316).  Forward only: the reference casts the mask from a

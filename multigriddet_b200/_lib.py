@@ -111,7 +111,8 @@ EXPORTS = ("mgd_version", "mgd_last_error", "mgd_device_count", "mgd_encode_targ
            "mgd_encode_ignore_mask", "mgd_exchange_create", "mgd_exchange_connect",
            "mgd_exchange_buffer", "mgd_exchange_timeouts", "mgd_exchange_destroy",
            "mgd_map_record_bytes", "mgd_map_update", "mgd_map_compute", "mgd_map_partition",
-           "mgd_map_compute_merged", "mgd_map_compute_pr", "mgd_map_compute_merged_pr")
+           "mgd_map_compute_merged", "mgd_map_compute_pr", "mgd_map_compute_merged_pr",
+           "mgd_confusion_update")
 
 IPC_HANDLE_BYTES = 64
 
@@ -263,6 +264,11 @@ def load():
         ctypes.POINTER(MapConfig), ctypes.c_void_p, ctypes.c_longlong, ctypes.c_void_p, ctypes.c_void_p,
         ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.POINTER(MapPr), ctypes.c_int,
         ctypes.c_void_p, ctypes.c_int]
+    lib.mgd_confusion_update.restype = ctypes.c_int
+    lib.mgd_confusion_update.argtypes = [
+        ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_int,
+        ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_double,
+        ctypes.c_int, _DP, ctypes.c_int, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_int]
     lib.mgd_profile_begin.restype = ctypes.c_int
     lib.mgd_profile_end.restype = ctypes.c_int
     lib.mgd_profile_end.argtypes = [_DP, _LLP]

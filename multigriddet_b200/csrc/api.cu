@@ -402,6 +402,7 @@ int status_to_error(int st)
                     "negative class id on a valid box (the reference would write a wrong channel)");
     if (st & 4) return fail(MGD_ERR_CLASS_RANGE, "mAP update: class id outside [0, num_classes)");
     if (st & 8) return fail(MGD_ERR_INVALID_ARGUMENT, "mAP partition: owner table entry outside [0, world)");
+    if (st & 16) return fail(MGD_ERR_CLASS_RANGE, "confusion update: class id outside [0, num_classes)");
     return MGD_OK;
 }
 
@@ -2197,6 +2198,77 @@ int mgd_map_compute_merged_pr(const mgd_map_config* cfg, const void* records, lo
                                        scratch, st, pr));
     if ((rc = map_workspace_done(device, st))) return rc;
     if (flags & MGD_FLAG_SYNC) CUDA_TRY(cudaStreamSynchronize(st));
+    return MGD_OK;
+}
+
+int mgd_confusion_update(const double* det_boxes, const double* det_scores, const int* det_classes,
+                         const int* det_counts, int batch, int max_dets, const double* gt_boxes,
+                         const int* gt_classes, const int* gt_counts, int max_gt, int num_classes,
+                         double iou_threshold, int iou_mode, const double* confidences, int num_confidences,
+                         long long* matrix, int device, void* stream, int flags)
+{
+    nvtx_range nv_api("mgd_confusion_update");
+    int rc;
+    if (batch < 0 || max_dets < 0 || max_gt < 0)
+        return fail(MGD_ERR_INVALID_ARGUMENT, "batch, max_dets and max_gt must be >= 0");
+    if (num_classes < 1) return fail(MGD_ERR_INVALID_ARGUMENT, "num_classes must be >= 1, got %d", num_classes);
+    if (!(iou_threshold > 0.0 && iou_threshold <= 1.0))
+        return fail(MGD_ERR_INVALID_ARGUMENT, "iou_threshold must be in (0, 1], got %g", iou_threshold);
+    if (iou_mode != MGD_IOU_CORNER && iou_mode != MGD_IOU_CENTRE)
+        return fail(MGD_ERR_INVALID_ARGUMENT, "iou_mode must be MGD_IOU_CORNER or MGD_IOU_CENTRE");
+    if (num_confidences < 1 || num_confidences > MGD_MAP_MAX_CONFIDENCES)
+        return fail(MGD_ERR_INVALID_ARGUMENT, "num_confidences must be in [1, %d], got %d",
+                    MGD_MAP_MAX_CONFIDENCES, num_confidences);
+    if (!confidences) return fail(MGD_ERR_INVALID_ARGUMENT, "confidences is NULL");
+    for (int q = 0; q < num_confidences; ++q)
+        if (!isfinite(confidences[q]))
+            return fail(MGD_ERR_INVALID_ARGUMENT, "confidences[%d] is not finite", q);
+    if (max_dets > 65535) return fail(MGD_ERR_UNSUPPORTED, "max_dets per image must be <= 65535");
+    if ((size_t)max_dets * 2 + (size_t)max_gt / 8 > 48 * 1024)
+        return fail(MGD_ERR_UNSUPPORTED, "max_dets / max_gt too large for one warp's shared memory");
+    if (!matrix) return fail(MGD_ERR_INVALID_ARGUMENT, "matrix is NULL");
+    if (batch > 0 && (!det_counts || !gt_counts))
+        return fail(MGD_ERR_INVALID_ARGUMENT, "NULL tensor");
+    if ((long long)batch * max_dets > 0 && (!det_boxes || !det_scores || !det_classes))
+        return fail(MGD_ERR_INVALID_ARGUMENT, "NULL detection tensor");
+    if ((long long)batch * max_gt > 0 && (!gt_boxes || !gt_classes))
+        return fail(MGD_ERR_INVALID_ARGUMENT, "NULL ground-truth tensor");
+    int num_sms;
+    DeviceScope dev_scope;
+    if ((rc = prepare_device(device, &num_sms, &dev_scope))) return rc;
+    if (batch == 0) return MGD_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    ConfusionArgs c;
+    memset(&c, 0, sizeof(c));
+    if ((rc = deferred_status_word(device, &c.status))) return rc;
+    Arena* ws;
+    if ((rc = map_workspace(device, st, &ws))) return rc;
+    const size_t slots = (size_t)batch * max_dets;
+    int* counters;
+    CUDA_TRY(ws->take(reinterpret_cast<void**>(&counters), 2 * sizeof(int)));
+    CUDA_TRY(cudaMemsetAsync(counters, 0, 2 * sizeof(int), st));
+    // stage 1: the reference's matcher, once, at the one threshold
+    MatchArgs m;
+    memset(&m, 0, sizeof(m));
+    m.B = batch; m.M = max_dets; m.N = max_gt; m.T = 1; m.thr[0] = iou_threshold; m.mode = iou_mode;
+    m.det_boxes = det_boxes; m.det_scores = det_scores; m.det_classes = det_classes; m.det_counts = det_counts;
+    m.gt_boxes = gt_boxes; m.gt_classes = gt_classes; m.gt_counts = gt_counts;
+    CUDA_TRY(ws->take(reinterpret_cast<void**>(&m.matched), slots * sizeof(int)));
+    CUDA_TRY(ws->take(reinterpret_cast<void**>(&m.tp), slots));
+    m.next_image = counters;
+    if (slots) CUDA_TRY(launch_match(m, num_sms, st));
+    // stage 2 and the counts
+    c.B = batch; c.M = max_dets; c.N = max_gt; c.C = num_classes; c.Q = num_confidences;
+    c.mode = iou_mode; c.thr = iou_threshold;
+    for (int q = 0; q < num_confidences; ++q) c.conf[q] = confidences[q];
+    c.det_boxes = det_boxes; c.det_scores = det_scores; c.det_classes = det_classes; c.det_counts = det_counts;
+    c.gt_boxes = gt_boxes; c.gt_classes = gt_classes; c.gt_counts = gt_counts;
+    c.matched = m.matched;
+    c.matrix = reinterpret_cast<unsigned long long*>(matrix);
+    c.next_image = counters + 1;
+    CUDA_TRY(launch_confusion(c, num_sms, st));
+    if ((rc = map_workspace_done(device, st))) return rc;
+    if (flags & MGD_FLAG_SYNC) return mgd_poll_status(device, stream);
     return MGD_OK;
 }
 

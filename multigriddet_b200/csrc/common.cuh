@@ -149,6 +149,23 @@ struct MatchArgs {
     int* next_image;                  // work counter, zeroed by the caller
 };
 
+// ---- detection confusion matrix (match.cu: confusion_kernel) ---------------------------
+// Stage 1 is one match_kernel walk at `thr` (T = 1, no band); confusion_kernel takes its claims
+// and runs the cross-class stage for every confidence.
+struct ConfusionArgs {
+    int B, M, N, C, Q;
+    int mode;                         // MGD_IOU_CORNER / MGD_IOU_CENTRE, as for stage 1
+    double thr;
+    double conf[MGD_MAP_MAX_CONFIDENCES];
+    const double* det_boxes; const double* det_scores; const int* det_classes; const int* det_counts;
+    const double* gt_boxes; const int* gt_classes; const int* gt_counts;
+    const int* matched;               // (B, M) stage-1 claim of each detection, -1 = none
+    unsigned long long* matrix;       // (Q, C+1, C+1) counts, added to
+    int* next_image;                  // work counter, zeroed by the caller
+    int* status;                      // bit 4: class id outside [0, C)
+};
+cudaError_t launch_confusion(const ConfusionArgs& a, int num_sms, cudaStream_t stream);
+
 // Area band of an xyxy box for the per-scale APs: 0 = S (-inf, 1024), 1 = M [1024, 9216),
 // 2 = L [9216, inf), 3 = none (NaN area).  The area is (x2-x1)*(y2-y1) in float64
 // (metrics.py:_box_area) and the bounds are compared as _filter_by_area does.

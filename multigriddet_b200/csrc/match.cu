@@ -14,6 +14,7 @@
 // decides identically.  An optional area band (MatchArgs::band) restricts the walk to the
 // boxes calculate_map's per-scale filter keeps, which is the filtered lists' result: their
 // relative visiting order and ground-truth index order are those of the full lists.
+// confusion_kernel extends one such walk with a cross-class stage (mgd_confusion_update).
 #include <math.h>
 #include "common.cuh"
 
@@ -147,6 +148,131 @@ match_kernel(const __grid_constant__ MatchArgs a)
     }
 }
 
+// Detection confusion matrix at each confidence conf[q] (mgd_confusion_update), one warp per
+// image.  The kept detections (score >= conf[q]) are a prefix of match_kernel's visiting order:
+// equal scores are never split by the filter, and the greedy walk never looks ahead, so stage 1
+// on the kept set is the full walk's claims (a.matched) restricted to that prefix.
+//   stage 1: each claim of a kept detection counts [c, c];
+//   stage 2: the kept detections stage 1 left unmatched, in the same order, each claim the
+//            unclaimed ground truth of ANY class with the highest IoU (equal IoU: lowest index)
+//            when it is >= thr, counted [gt class, det class].  Such a pair is never of one
+//            class: at the detection's stage-1 turn every unclaimed ground truth of its class had
+//            IoU < thr, and the unclaimed set has only shrunk since;
+//   the kept detections still unmatched count [C, det class] (background row), the ground truth
+//   still unclaimed [gt class, C] (background column).
+// The shared memory per warp is match_kernel's: the visiting order and the claimed bitmap.
+__global__ void __launch_bounds__(kMatchWarps * 32)
+confusion_kernel(const __grid_constant__ ConfusionArgs a)
+{
+    extern __shared__ __align__(16) unsigned char dyn[];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const size_t per_warp = (size_t)a.M * 2 + (size_t)((a.N + 31) / 32) * 4 + 16;
+    unsigned short* order = reinterpret_cast<unsigned short*>(dyn + warp * ((per_warp + 15) & ~(size_t)15));
+    unsigned* taken = reinterpret_cast<unsigned*>(order + ((a.M + 1) & ~1));
+    const int words = (a.N + 31) / 32;
+    const long long C1 = (long long)a.C + 1;
+
+    for (;;) {
+        int b = 0;
+        if (lane == 0) b = atomicAdd(a.next_image, 1);
+        b = __shfl_sync(0xffffffffu, b, 0);
+        if (b >= a.B) break;
+        const int n = min(max(a.det_counts[b], 0), a.M);
+        const int g = min(max(a.gt_counts[b], 0), a.N);
+        const double* dbox = a.det_boxes + (size_t)b * a.M * 4;
+        const double* dsc = a.det_scores + (size_t)b * a.M;
+        const int* dcl = a.det_classes + (size_t)b * a.M;
+        const double* gbox = a.gt_boxes + (size_t)b * a.N * 4;
+        const int* gcl = a.gt_classes + (size_t)b * a.N;
+        const int* who = a.matched + (size_t)b * a.M;
+
+        // class ids of the real slots; a cell with an id out of range is never counted
+        bool bad = false;
+        for (int i = lane; i < n; i += 32) bad |= (unsigned)dcl[i] >= (unsigned)a.C;
+        for (int j = lane; j < g; j += 32) bad |= (unsigned)gcl[j] >= (unsigned)a.C;
+        if (__any_sync(0xffffffffu, bad) && lane == 0) atomicOr(a.status, 16);
+
+        // match_kernel's visiting order: score descending, equal scores later slot first
+        for (int i = lane; i < n; i += 32) {
+            const double si = dsc[i];
+            int rank = 0;
+            for (int j = 0; j < n; ++j) {
+                const double sj = dsc[j];
+                rank += (sj > si) || (sj == si && j > i);
+            }
+            order[rank] = (unsigned short)i;
+        }
+        __syncwarp();
+
+        for (int q = 0; q < a.Q; ++q) {
+            unsigned long long* mat = a.matrix + (size_t)q * C1 * C1;
+            const double conf = a.conf[q];
+            int K = 0;                                  // kept detections: order[0, K)
+            for (int i = lane; i < n; i += 32) K += dsc[i] >= conf;
+            #pragma unroll
+            for (int o = 16; o > 0; o >>= 1) K += __shfl_xor_sync(0xffffffffu, K, o);
+
+            // stage 1
+            for (int w = lane; w < words; w += 32) taken[w] = 0u;
+            __syncwarp();
+            for (int k = lane; k < K; k += 32) {
+                const int d = order[k];
+                const int j = who[d];
+                if (j < 0) continue;
+                atomicOr(&taken[j >> 5], 1u << (j & 31));
+                const int c = dcl[d];
+                if ((unsigned)c < (unsigned)a.C) atomicAdd(mat + c * C1 + c, 1ull);
+            }
+            __syncwarp();
+
+            // stage 2 and the background row
+            for (int k = 0; k < K; ++k) {
+                const int d = order[k];
+                if (who[d] >= 0) continue;
+                const double p[4] = {dbox[4 * d], dbox[4 * d + 1], dbox[4 * d + 2], dbox[4 * d + 3]};
+                double best = 0.0;                      // thr > 0: an IoU of 0 never claims
+                int best_j = -1;
+                for (int j = lane; j < g; j += 32) {
+                    if ((taken[j >> 5] >> (j & 31)) & 1u) continue;
+                    const double qb[4] = {gbox[4 * j], gbox[4 * j + 1], gbox[4 * j + 2], gbox[4 * j + 3]};
+                    const double v = a.mode ? iou_centre(p, qb) : iou_corner(p, qb);
+                    if (v > best) { best = v; best_j = j; }
+                }
+                // most unmatched detections have no candidate at all: skip the reduction
+                const bool hit = __any_sync(0xffffffffu, best_j >= 0 && best >= a.thr);
+                if (hit) {
+                    #pragma unroll
+                    for (int o = 16; o > 0; o >>= 1) {
+                        const double ov = __shfl_xor_sync(0xffffffffu, best, o);
+                        const int oj = __shfl_xor_sync(0xffffffffu, best_j, o);
+                        const bool take = oj >= 0 && (best_j < 0 || ov > best || (ov == best && oj < best_j));
+                        if (take) { best = ov; best_j = oj; }
+                    }
+                }
+                if (lane == 0) {
+                    const int c = dcl[d];
+                    int row = a.C;
+                    if (hit) {                              // the maximum is >= thr
+                        taken[best_j >> 5] |= 1u << (best_j & 31);
+                        row = gcl[best_j];
+                    }
+                    if ((unsigned)c < (unsigned)a.C && (unsigned)row <= (unsigned)a.C)
+                        atomicAdd(mat + row * C1 + c, 1ull);
+                }
+                __syncwarp();
+            }
+
+            // background column
+            for (int j = lane; j < g; j += 32) {
+                const int c = gcl[j];
+                if (!((taken[j >> 5] >> (j & 31)) & 1u) && (unsigned)c < (unsigned)a.C)
+                    atomicAdd(mat + c * C1 + a.C, 1ull);
+            }
+            __syncwarp();
+        }
+    }
+}
+
 __global__ void iou_matrix_kernel(const double* b1, int n, const double* b2, int m, double* out)
 {
     const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -169,6 +295,21 @@ cudaError_t launch_match(const MatchArgs& a, int num_sms, cudaStream_t stream)
     if (grid < 1) grid = 1;
     prof_mark_begin(PROF_OTHER, stream);
     kernel<<<(unsigned)grid, kMatchWarps * 32, smem, stream>>>(a);
+    prof_mark_end(PROF_OTHER, stream);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_confusion(const ConfusionArgs& a, int num_sms, cudaStream_t stream)
+{
+    const size_t per_warp = ((size_t)a.M * 2 + (size_t)((a.N + 31) / 32) * 4 + 16 + 15) & ~(size_t)15;
+    const size_t smem = per_warp * kMatchWarps;
+    cudaError_t e = cudaFuncSetAttribute(confusion_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    long long grid = ((long long)a.B + kMatchWarps - 1) / kMatchWarps;
+    if (grid > (long long)num_sms * 8) grid = (long long)num_sms * 8;
+    if (grid < 1) grid = 1;
+    prof_mark_begin(PROF_OTHER, stream);
+    confusion_kernel<<<(unsigned)grid, kMatchWarps * 32, smem, stream>>>(a);
     prof_mark_end(PROF_OTHER, stream);
     return cudaGetLastError();
 }

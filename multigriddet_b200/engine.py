@@ -443,6 +443,9 @@ def profile_end():
 # mAP matching (reference multigriddet/evaluation/metrics.py)
 # ------------------------------------------------------------------------------
 
+_IOU_MODES = {"corner": _lib.IOU_CORNER, "centre": _lib.IOU_CENTRE, "center": _lib.IOU_CENTRE}
+
+
 def match_detections(det_boxes, det_scores, det_classes, det_counts, gt_boxes, gt_classes, gt_counts,
                      iou_thresholds, iou_mode="corner", return_matched=False, sync=True):
     """TP flags of padded per-image detections against padded per-image ground truth
@@ -453,7 +456,7 @@ def match_detections(det_boxes, det_scores, det_classes, det_counts, gt_boxes, g
     (and ``matched_gt`` (T, B, M) int32 when asked) in the same memory space.
     """
     lib = _lib.load()
-    mode = {"corner": _lib.IOU_CORNER, "centre": _lib.IOU_CENTRE, "center": _lib.IOU_CENTRE}[iou_mode]
+    mode = _IOU_MODES[iou_mode]
     thr = np.ascontiguousarray(np.asarray(iou_thresholds, dtype=np.float64).reshape(-1))
     T = int(thr.shape[0])
     thr_p = thr.ctypes.data_as(ctypes.POINTER(ctypes.c_double))
@@ -768,6 +771,72 @@ def map_compute_merged_pr(cfg, records, num_records, gt_hist, owner, rank, views
                                        ctypes.c_void_p(_torch_stream(idx)), 0)
     _lib.raise_for_status(rc)
     return {"det_hist": det_hist, "ap" if coco else "voc": out, "pr": tensors}
+
+
+def confusion_config(num_classes, iou_threshold=0.5, confidences=None, iou_mode="corner"):
+    """Check the settings of a confusion matrix the way ``mgd_confusion_update`` would, before any
+    device work.  Returns ``(num_classes, iou_threshold, confidences (Q,) float64, iou_mode code)``;
+    ``confidences=None`` is one matrix over every detection (the most negative float64, which
+    every finite score passes)."""
+    if isinstance(num_classes, bool) or int(num_classes) != num_classes or int(num_classes) < 1:
+        raise ValueError(f"num_classes must be an integer >= 1, got {num_classes}")
+    thr = float(iou_threshold)
+    if not 0.0 < thr <= 1.0:
+        raise ValueError(f"iou_threshold must be in (0, 1], got {iou_threshold}")
+    if iou_mode not in _IOU_MODES:
+        raise ValueError(f"iou_mode must be 'corner' or 'centre', got {iou_mode!r}")
+    conf = np.asarray([np.finfo(np.float64).min] if confidences is None else confidences, dtype=np.float64)
+    conf = np.ascontiguousarray(conf.reshape(-1))
+    if not 1 <= len(conf) <= _lib.MAP_MAX_CONFIDENCES:
+        raise ValueError(f"between 1 and {_lib.MAP_MAX_CONFIDENCES} confidences supported, got {len(conf)}")
+    if not np.all(np.isfinite(conf)):
+        raise ValueError("confidences must be finite")
+    return int(num_classes), thr, conf, _IOU_MODES[iou_mode]
+
+
+def confusion_update(matrix, confidences, iou_threshold, iou_mode, det_boxes, det_scores, det_classes, det_counts,
+                     gt_boxes, gt_classes, gt_counts, sync=False):
+    """Add one batch's detection confusion matrices to ``matrix`` ((Q, C+1, C+1) int64 CUDA tensor;
+    rows: true class, columns: detected class, index C: background) at each of the Q
+    ``confidences``, one IoU threshold and ``iou_mode`` 'corner' / 'centre'
+    (``mgd_confusion_update``).  Torch CUDA tensors in ``match_detections``' layout; boxes may be
+    int32 (``decode_nms``' ``boxes_xyxy``).  Enqueued on the current stream; class-range errors
+    surface at the next ``poll_status`` unless ``sync``."""
+    import torch
+    lib = _lib.load()
+    if not (_is_torch(matrix) and matrix.dim() == 3 and matrix.shape[1] == matrix.shape[2] and matrix.shape[1] >= 2):
+        raise ValueError("matrix must be a (Q, C+1, C+1) tensor")
+    C, thr, conf, mode = confusion_config(int(matrix.shape[1]) - 1, iou_threshold, confidences, iou_mode)
+    if matrix.shape[0] != len(conf):
+        raise ValueError(f"matrix holds {matrix.shape[0]} confidences, {len(conf)} given")
+    tensors = (("det_boxes", det_boxes), ("det_scores", det_scores), ("det_classes", det_classes),
+               ("det_counts", det_counts), ("gt_boxes", gt_boxes), ("gt_classes", gt_classes), ("gt_counts", gt_counts))
+    for name, t in tensors:
+        if not _is_torch(t):
+            raise ValueError(f"{name} must be a torch tensor")
+    db, ds, dc, dn, gb, gc, gn = (t for _, t in tensors)
+    if ds.dim() != 2 or tuple(db.shape) != (*ds.shape, 4) or dc.shape != ds.shape or tuple(dn.shape) != (ds.shape[0],):
+        raise ValueError("detections must be det_boxes (B, M, 4), det_scores / det_classes (B, M), det_counts (B,)")
+    B, M = int(ds.shape[0]), int(ds.shape[1])
+    if gc.dim() != 2 or gc.shape[0] != B or tuple(gb.shape) != (*gc.shape, 4) or tuple(gn.shape) != (B,):
+        raise ValueError("ground truth must be gt_boxes (B, N, 4), gt_classes (B, N), gt_counts (B,)")
+    N = int(gc.shape[1])
+    if not (matrix.is_cuda and matrix.dtype == torch.int64 and matrix.is_contiguous()):
+        raise ValueError("matrix must be a contiguous int64 CUDA tensor")
+    dev = matrix.device
+    for name, t in tensors:
+        if t.device != dev:
+            raise ValueError(f"{name} must be a torch tensor on {dev}")
+    f64 = lambda x: x.to(torch.float64).contiguous()
+    i32 = lambda x: x.to(torch.int32).contiguous()
+    db, ds, dc, dn, gb, gc, gn = f64(db), f64(ds), i32(dc), i32(dn), f64(gb), i32(gc), i32(gn)
+    p = lambda x: ctypes.c_void_p(x.data_ptr()) if x.numel() else None
+    idx = dev.index or 0
+    rc = lib.mgd_confusion_update(p(db), p(ds), p(dc), p(dn), B, M, p(gb), p(gc), p(gn), N, C, thr, mode,
+                                  conf.ctypes.data_as(ctypes.POINTER(ctypes.c_double)), len(conf),
+                                  ctypes.c_void_p(matrix.data_ptr()), idx, ctypes.c_void_p(_torch_stream(idx)),
+                                  _lib.FLAG_SYNC if sync else 0)
+    _lib.raise_for_status(rc)
 
 
 def iou_matrix(boxes1, boxes2):

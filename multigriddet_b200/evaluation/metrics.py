@@ -642,3 +642,98 @@ class ShardedMapAccumulator(MapAccumulator):
         if pr:
             res["pr"] = dict(pr, **dict(zip(engine._MAP_PR_TABLES, summed[2:])))
         return res
+
+
+class ConfusionMatrixAccumulator:
+    """Detection confusion matrix at chosen confidences, fed batch by batch with device tensors.
+
+    For each confidence ``confidences[q]`` the detections with ``score >= confidences[q]`` are
+    matched first with the reference's matcher of their own class (``match_predictions_to_gt_cached``
+    with ``iou_mode='corner'``, ``match_predictions_to_gt`` with 'centre'), then the ones left
+    unmatched claim, in the same order, the still-unclaimed ground truth of any class with the
+    highest IoU when it is ``>= iou_threshold`` (``mgd_confusion_update``).  ``compute`` returns a
+    host int64 array ``(Q, C+1, C+1)``: rows are the true class, columns the detected class, as in
+    ``sklearn.metrics.confusion_matrix``, and index C is background -- row C holds the false
+    positives on nothing, column C the missed objects.  The diagonal is the matcher's TP count at
+    that confidence; row g < C sums to the ground truth of class g, column d < C to the class-d
+    detections kept.
+
+    ``confidences=None`` is a single matrix (Q = 1) over every detection passed in; a typical
+    choice is the confidence ``MapAccumulator.compute(precision_recall=True)`` gives in
+    ``best_f1``, or up to 32 of them.  ``iou_mode='centre'`` is there only so that the diagonal
+    agrees with ``calculate_map`` where the reference switches to its un-cached matcher, which reads
+    the xyxy boxes as centre format (more than 10 000 predictions with ``use_parallel``, i.e. every
+    COCO-val-sized run); 'corner' is the correct IoU.
+
+    ``update`` takes ``MapAccumulator.update``'s tensors (``det_boxes`` may be the int32
+    ``boxes_xyxy`` of ``engine.decode_nms``) and only enqueues work on the current stream.  Scores
+    must be finite; ``compute`` raises AssertionError for a class id outside [0, num_classes).
+    """
+
+    def __init__(self, num_classes: int, iou_threshold: float = 0.5, confidences=None, iou_mode: str = "corner",
+                 device=None):
+        self.num_classes, self.iou_threshold, self.confidences, _ = engine.confusion_config(
+            num_classes, iou_threshold, confidences, iou_mode)
+        self.iou_mode = iou_mode
+        import torch
+        self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+        self.reset()
+
+    def reset(self) -> None:
+        """Forget every update."""
+        import torch
+        C1 = self.num_classes + 1
+        self._matrix = torch.zeros((len(self.confidences), C1, C1), dtype=torch.int64, device=self.device)
+
+    def update(self, det_boxes, det_scores, det_classes, det_counts, gt_boxes, gt_classes, gt_counts) -> None:
+        """Add one batch: det_boxes (B, M, 4) xyxy, det_scores (B, M), det_classes (B, M),
+        det_counts (B,), gt_boxes (B, N, 4) xyxy, gt_classes (B, N), gt_counts (B,)."""
+        engine.confusion_update(self._matrix, self.confidences, self.iou_threshold, self.iou_mode, det_boxes,
+                                det_scores, det_classes, det_counts, gt_boxes, gt_classes, gt_counts)
+
+    def compute(self) -> np.ndarray:
+        """The (Q, C+1, C+1) int64 matrices over every update since construction or ``reset``."""
+        engine.poll_status(self.device.index or 0)
+        return self._matrix.cpu().numpy()
+
+
+class ShardedConfusionMatrixAccumulator(ConfusionMatrixAccumulator):
+    """``ConfusionMatrixAccumulator`` over a batch sharded across the ranks of ``group``.
+
+    ``update`` takes this rank's shard (any split of the images, possibly empty) and makes no
+    collective call.  ``compute`` is collective: one int64 all-reduce sums the ranks' matrices (on
+    the device with NCCL, through host memory with any other backend), with one more element for
+    the rank's class-range error, so a rank that saw one still joins the reduce and every rank then
+    raises AssertionError.  Every rank returns the same matrix, equal to the single-process one.
+    Without ``torch.distributed`` or at world size 1 it makes no collective call."""
+
+    def __init__(self, num_classes: int, iou_threshold: float = 0.5, confidences=None, iou_mode: str = "corner",
+                 device=None, group=None):
+        from ..sharding import _dist
+        d = _dist()
+        self.group = group
+        self.world_size = d.get_world_size(group) if d else 1
+        super().__init__(num_classes, iou_threshold, confidences, iou_mode, device)
+
+    def compute(self) -> np.ndarray:
+        """The (Q, C+1, C+1) int64 matrices over every rank's updates (collective)."""
+        import torch
+        from ..sharding import _dist
+        error = None
+        try:
+            engine.poll_status(self.device.index or 0)
+        except AssertionError as e:
+            error = str(e)
+        if self.world_size == 1:
+            if error:
+                raise AssertionError(error)
+            return self._matrix.cpu().numpy()
+        d = _dist()
+        wire = self.device if d.get_backend(self.group) == "nccl" else torch.device("cpu")
+        flat = torch.cat([self._matrix.reshape(-1),
+                          torch.tensor([1 if error else 0], dtype=torch.int64, device=self.device)]).to(wire)
+        d.all_reduce(flat, group=self.group)
+        flat = flat.cpu()
+        if int(flat[-1]):
+            raise AssertionError(error or f"class id outside [0, num_classes) on {int(flat[-1])} other rank(s)")
+        return flat[:-1].reshape(self._matrix.shape).numpy()
