@@ -355,6 +355,39 @@ MGD_API int mgd_map_compute(const mgd_map_config *cfg, const void *records, long
                     long long *det_hist_out, int device, void *stream, int flags);
 
 /*
+ * Average recall at detection limits, the AR@maxDets of pycocotools' COCOeval (its `maxDets`
+ * parameter, (1, 10, 100) by default), applied to this library's matcher: no crowd or ignore
+ * regions, and equal scores ordered later slot first where pycocotools takes the earlier first.
+ *
+ *   mgd_map_recall_update  reads the batch * max_dets records mgd_map_update wrote at slot_offset
+ *                          (enqueue it on the same stream, after that call, with the same cfg,
+ *                          batch and max_dets).  In every view of cfg->views, each record of a
+ *                          real slot gets its rank in its (image, class): the number of that
+ *                          image's records of its class visited before it by the matcher (score
+ *                          descending, equal scores later slot first); in the band views
+ *                          MGD_MAP_VIEW_S / _M / _L only the records in the view's band count.
+ *                          Each true positive at threshold t adds 1 to
+ *                            tp_out[view, class, t, k],  k the first limit with rank < limits[k]
+ *                          and nothing when rank >= limits[num_limits - 1].  The prefix sum over
+ *                          k is the number of true positives among the first limits[k]
+ *                          detections of every (image, class), which is what matching only those
+ *                          detections gives: the greedy walk never looks ahead, so a prefix of it
+ *                          makes the same claims.  Recall at limit k is that sum over
+ *                          gt_hist[view, class].
+ *     limits       num_limits HOST ints in [1, MGD_MAP_MAX_RECALL_LIMITS], each >= 1, strictly
+ *                  increasing
+ *     tp_out       (MGD_MAP_VIEWS, num_classes, num_thresholds, num_limits) int64, device
+ *                  memory, added to (the caller zeroes it once, then sums any number of updates
+ *                  into it)
+ * Device memory only; work is enqueued on `stream`; scratch comes from the calling thread's
+ * workspace (mgd_release_workspace).
+ */
+#define MGD_MAP_MAX_RECALL_LIMITS 8
+MGD_API int mgd_map_recall_update(const mgd_map_config *cfg, const void *records,
+                      long long slot_offset, int batch, int max_dets, const int *limits,
+                      int num_limits, long long *tp_out, int device, void *stream, int flags);
+
+/*
  * Sharded streaming mAP.  Each of `world` ranks runs mgd_map_update on its own shard of every
  * global batch; the APs of a class are then computed on the one rank that owns it.  The result
  * equals mgd_map_compute over the whole data, which orders equal scores of a class later

@@ -26,6 +26,7 @@ BOXES_I32, BOXES_F64 = 0, 1
 
 MAP_MAX_THRESHOLDS, MAP_VOC_POINTS = 32, 11
 MAP_MAX_CONFIDENCES = 32
+MAP_MAX_RECALL_LIMITS = 8
 MAP_COCO, MAP_VOC = 0, 1
 MAP_VIEW_CORNER, MAP_VIEW_CENTRE, MAP_VIEW_S, MAP_VIEW_M, MAP_VIEW_L, MAP_VIEWS = range(6)
 
@@ -112,7 +113,7 @@ EXPORTS = ("mgd_version", "mgd_last_error", "mgd_device_count", "mgd_encode_targ
            "mgd_exchange_buffer", "mgd_exchange_timeouts", "mgd_exchange_destroy",
            "mgd_map_record_bytes", "mgd_map_update", "mgd_map_compute", "mgd_map_partition",
            "mgd_map_compute_merged", "mgd_map_compute_pr", "mgd_map_compute_merged_pr",
-           "mgd_confusion_update")
+           "mgd_confusion_update", "mgd_map_recall_update")
 
 IPC_HANDLE_BYTES = 64
 
@@ -264,6 +265,10 @@ def load():
         ctypes.POINTER(MapConfig), ctypes.c_void_p, ctypes.c_longlong, ctypes.c_void_p, ctypes.c_void_p,
         ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.POINTER(MapPr), ctypes.c_int,
         ctypes.c_void_p, ctypes.c_int]
+    lib.mgd_map_recall_update.restype = ctypes.c_int
+    lib.mgd_map_recall_update.argtypes = [
+        ctypes.POINTER(MapConfig), ctypes.c_void_p, ctypes.c_longlong, ctypes.c_int, ctypes.c_int, _IP,
+        ctypes.c_int, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_int]
     lib.mgd_confusion_update.restype = ctypes.c_int
     lib.mgd_confusion_update.argtypes = [
         ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_int,

@@ -2009,6 +2009,49 @@ int mgd_map_update(const mgd_map_config* cfg, const double* det_boxes, const dou
     return MGD_OK;
 }
 
+int mgd_map_recall_update(const mgd_map_config* cfg, const void* records, long long slot_offset, int batch,
+                          int max_dets, const int* limits, int num_limits, long long* tp_out, int device,
+                          void* stream, int flags)
+{
+    nvtx_range nv_api("mgd_map_recall_update");
+    int rc;
+    if ((rc = check_map_config(cfg))) return rc;
+    if (num_limits < 1 || num_limits > MGD_MAP_MAX_RECALL_LIMITS)
+        return fail(MGD_ERR_INVALID_ARGUMENT, "num_limits must be in [1, %d], got %d",
+                    MGD_MAP_MAX_RECALL_LIMITS, num_limits);
+    if (!limits) return fail(MGD_ERR_INVALID_ARGUMENT, "limits is NULL");
+    for (int k = 0; k < num_limits; ++k)
+        if (limits[k] < 1 || (k > 0 && limits[k] <= limits[k - 1]))
+            return fail(MGD_ERR_INVALID_ARGUMENT, "limits must be >= 1 and strictly increasing");
+    if (batch < 0 || max_dets < 0 || slot_offset < 0)
+        return fail(MGD_ERR_INVALID_ARGUMENT, "batch, max_dets and slot_offset must be >= 0");
+    if (slot_offset + (long long)batch * max_dets > 0x7fffffffll)
+        return fail(MGD_ERR_UNSUPPORTED, "more than 2^31 - 1 detection slots in one evaluation");
+    if (max_dets > 65535) return fail(MGD_ERR_UNSUPPORTED, "max_dets per image must be <= 65535");
+    if ((long long)batch * max_dets > 0 && (!records || !tp_out))
+        return fail(MGD_ERR_INVALID_ARGUMENT, "NULL tensor");
+    int num_sms;
+    DeviceScope dev_scope;
+    if ((rc = prepare_device(device, &num_sms, &dev_scope))) return rc;
+    if ((long long)batch * max_dets == 0) return MGD_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    Arena* ws;
+    if ((rc = map_workspace(device, st, &ws))) return rc;
+    MapRecallArgs a;
+    memset(&a, 0, sizeof(a));
+    CUDA_TRY(ws->take(reinterpret_cast<void**>(&a.next_image), sizeof(int)));
+    CUDA_TRY(cudaMemsetAsync(a.next_image, 0, sizeof(int), st));
+    a.B = batch; a.M = max_dets; a.C = cfg->num_classes; a.T = cfg->num_thresholds; a.K = num_limits;
+    a.views = cfg->views;
+    for (int k = 0; k < num_limits; ++k) a.limits[k] = limits[k];
+    a.recs = static_cast<const MapRec*>(records) + slot_offset;
+    a.tp = reinterpret_cast<unsigned long long*>(tp_out);
+    CUDA_TRY(launch_map_recall(a, num_sms, st));
+    if ((rc = map_workspace_done(device, st))) return rc;
+    if (flags & MGD_FLAG_SYNC) return mgd_poll_status(device, stream);
+    return MGD_OK;
+}
+
 int mgd_map_compute(const mgd_map_config* cfg, const void* records, long long num_slots,
                     const long long* gt_hist, double* ap_out, double* voc_points_out,
                     long long* det_hist_out, int device, void* stream, int flags)

@@ -200,6 +200,17 @@ struct MapWriteArgs {
 };
 cudaError_t launch_map_write(const MapWriteArgs& a, cudaStream_t stream);
 
+// average recall (recall.cu: map_recall_kernel, mgd_map_recall_update): reads one update's
+// records only
+struct MapRecallArgs {
+    int B, M, C, T, K, views;
+    int limits[MGD_MAP_MAX_RECALL_LIMITS];    // strictly increasing, >= 1
+    const MapRec* recs;               // the update's first record, (B, M)
+    unsigned long long* tp;           // (MGD_MAP_VIEWS, C, T, K) counts, added to
+    int* next_image;                  // work counter, zeroed by the caller
+};
+cudaError_t launch_map_recall(const MapRecallArgs& a, int num_sms, cudaStream_t stream);
+
 // scratch of map_compute (bytes), and the enqueue of sort + AP kernels; with `pr` (validated by
 // the caller) also the curves and operating points of mgd_map_compute_pr
 size_t map_compute_scratch_bytes(long long n, int T);

@@ -558,6 +558,48 @@ def map_update(cfg, records, slot_offset, gt_hist, det_boxes, det_scores, det_cl
     _lib.raise_for_status(rc)
 
 
+def recall_limits(max_dets):
+    """Check average-recall detection limits (pycocotools' ``maxDets``) the way
+    ``mgd_map_recall_update`` would, before any device work: 1 to 8 int32 values >= 1, strictly
+    increasing.  Returns them as a tuple of ints."""
+    try:
+        lim = list(max_dets)
+    except TypeError:
+        raise ValueError(f"recall_max_dets must be a sequence of integers, got {max_dets!r}") from None
+    if not 1 <= len(lim) <= _lib.MAP_MAX_RECALL_LIMITS:
+        raise ValueError(f"between 1 and {_lib.MAP_MAX_RECALL_LIMITS} recall limits supported, got {len(lim)}")
+    for k in lim:
+        if isinstance(k, (bool, np.bool_)) or not isinstance(k, (int, np.integer)) or not 1 <= k < 2 ** 31:
+            raise ValueError(f"recall limits must be int32 values >= 1, got {k!r}")
+    if any(b <= a for a, b in zip(lim, lim[1:])):
+        raise ValueError(f"recall limits must be strictly increasing, got {lim}")
+    return tuple(int(k) for k in lim)
+
+
+def map_recall_update(cfg, records, slot_offset, batch, max_dets, limits, tp):
+    """Count the true positives of the ``batch * max_dets`` records ``map_update`` wrote at
+    ``slot_offset`` by their first limit bucket: adds to ``tp`` ((MAP_VIEWS, C, T, K) int64 CUDA
+    tensor) (``mgd_map_recall_update``).  Enqueued on the current stream, behind that
+    ``map_update``."""
+    import torch
+    lib = _lib.load()
+    lim = recall_limits(limits)
+    V, C, T, K = _lib.MAP_VIEWS, cfg.num_classes, cfg.num_thresholds, len(lim)
+    if not (_is_torch(tp) and tp.is_cuda and tp.dtype == torch.int64 and tp.is_contiguous()
+            and tuple(tp.shape) == (V, C, T, K)):
+        raise ValueError(f"tp must be a contiguous int64 CUDA tensor of shape {(V, C, T, K)}")
+    dev = tp.device
+    if not (_is_torch(records) and records.device == dev and records.dtype == torch.uint8
+            and records.numel() >= (slot_offset + batch * max_dets) * map_record_bytes()):
+        raise ValueError(f"records is not a uint8 tensor on {dev} large enough for this update")
+    arr = (ctypes.c_int * K)(*lim)
+    idx = dev.index or 0
+    rc = lib.mgd_map_recall_update(ctypes.byref(cfg), ctypes.c_void_p(records.data_ptr()) if records.numel() else None,
+                                   int(slot_offset), int(batch), int(max_dets), arr, K, ctypes.c_void_p(tp.data_ptr()),
+                                   idx, ctypes.c_void_p(_torch_stream(idx)), 0)
+    _lib.raise_for_status(rc)
+
+
 def map_compute(cfg, records, num_slots, gt_hist):
     """Sort the first ``num_slots`` records and compute every view's per-(class, threshold)
     AP (``mgd_map_compute``).  Returns NumPy ``det_hist`` (MAP_VIEWS, C) int64 and ``ap``

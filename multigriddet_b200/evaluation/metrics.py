@@ -350,6 +350,27 @@ def _precision_recall(pr, view, num_records, gt_hist, confidences) -> Dict[str, 
     return res
 
 
+def _average_recall(tp, gt_hist, view, max_dets, per_scale) -> Dict[str, Any]:
+    """compute()'s average-recall keys from the ``(MAP_VIEWS, C, T, K)`` true positives counted by
+    ``mgd_map_recall_update`` in the first limit bucket above their rank.  ``recall[v, c, t, k]`` is
+    the prefix sum over the buckets over ``gt_hist[v, c]``, -1.0 where that is 0; an AR is its mean
+    over the classes with ground truth and every threshold, 0.0 when no class has any."""
+    gt = np.asarray(gt_hist, dtype=np.int64)[:, :, None, None]
+    cum = np.cumsum(np.asarray(tp, dtype=np.int64), axis=-1)
+    with np.errstate(divide="ignore", invalid="ignore"):
+        recall = np.where(gt > 0, cum / gt, -1.0)
+
+    def mean(v, k):
+        has = gt_hist[v] > 0
+        return float(np.mean(recall[v][has][:, :, k])) if has.any() else 0.0
+    res = {f"AR{m}": mean(view, k) for k, m in enumerate(max_dets)}
+    for key, v in (("ARS", _lib.MAP_VIEW_S), ("ARM", _lib.MAP_VIEW_M), ("ARL", _lib.MAP_VIEW_L)):
+        res[key] = mean(v, len(max_dets) - 1) if per_scale else 0.0
+    res["recall"] = {"max_dets": tuple(max_dets), "matcher": "corner" if view == _lib.MAP_VIEW_CORNER else "centre",
+                     "num_gt": np.array(gt_hist[view]), "recall": recall[view]}
+    return res
+
+
 class MapAccumulator:
     """``calculate_map`` fed batch by batch with device tensors, without the lists of dicts.
 
@@ -368,11 +389,20 @@ class MapAccumulator:
     dispatch, the pin of ``oracle/ref_loader.py``).  Where NumPy dispatches its argsort to
     AVX-512 or AVX2 it orders those ties differently, and ``calculate_map`` itself then gives
     different numbers from one CPU to another.
+
+    ``recall_max_dets`` (e.g. pycocotools' ``(1, 10, 100)``; up to 8 increasing limits) adds
+    COCO-style average recall to every ``compute()`` dict: ``AR{k}`` per limit, ``ARS`` / ``ARM`` /
+    ``ARL`` at the largest limit (0.0 without ``compute_per_scale``, as ``APS`` is), and ``"recall"``
+    (see ``compute``).  It is pycocotools' AR with this matcher: per (image, class) the first k
+    detections by descending score (equal scores: later slot first, where pycocotools takes the
+    earlier first) are kept, and there are no crowd or ignore regions, so the numbers are not
+    pycocotools' own.  It costs one more kernel per ``update``; ``None`` adds nothing.
     """
 
     def __init__(self, num_classes: int, iou_thresholds: List[float] = None, class_names: List[str] = None,
                  method: str = "coco", use_parallel: bool = True, optimize_classes: bool = True,
-                 cache_ious: bool = True, compute_per_scale: bool = True, device=None):
+                 cache_ious: bool = True, compute_per_scale: bool = True, device=None, recall_max_dets=None):
+        self._recall_limits = None if recall_max_dets is None else engine.recall_limits(recall_max_dets)
         if iou_thresholds is None:
             iou_thresholds = list(COCO_THRESHOLDS)
         if class_names is None:
@@ -398,6 +428,9 @@ class MapAccumulator:
         self._records = torch.empty((0,), dtype=torch.uint8, device=self.device)
         self._slots = 0
         self._gt_hist = torch.zeros((_lib.MAP_VIEWS, self._cfg.num_classes), dtype=torch.int64, device=self.device)
+        if self._recall_limits is not None:
+            self._recall_tp = torch.zeros((_lib.MAP_VIEWS, self._cfg.num_classes, self._cfg.num_thresholds,
+                                           len(self._recall_limits)), dtype=torch.int64, device=self.device)
 
     def update(self, det_boxes, det_scores, det_classes, det_counts, gt_boxes, gt_classes, gt_counts) -> None:
         """Add one batch: det_boxes (B, M, 4) xyxy, det_scores (B, M), det_classes (B, M),
@@ -412,6 +445,9 @@ class MapAccumulator:
             self._records = grown
         engine.map_update(self._cfg, self._records, self._slots, self._gt_hist, det_boxes, det_scores,
                           det_classes, det_counts, gt_boxes, gt_classes, gt_counts)
+        if self._recall_limits is not None:
+            engine.map_recall_update(self._cfg, self._records, self._slots, int(det_scores.shape[0]),
+                                     int(det_scores.shape[1]), self._recall_limits, self._recall_tp)
         self._slots += slots
 
     def compute(self, precision_recall: bool = False, confidences=None) -> Dict[str, Any]:
@@ -434,6 +470,14 @@ class MapAccumulator:
         - ``at_confidence`` (C, T, Q, 3), with ``confidences`` (up to 32 finite values): the
           (precision, recall, F1) of the detections with ``score >= confidences[q]``, zeros where
           none is left.  Equal to filtering the detections by that score and evaluating again.
+
+        With ``recall_max_dets`` the dict also holds ``AR{k}``, ``ARS`` / ``ARM`` / ``ARL`` and
+        ``"recall"``: ``max_dets``, ``matcher`` (the main APs' view, as above), ``num_gt`` (C,) and
+        ``recall`` (C, T, K) float64, the true positives among the first ``max_dets[k]`` detections of
+        every (image, class) over ``num_gt``, -1.0 for a class without ground truth.  ``AR{k}`` is
+        the mean of ``recall[..., k]`` over the classes with ground truth and every threshold (0.0
+        if there are none); at a limit >= the detections per image it is the final recall of the
+        curves above.  The band ARs do the same in the area band's view at the largest limit.
         """
         _check_pr_args(precision_recall, confidences)
         if precision_recall:
@@ -441,7 +485,18 @@ class MapAccumulator:
         out = engine.map_compute(self._cfg, self._records, self._slots, self._gt_hist)
         engine.poll_status(self.device.index or 0)
         full = _lib.MAP_VIEW_CORNER if self._args[6] else _lib.MAP_VIEW_CENTRE    # a view always matched
-        return _map_results(_DeviceSource(out, self._gt_hist.cpu().numpy(), full), *self._args)
+        gt = self._gt_hist.cpu().numpy()
+        src = _DeviceSource(out, gt, full)
+        return self._with_recall(_map_results(src, *self._args), src, gt, self._recall_tp_host())
+
+    def _recall_tp_host(self):
+        return None if self._recall_limits is None else self._recall_tp.cpu().numpy()
+
+    def _with_recall(self, res, src, gt, recall_tp) -> Dict[str, Any]:
+        """``res`` with the average-recall keys, in the view ``_map_results`` took its APs from."""
+        if recall_tp is not None:
+            res.update(_average_recall(recall_tp, gt, src.matcher_view, self._recall_limits, self._args[7]))
+        return res
 
     def _compute_pr(self, confidences) -> Dict[str, Any]:
         # the matcher of the main APs is only known from the counts: curves of both full-set views
@@ -454,7 +509,7 @@ class MapAccumulator:
         res = _map_results(src, *self._args)
         n = int(out["det_hist"][src.matcher_view].sum())
         res["precision_recall"] = _precision_recall(out["pr"], src.matcher_view, n, gt, confidences)
-        return res
+        return self._with_recall(res, src, gt, self._recall_tp_host())
 
 
 def global_slot_segments(updates, rank: int, world_size: int):
@@ -514,18 +569,21 @@ class ShardedMapAccumulator(MapAccumulator):
     order, because every record carries its global slot (``global_slot_segments``).  The
     update sequences and the class-range status of all ranks are compared first, so a class id
     out of range raises AssertionError on every rank.  Without ``torch.distributed`` or at world
-    size 1 the same partition and merged compute run without collectives."""
+    size 1 the same partition and merged compute run without collectives.  With
+    ``recall_max_dets`` each rank counts the true positives of its own images by rank, and the
+    counts join the one all-reduce."""
 
     def __init__(self, num_classes: int, iou_thresholds: List[float] = None, class_names: List[str] = None,
                  method: str = "coco", use_parallel: bool = True, optimize_classes: bool = True,
-                 cache_ious: bool = True, compute_per_scale: bool = True, device=None, group=None):
+                 cache_ious: bool = True, compute_per_scale: bool = True, device=None, group=None,
+                 recall_max_dets=None):
         import torch
         from ..sharding import _dist
         d = _dist()
         self.group = group
         self.rank, self.world_size = (d.get_rank(group), d.get_world_size(group)) if d else (0, 1)
         super().__init__(num_classes, iou_thresholds, class_names, method, use_parallel, optimize_classes,
-                         cache_ious, compute_per_scale, device)
+                         cache_ious, compute_per_scale, device, recall_max_dets)
         self._owner = (torch.arange(int(num_classes), device=self.device) % self.world_size).to(torch.int32)
 
     def reset(self) -> None:
@@ -558,7 +616,7 @@ class ShardedMapAccumulator(MapAccumulator):
         collective calls: every rank holds the whole ``best_f1`` / ``best_index`` /
         ``at_confidence`` tables (they join the one all-reduce), while the curves stay on the
         rank that owns the class.  ``owned`` (C,) marks this rank's classes; the other classes
-        have empty curve segments here."""
+        have empty curve segments here.  The average-recall keys are the same on every rank."""
         import torch
         _check_pr_args(precision_recall, confidences)
         error = None
@@ -582,6 +640,8 @@ class ShardedMapAccumulator(MapAccumulator):
                                                _full_views(self._cfg), confidences)
         else:
             out = engine.map_compute_merged(self._cfg, recs, n_recv, gt_hist, self._owner, self.rank)
+        if self._recall_limits is not None:
+            out["recall_tp"] = self._recall_tp
         self._mark("merged")
         if self.world_size > 1:
             out = self._all_reduce(out)
@@ -591,7 +651,7 @@ class ShardedMapAccumulator(MapAccumulator):
         full = _lib.MAP_VIEW_CORNER if self._args[6] else _lib.MAP_VIEW_CENTRE
         gt = gt_hist.cpu().numpy()
         src = _DeviceSource(host, gt, full)
-        res = _map_results(src, *self._args)
+        res = self._with_recall(_map_results(src, *self._args), src, gt, host.pop("recall_tp", None))
         if pr is not None:
             for k in engine._MAP_PR_TABLES:
                 pr[k] = pr[k].cpu().numpy()
@@ -625,22 +685,27 @@ class ShardedMapAccumulator(MapAccumulator):
 
     def _all_reduce(self, out):
         """Sum the ranks' tables: each (view, class) is non-zero on its owner only, so the sums are
-        exact.  One float64 all-reduce; the detection counts and best indices travel as float64
-        (exact below 2^53).  The curves are not sent."""
+        exact.  One float64 all-reduce; the detection counts, best indices and the average-recall
+        counts of each rank's own images travel as float64 (exact below 2^53).  The curves are not
+        sent."""
         import torch
         from ..sharding import _dist
         key = "ap" if "ap" in out else "voc"
         pr = out.get("pr")
-        tables = [out[key], out["det_hist"]] + ([pr[k] for k in engine._MAP_PR_TABLES] if pr else [])
+        recall_tp = out.get("recall_tp")
+        tables = [out[key], out["det_hist"]] + ([recall_tp] if recall_tp is not None else []) + \
+            ([pr[k] for k in engine._MAP_PR_TABLES] if pr else [])
         flat = torch.cat([t.reshape(-1).to(torch.float64) for t in tables]).to(self._wire())
         _dist().all_reduce(flat, group=self.group)
         summed, lo = [], 0
         for t in tables:
             summed.append(flat[lo:lo + t.numel()].to(t.dtype).reshape(t.shape))
             lo += t.numel()
-        res = {key: summed[0], "det_hist": summed[1]}
+        res = {key: summed.pop(0), "det_hist": summed.pop(0)}
+        if recall_tp is not None:
+            res["recall_tp"] = summed.pop(0)
         if pr:
-            res["pr"] = dict(pr, **dict(zip(engine._MAP_PR_TABLES, summed[2:])))
+            res["pr"] = dict(pr, **dict(zip(engine._MAP_PR_TABLES, summed)))
         return res
 
 
