@@ -518,6 +518,60 @@ MGD_API int mgd_confusion_update(const double *det_boxes, const double *det_scor
                       long long *matrix, int device, void *stream, int flags);
 
 /*
+ * TIDE-style detection error analysis (Bolya et al., ECCV 2020) with this project's matcher, at
+ * one positive IoU threshold t_f and one background threshold t_b, 0 < t_b <= t_f <= 1.  Every
+ * IoU below is that of iou_mode (as for mgd_match_detections); every detection is used.
+ *   base   the reference's matcher at t_f (one match_kernel walk, T = 1): its TP flags and claims.
+ *   type   of each detection d the base left unmatched: s = its largest IoU with any ground
+ *          truth of its own class in the image, claimed or not; o = the same over the ground
+ *          truth of every other class; the target is the one attaining s or o (equal IoU: the
+ *          lowest index).  The first rule that applies:
+ *            Bkg   max(s, o) < t_b
+ *            Cls   o >= t_f          target: argmax of o
+ *            Dupe  s >= t_f          (its target was claimed before d's turn)
+ *            Loc   s >= t_b          target: argmax of s
+ *            Both  otherwise (o >= t_b)
+ *   Miss   a ground truth the base left unclaimed that no Cls or Loc error names as target.
+ *   fixes  each applied alone to the base:
+ *            Cls   d takes its target's class; in the visiting order (score descending, equal
+ *                  scores later slot first, over all classes) it becomes a TP and claims the
+ *                  target if nobody holds it yet, else it is dropped
+ *            Loc   the same, keeping d's class
+ *            Both / Dupe / Bkg  those detections are dropped
+ *            Miss  each class's ground-truth count goes down by its Miss count
+ *            FP    every false positive is dropped
+ *            FN    each class's ground-truth count becomes its claimed count
+ *          Claims of the Cls fix and of the Loc fix are separate: each starts from the base's.
+ * Records (mgd_map_record_bytes each): image b of the update owns MGD_TIDE_SETS * max_dets
+ * consecutive records at records + slot_offset + b * MGD_TIDE_SETS * max_dets, one block of
+ * max_dets per set f in the order of enum mgd_tide_set.  A record of set f has class
+ * f * num_classes + c and its TP flag in bit 0 of the MGD_MAP_VIEW_CORNER word; a padding slot or
+ * a detection the set drops has class -1.  So one mgd_map_compute (or the sharded partition +
+ * merged compute) with num_classes' = MGD_TIDE_SETS * num_classes, one threshold and views =
+ * CORNER gives the AP of every class in every set.
+ *   gt_hist   (MGD_MAP_VIEWS, MGD_TIDE_SETS * num_classes) int64, device: the sets' ground-truth
+ *             counts are added to its MGD_MAP_VIEW_CORNER row
+ *   counts    (num_classes, MGD_TIDE_ERRORS) int64, device: errors per class in the order of enum
+ *             mgd_tide_error (a false positive counts under its detection's class, a Miss under
+ *             its ground truth's), added to
+ * Inputs as for mgd_confusion_update.  A class id outside [0, num_classes) on a real slot is
+ * reported as MGD_ERR_CLASS_RANGE through mgd_poll_status (MGD_FLAG_SYNC synchronises and reports
+ * it).  Device memory only; work is enqueued on `stream`; scratch comes from the calling thread's
+ * workspace.
+ */
+enum mgd_tide_set { MGD_TIDE_BASE = 0, MGD_TIDE_FIX_CLS = 1, MGD_TIDE_FIX_LOC = 2, MGD_TIDE_FIX_BOTH = 3,
+                    MGD_TIDE_FIX_DUPE = 4, MGD_TIDE_FIX_BKG = 5, MGD_TIDE_FIX_MISS = 6, MGD_TIDE_FIX_FP = 7,
+                    MGD_TIDE_FIX_FN = 8, MGD_TIDE_SETS = 9 };
+enum mgd_tide_error { MGD_TIDE_CLS = 0, MGD_TIDE_LOC = 1, MGD_TIDE_BOTH = 2, MGD_TIDE_DUPE = 3,
+                      MGD_TIDE_BKG = 4, MGD_TIDE_MISS = 5, MGD_TIDE_ERRORS = 6 };
+MGD_API int mgd_tide_update(const double *det_boxes, const double *det_scores,
+                      const int *det_classes, const int *det_counts, int batch, int max_dets,
+                      const double *gt_boxes, const int *gt_classes, const int *gt_counts, int max_gt,
+                      int num_classes, double pos_threshold, double background_threshold, int iou_mode,
+                      long long slot_offset, void *records, long long *gt_hist, long long *counts,
+                      int device, void *stream, int flags);
+
+/*
  * Loss-side ignore mask.  Replaces MultiGridLoss._compute_ignore_mask and
  * _compute_iou_batch (multigriddet/losses/multigrid_loss.py:494-703, 445-492), called once
  * per layer from the loss (:316).  Forward only: the reference casts the mask from a

@@ -29,6 +29,7 @@ MAP_MAX_CONFIDENCES = 32
 MAP_MAX_RECALL_LIMITS = 8
 MAP_COCO, MAP_VOC = 0, 1
 MAP_VIEW_CORNER, MAP_VIEW_CENTRE, MAP_VIEW_S, MAP_VIEW_M, MAP_VIEW_L, MAP_VIEWS = range(6)
+TIDE_SETS, TIDE_ERRORS = 9, 6          # enum mgd_tide_set / mgd_tide_error
 
 OK, ERR_INVALID_ARGUMENT, ERR_CLASS_RANGE, ERR_CUDA, ERR_NO_DEVICE, ERR_UNSUPPORTED = range(6)
 
@@ -113,7 +114,7 @@ EXPORTS = ("mgd_version", "mgd_last_error", "mgd_device_count", "mgd_encode_targ
            "mgd_exchange_buffer", "mgd_exchange_timeouts", "mgd_exchange_destroy",
            "mgd_map_record_bytes", "mgd_map_update", "mgd_map_compute", "mgd_map_partition",
            "mgd_map_compute_merged", "mgd_map_compute_pr", "mgd_map_compute_merged_pr",
-           "mgd_confusion_update", "mgd_map_recall_update")
+           "mgd_confusion_update", "mgd_map_recall_update", "mgd_tide_update")
 
 IPC_HANDLE_BYTES = 64
 
@@ -274,6 +275,12 @@ def load():
         ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_int,
         ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_double,
         ctypes.c_int, _DP, ctypes.c_int, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_int]
+    lib.mgd_tide_update.restype = ctypes.c_int
+    lib.mgd_tide_update.argtypes = [
+        ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_int,
+        ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_double,
+        ctypes.c_double, ctypes.c_int, ctypes.c_longlong, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
+        ctypes.c_int, ctypes.c_void_p, ctypes.c_int]
     lib.mgd_profile_begin.restype = ctypes.c_int
     lib.mgd_profile_end.restype = ctypes.c_int
     lib.mgd_profile_end.argtypes = [_DP, _LLP]

@@ -403,6 +403,7 @@ int status_to_error(int st)
     if (st & 4) return fail(MGD_ERR_CLASS_RANGE, "mAP update: class id outside [0, num_classes)");
     if (st & 8) return fail(MGD_ERR_INVALID_ARGUMENT, "mAP partition: owner table entry outside [0, world)");
     if (st & 16) return fail(MGD_ERR_CLASS_RANGE, "confusion update: class id outside [0, num_classes)");
+    if (st & 32) return fail(MGD_ERR_CLASS_RANGE, "error analysis update: class id outside [0, num_classes)");
     return MGD_OK;
 }
 
@@ -2310,6 +2311,78 @@ int mgd_confusion_update(const double* det_boxes, const double* det_scores, cons
     c.matrix = reinterpret_cast<unsigned long long*>(matrix);
     c.next_image = counters + 1;
     CUDA_TRY(launch_confusion(c, num_sms, st));
+    if ((rc = map_workspace_done(device, st))) return rc;
+    if (flags & MGD_FLAG_SYNC) return mgd_poll_status(device, stream);
+    return MGD_OK;
+}
+
+int mgd_tide_update(const double* det_boxes, const double* det_scores, const int* det_classes,
+                    const int* det_counts, int batch, int max_dets, const double* gt_boxes,
+                    const int* gt_classes, const int* gt_counts, int max_gt, int num_classes,
+                    double pos_threshold, double background_threshold, int iou_mode, long long slot_offset,
+                    void* records, long long* gt_hist, long long* counts, int device, void* stream, int flags)
+{
+    nvtx_range nv_api("mgd_tide_update");
+    int rc;
+    if (batch < 0 || max_dets < 0 || max_gt < 0 || slot_offset < 0)
+        return fail(MGD_ERR_INVALID_ARGUMENT, "batch, max_dets, max_gt and slot_offset must be >= 0");
+    if (num_classes < 1) return fail(MGD_ERR_INVALID_ARGUMENT, "num_classes must be >= 1, got %d", num_classes);
+    if ((long long)num_classes * MGD_TIDE_SETS > 0x7fffffffll)
+        return fail(MGD_ERR_UNSUPPORTED, "num_classes * %d must fit an int32", (int)MGD_TIDE_SETS);
+    if (!(pos_threshold > 0.0 && pos_threshold <= 1.0))
+        return fail(MGD_ERR_INVALID_ARGUMENT, "pos_threshold must be in (0, 1], got %g", pos_threshold);
+    if (!(background_threshold > 0.0 && background_threshold <= pos_threshold))
+        return fail(MGD_ERR_INVALID_ARGUMENT, "background_threshold must be in (0, pos_threshold], got %g",
+                    background_threshold);
+    if (iou_mode != MGD_IOU_CORNER && iou_mode != MGD_IOU_CENTRE)
+        return fail(MGD_ERR_INVALID_ARGUMENT, "iou_mode must be MGD_IOU_CORNER or MGD_IOU_CENTRE");
+    if (slot_offset + (long long)batch * max_dets * MGD_TIDE_SETS > 0x7fffffffll)
+        return fail(MGD_ERR_UNSUPPORTED, "more than 2^31 - 1 record slots in one evaluation");
+    if (max_dets > 65535) return fail(MGD_ERR_UNSUPPORTED, "max_dets per image must be <= 65535");
+    // per warp: the visiting order and three claimed bitmaps
+    if ((size_t)max_dets * 2 + (size_t)max_gt * 3 / 8 > 48 * 1024)
+        return fail(MGD_ERR_UNSUPPORTED, "max_dets / max_gt too large for one warp's shared memory");
+    if (batch > 0 && (!det_counts || !gt_counts || !gt_hist || !counts))
+        return fail(MGD_ERR_INVALID_ARGUMENT, "NULL tensor");
+    if ((long long)batch * max_dets > 0 && (!det_boxes || !det_scores || !det_classes || !records))
+        return fail(MGD_ERR_INVALID_ARGUMENT, "NULL detection tensor");
+    if ((long long)batch * max_gt > 0 && (!gt_boxes || !gt_classes))
+        return fail(MGD_ERR_INVALID_ARGUMENT, "NULL ground-truth tensor");
+    int num_sms;
+    DeviceScope dev_scope;
+    if ((rc = prepare_device(device, &num_sms, &dev_scope))) return rc;
+    if (batch == 0) return MGD_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    TideArgs t;
+    memset(&t, 0, sizeof(t));
+    if ((rc = deferred_status_word(device, &t.status))) return rc;
+    Arena* ws;
+    if ((rc = map_workspace(device, st, &ws))) return rc;
+    const size_t slots = (size_t)batch * max_dets;
+    int* counters;
+    CUDA_TRY(ws->take(reinterpret_cast<void**>(&counters), 2 * sizeof(int)));
+    CUDA_TRY(cudaMemsetAsync(counters, 0, 2 * sizeof(int), st));
+    // the base: the reference's matcher, once, at pos_threshold
+    MatchArgs m;
+    memset(&m, 0, sizeof(m));
+    m.B = batch; m.M = max_dets; m.N = max_gt; m.T = 1; m.thr[0] = pos_threshold; m.mode = iou_mode;
+    m.det_boxes = det_boxes; m.det_scores = det_scores; m.det_classes = det_classes; m.det_counts = det_counts;
+    m.gt_boxes = gt_boxes; m.gt_classes = gt_classes; m.gt_counts = gt_counts;
+    CUDA_TRY(ws->take(reinterpret_cast<void**>(&m.matched), slots * sizeof(int)));
+    CUDA_TRY(ws->take(reinterpret_cast<void**>(&m.tp), slots));
+    m.next_image = counters;
+    if (slots) CUDA_TRY(launch_match(m, num_sms, st));
+    // error types, fixed records and counts
+    t.B = batch; t.M = max_dets; t.N = max_gt; t.C = num_classes; t.mode = iou_mode;
+    t.t_f = pos_threshold; t.t_b = background_threshold;
+    t.det_boxes = det_boxes; t.det_scores = det_scores; t.det_classes = det_classes; t.det_counts = det_counts;
+    t.gt_boxes = gt_boxes; t.gt_classes = gt_classes; t.gt_counts = gt_counts;
+    t.matched = m.matched;
+    t.recs = static_cast<MapRec*>(records) + slot_offset;
+    t.gt_hist = reinterpret_cast<unsigned long long*>(gt_hist) + (size_t)MGD_MAP_VIEW_CORNER * MGD_TIDE_SETS * num_classes;
+    t.counts = reinterpret_cast<unsigned long long*>(counts);
+    t.next_image = counters + 1;
+    CUDA_TRY(launch_tide(t, num_sms, st));
     if ((rc = map_workspace_done(device, st))) return rc;
     if (flags & MGD_FLAG_SYNC) return mgd_poll_status(device, stream);
     return MGD_OK;

@@ -211,6 +211,24 @@ struct MapRecallArgs {
 };
 cudaError_t launch_map_recall(const MapRecallArgs& a, int num_sms, cudaStream_t stream);
 
+// ---- detection error analysis (match.cu: tide_kernel, mgd_tide_update) -------------------
+// The base is one match_kernel walk at t_f (T = 1, no band); tide_kernel types the false positives
+// and misses and writes the records of every fixed set.
+struct TideArgs {
+    int B, M, N, C;
+    int mode;                         // MGD_IOU_CORNER / MGD_IOU_CENTRE, as for the base walk
+    double t_f, t_b;
+    const double* det_boxes; const double* det_scores; const int* det_classes; const int* det_counts;
+    const double* gt_boxes; const int* gt_classes; const int* gt_counts;
+    const int* matched;               // (B, M) base claim of each detection, -1 = none
+    MapRec* recs;                     // the update's first record: (B, MGD_TIDE_SETS, M)
+    unsigned long long* gt_hist;      // (MGD_TIDE_SETS * C) the CORNER row, added to
+    unsigned long long* counts;       // (C, MGD_TIDE_ERRORS), added to
+    int* next_image;                  // work counter, zeroed by the caller
+    int* status;                      // bit 5: class id outside [0, C)
+};
+cudaError_t launch_tide(const TideArgs& a, int num_sms, cudaStream_t stream);
+
 // scratch of map_compute (bytes), and the enqueue of sort + AP kernels; with `pr` (validated by
 // the caller) also the curves and operating points of mgd_map_compute_pr
 size_t map_compute_scratch_bytes(long long n, int T);

@@ -14,7 +14,8 @@
 // decides identically.  An optional area band (MatchArgs::band) restricts the walk to the
 // boxes calculate_map's per-scale filter keeps, which is the filtered lists' result: their
 // relative visiting order and ground-truth index order are those of the full lists.
-// confusion_kernel extends one such walk with a cross-class stage (mgd_confusion_update).
+// confusion_kernel extends one such walk with a cross-class stage (mgd_confusion_update), and
+// tide_kernel types its errors and writes the error-fixed record sets (mgd_tide_update).
 #include <math.h>
 #include "common.cuh"
 
@@ -273,6 +274,158 @@ confusion_kernel(const __grid_constant__ ConfusionArgs a)
     }
 }
 
+// Detection error analysis (mgd_tide_update), one warp per image, after the base walk at t_f
+// (a.matched).  The visiting order and the base's claimed bitmap are confusion_kernel's; two more
+// bitmaps hold the claims of the Cls fix and of the Loc fix, each starting from the base's.  The
+// detections are taken in visiting order: a TP keeps its record in every set; a false positive is
+// typed from its best same-class IoU s and best other-class IoU o over every ground truth of the
+// image (claimed or not, so the type does not depend on the order), and only the Cls / Loc claims
+// do.  A ground truth named by a Cls or Loc error lies in that fix's bitmap afterwards (claimed by
+// that error or by an earlier one of the same type), so Miss = in none of the three bitmaps.
+// Record of set f: class f * C + c, TP flag in bits[MGD_MAP_VIEW_CORNER] bit 0; dropped: class -1.
+__global__ void __launch_bounds__(kMatchWarps * 32)
+tide_kernel(const __grid_constant__ TideArgs a)
+{
+    extern __shared__ __align__(16) unsigned char dyn[];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int words = (a.N + 31) / 32;
+    const size_t per_warp = (size_t)a.M * 2 + (size_t)words * 12 + 16;
+    unsigned short* order = reinterpret_cast<unsigned short*>(dyn + warp * ((per_warp + 15) & ~(size_t)15));
+    unsigned* taken = reinterpret_cast<unsigned*>(order + ((a.M + 1) & ~1));   // base claims
+    unsigned* fix_cls = taken + words;                                         // Cls fix claims
+    unsigned* fix_loc = fix_cls + words;                                       // Loc fix claims
+
+    for (;;) {
+        int b = 0;
+        if (lane == 0) b = atomicAdd(a.next_image, 1);
+        b = __shfl_sync(0xffffffffu, b, 0);
+        if (b >= a.B) break;
+        const int n = min(max(a.det_counts[b], 0), a.M);
+        const int g = min(max(a.gt_counts[b], 0), a.N);
+        const double* dbox = a.det_boxes + (size_t)b * a.M * 4;
+        const double* dsc = a.det_scores + (size_t)b * a.M;
+        const int* dcl = a.det_classes + (size_t)b * a.M;
+        const double* gbox = a.gt_boxes + (size_t)b * a.N * 4;
+        const int* gcl = a.gt_classes + (size_t)b * a.N;
+        const int* who = a.matched + (size_t)b * a.M;
+        MapRec* recs = a.recs + (size_t)b * MGD_TIDE_SETS * a.M;
+
+        bool bad = false;
+        for (int i = lane; i < n; i += 32) bad |= (unsigned)dcl[i] >= (unsigned)a.C;
+        for (int j = lane; j < g; j += 32) bad |= (unsigned)gcl[j] >= (unsigned)a.C;
+        if (__any_sync(0xffffffffu, bad) && lane == 0) atomicOr(a.status, 32);
+
+        // match_kernel's visiting order: score descending, equal scores later slot first
+        for (int i = lane; i < n; i += 32) {
+            const double si = dsc[i];
+            int rank = 0;
+            for (int j = 0; j < n; ++j) {
+                const double sj = dsc[j];
+                rank += (sj > si) || (sj == si && j > i);
+            }
+            order[rank] = (unsigned short)i;
+        }
+        for (int w = lane; w < 3 * words; w += 32) taken[w] = 0u;
+        __syncwarp();
+        for (int i = lane; i < n; i += 32) {
+            const int j = who[i];
+            if (j >= 0) atomicOr(&taken[j >> 5], 1u << (j & 31));
+        }
+        __syncwarp();
+        for (int w = lane; w < words; w += 32) fix_cls[w] = fix_loc[w] = taken[w];
+        // padding slots: class -1 in every set
+        for (int k = lane; k < (a.M - n) * MGD_TIDE_SETS; k += 32) {
+            const int f = k / (a.M - n), i = n + k % (a.M - n);
+            MapRec r;
+            r.score = dsc[i]; r.cls = -1; r.band = 3; r.pad = 0u;
+            for (int v = 0; v < MGD_MAP_VIEWS; ++v) r.bits[v] = 0u;
+            recs[(size_t)f * a.M + i] = r;
+        }
+        __syncwarp();
+
+        for (int k = 0; k < n; ++k) {
+            const int d = order[k];
+            const int c = dcl[d];
+            const bool ok = (unsigned)c < (unsigned)a.C;
+            // kind: -1 TP, else the mgd_tide_error type; to: the target's class (Cls fix) or c
+            int kind = -1, fixed = -1;
+            if (who[d] < 0) {
+                const double p[4] = {dbox[4 * d], dbox[4 * d + 1], dbox[4 * d + 2], dbox[4 * d + 3]};
+                double s = 0.0, o = 0.0;
+                int sj = -1, oj = -1;
+                for (int j = lane; j < g; j += 32) {
+                    const double q[4] = {gbox[4 * j], gbox[4 * j + 1], gbox[4 * j + 2], gbox[4 * j + 3]};
+                    const double v = a.mode ? iou_centre(p, q) : iou_corner(p, q);
+                    if (gcl[j] == c) { if (v > s) { s = v; sj = j; } }
+                    else if (v > o) { o = v; oj = j; }
+                }
+                #pragma unroll
+                for (int w = 16; w > 0; w >>= 1) {
+                    const double os = __shfl_xor_sync(0xffffffffu, s, w);
+                    const int osj = __shfl_xor_sync(0xffffffffu, sj, w);
+                    const double oo = __shfl_xor_sync(0xffffffffu, o, w);
+                    const int ooj = __shfl_xor_sync(0xffffffffu, oj, w);
+                    if (osj >= 0 && (sj < 0 || os > s || (os == s && osj < sj))) { s = os; sj = osj; }
+                    if (ooj >= 0 && (oj < 0 || oo > o || (oo == o && ooj < oj))) { o = oo; oj = ooj; }
+                }
+                // every lane holds the same s, o and targets
+                int target = -1;
+                unsigned* fix = nullptr;
+                if (fmax(s, o) < a.t_b) kind = MGD_TIDE_BKG;
+                else if (o >= a.t_f) { kind = MGD_TIDE_CLS; target = oj; fix = fix_cls; }
+                else if (s >= a.t_f) kind = MGD_TIDE_DUPE;
+                else if (s >= a.t_b) { kind = MGD_TIDE_LOC; target = sj; fix = fix_loc; }
+                else kind = MGD_TIDE_BOTH;
+                if (fix) {
+                    const int tc = kind == MGD_TIDE_CLS ? gcl[target] : c;
+                    if (!((fix[target >> 5] >> (target & 31)) & 1u) && (unsigned)tc < (unsigned)a.C) fixed = tc;
+                    __syncwarp();
+                    if (lane == 0 && fixed >= 0) fix[target >> 5] |= 1u << (target & 31);
+                    __syncwarp();
+                }
+                if (lane == 0 && ok) atomicAdd(a.counts + (size_t)c * MGD_TIDE_ERRORS + kind, 1ull);
+            }
+            // lane f writes set f's record
+            if (lane < MGD_TIDE_SETS) {
+                const int f = lane;
+                int cls = c, tp = kind < 0;
+                if (kind >= 0) {
+                    if (f == MGD_TIDE_FIX_FP) cls = -1;
+                    else if (f == MGD_TIDE_FIX_CLS && kind == MGD_TIDE_CLS) { cls = fixed; tp = 1; }
+                    else if (f == MGD_TIDE_FIX_LOC && kind == MGD_TIDE_LOC) { cls = fixed; tp = 1; }
+                    else if ((f == MGD_TIDE_FIX_BOTH && kind == MGD_TIDE_BOTH) ||
+                             (f == MGD_TIDE_FIX_DUPE && kind == MGD_TIDE_DUPE) ||
+                             (f == MGD_TIDE_FIX_BKG && kind == MGD_TIDE_BKG)) cls = -1;
+                }
+                MapRec r;
+                r.score = dsc[d];
+                r.cls = ok && cls >= 0 ? f * a.C + cls : -1;
+                r.band = r.cls >= 0 ? map_area_band(dbox + 4 * d) : 3;
+                r.pad = 0u;
+                for (int v = 0; v < MGD_MAP_VIEWS; ++v) r.bits[v] = 0u;
+                r.bits[MGD_MAP_VIEW_CORNER] = r.cls >= 0 ? (unsigned)tp : 0u;
+                recs[(size_t)f * a.M + d] = r;
+            }
+        }
+        __syncwarp();
+
+        // ground-truth counts of every set, and the misses
+        for (int j = lane; j < g; j += 32) {
+            const int c = gcl[j];
+            if ((unsigned)c >= (unsigned)a.C) continue;
+            const unsigned bit = 1u << (j & 31);
+            const bool claimed = taken[j >> 5] & bit;
+            const bool miss = !claimed && !(fix_cls[j >> 5] & bit) && !(fix_loc[j >> 5] & bit);
+            for (int f = 0; f < MGD_TIDE_SETS; ++f) {
+                if ((f == MGD_TIDE_FIX_MISS && miss) || (f == MGD_TIDE_FIX_FN && !claimed)) continue;
+                atomicAdd(a.gt_hist + f * (long long)a.C + c, 1ull);
+            }
+            if (miss) atomicAdd(a.counts + (size_t)c * MGD_TIDE_ERRORS + MGD_TIDE_MISS, 1ull);
+        }
+        __syncwarp();
+    }
+}
+
 __global__ void iou_matrix_kernel(const double* b1, int n, const double* b2, int m, double* out)
 {
     const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -310,6 +463,21 @@ cudaError_t launch_confusion(const ConfusionArgs& a, int num_sms, cudaStream_t s
     if (grid < 1) grid = 1;
     prof_mark_begin(PROF_OTHER, stream);
     confusion_kernel<<<(unsigned)grid, kMatchWarps * 32, smem, stream>>>(a);
+    prof_mark_end(PROF_OTHER, stream);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_tide(const TideArgs& a, int num_sms, cudaStream_t stream)
+{
+    const size_t per_warp = ((size_t)a.M * 2 + (size_t)((a.N + 31) / 32) * 12 + 16 + 15) & ~(size_t)15;
+    const size_t smem = per_warp * kMatchWarps;
+    cudaError_t e = cudaFuncSetAttribute(tide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    long long grid = ((long long)a.B + kMatchWarps - 1) / kMatchWarps;
+    if (grid > (long long)num_sms * 8) grid = (long long)num_sms * 8;
+    if (grid < 1) grid = 1;
+    prof_mark_begin(PROF_OTHER, stream);
+    tide_kernel<<<(unsigned)grid, kMatchWarps * 32, smem, stream>>>(a);
     prof_mark_end(PROF_OTHER, stream);
     return cudaGetLastError();
 }

@@ -881,6 +881,73 @@ def confusion_update(matrix, confidences, iou_threshold, iou_mode, det_boxes, de
     _lib.raise_for_status(rc)
 
 
+def tide_config(num_classes, pos_threshold=0.5, background_threshold=0.1, iou_mode="corner"):
+    """Check the settings of an error analysis the way ``mgd_tide_update`` would, before any device
+    work.  Returns ``(num_classes, pos_threshold, background_threshold, iou_mode code)``."""
+    if isinstance(num_classes, bool) or int(num_classes) != num_classes or int(num_classes) < 1:
+        raise ValueError(f"num_classes must be an integer >= 1, got {num_classes}")
+    if int(num_classes) * _lib.TIDE_SETS > 2 ** 31 - 1:
+        raise ValueError(f"num_classes must be below 2^31 / {_lib.TIDE_SETS}, got {num_classes}")
+    t_f, t_b = float(pos_threshold), float(background_threshold)
+    if not 0.0 < t_f <= 1.0:
+        raise ValueError(f"pos_threshold must be in (0, 1], got {pos_threshold}")
+    if not 0.0 < t_b <= t_f:
+        raise ValueError(f"background_threshold must be in (0, pos_threshold], got {background_threshold}")
+    if iou_mode not in _IOU_MODES:
+        raise ValueError(f"iou_mode must be 'corner' or 'centre', got {iou_mode!r}")
+    return int(num_classes), t_f, t_b, _IOU_MODES[iou_mode]
+
+
+def tide_update(records, slot_offset, gt_hist, counts, pos_threshold, background_threshold, iou_mode,
+                det_boxes, det_scores, det_classes, det_counts, gt_boxes, gt_classes, gt_counts, sync=False):
+    """Type one batch's errors and write the records of every error-fixed set (``mgd_tide_update``):
+    ``TIDE_SETS * B * M`` records at ``slot_offset`` of ``records`` (a CUDA byte tensor), image by
+    image, one block of M per set; the sets' ground-truth counts are added to the MAP_VIEW_CORNER row
+    of ``gt_hist`` ((MAP_VIEWS, TIDE_SETS * C) int64) and the error counts to ``counts`` ((C,
+    TIDE_ERRORS) int64).  Torch CUDA tensors in ``match_detections``' layout; boxes may be int32
+    (``decode_nms``' ``boxes_xyxy``).  Enqueued on the current stream; class-range errors surface at
+    the next ``poll_status`` unless ``sync``."""
+    import torch
+    lib = _lib.load()
+    if not (_is_torch(counts) and counts.dim() == 2 and counts.shape[1] == _lib.TIDE_ERRORS):
+        raise ValueError(f"counts must be a (C, {_lib.TIDE_ERRORS}) tensor")
+    C, t_f, t_b, mode = tide_config(int(counts.shape[0]), pos_threshold, background_threshold, iou_mode)
+    tensors = (("det_boxes", det_boxes), ("det_scores", det_scores), ("det_classes", det_classes),
+               ("det_counts", det_counts), ("gt_boxes", gt_boxes), ("gt_classes", gt_classes), ("gt_counts", gt_counts))
+    for name, t in tensors:
+        if not _is_torch(t):
+            raise ValueError(f"{name} must be a torch tensor")
+    db, ds, dc, dn, gb, gc, gn = (t for _, t in tensors)
+    if ds.dim() != 2 or tuple(db.shape) != (*ds.shape, 4) or dc.shape != ds.shape or tuple(dn.shape) != (ds.shape[0],):
+        raise ValueError("detections must be det_boxes (B, M, 4), det_scores / det_classes (B, M), det_counts (B,)")
+    B, M = int(ds.shape[0]), int(ds.shape[1])
+    if gc.dim() != 2 or gc.shape[0] != B or tuple(gb.shape) != (*gc.shape, 4) or tuple(gn.shape) != (B,):
+        raise ValueError("ground truth must be gt_boxes (B, N, 4), gt_classes (B, N), gt_counts (B,)")
+    N = int(gc.shape[1])
+    if not (counts.is_cuda and counts.dtype == torch.int64 and counts.is_contiguous()):
+        raise ValueError("counts must be a contiguous int64 CUDA tensor")
+    dev = counts.device
+    if not (_is_torch(gt_hist) and gt_hist.device == dev and gt_hist.dtype == torch.int64 and gt_hist.is_contiguous()
+            and tuple(gt_hist.shape) == (_lib.MAP_VIEWS, _lib.TIDE_SETS * C)):
+        raise ValueError(f"gt_hist must be a contiguous ({_lib.MAP_VIEWS}, {_lib.TIDE_SETS * C}) int64 tensor on {dev}")
+    slot_offset = int(slot_offset)
+    if not (_is_torch(records) and records.device == dev and records.dtype == torch.uint8 and slot_offset >= 0
+            and records.numel() >= (slot_offset + _lib.TIDE_SETS * B * M) * map_record_bytes()):
+        raise ValueError(f"records is not a uint8 tensor on {dev} large enough for this update")
+    for name, t in tensors:
+        if t.device != dev:
+            raise ValueError(f"{name} must be a torch tensor on {dev}")
+    f64 = lambda x: x.to(torch.float64).contiguous()
+    i32 = lambda x: x.to(torch.int32).contiguous()
+    db, ds, dc, dn, gb, gc, gn = f64(db), f64(ds), i32(dc), i32(dn), f64(gb), i32(gc), i32(gn)
+    p = lambda x: ctypes.c_void_p(x.data_ptr()) if x.numel() else None
+    idx = dev.index or 0
+    rc = lib.mgd_tide_update(p(db), p(ds), p(dc), p(dn), B, M, p(gb), p(gc), p(gn), N, C, t_f, t_b, mode,
+                             slot_offset, p(records), p(gt_hist), p(counts), idx, ctypes.c_void_p(_torch_stream(idx)),
+                             _lib.FLAG_SYNC if sync else 0)
+    _lib.raise_for_status(rc)
+
+
 def iou_matrix(boxes1, boxes2):
     """(n, m) float64 IoU matrix of xyxy boxes (``mgd_iou_matrix``), NumPy in / out."""
     lib = _lib.load()

@@ -435,20 +435,24 @@ class MapAccumulator:
     def update(self, det_boxes, det_scores, det_classes, det_counts, gt_boxes, gt_classes, gt_counts) -> None:
         """Add one batch: det_boxes (B, M, 4) xyxy, det_scores (B, M), det_classes (B, M),
         det_counts (B,), gt_boxes (B, N, 4) xyxy, gt_classes (B, N), gt_counts (B,)."""
-        import torch
         slots = int(det_scores.shape[0]) * int(det_scores.shape[1])
-        need = (self._slots + slots) * self._record_bytes
-        if need > self._records.numel():              # grow by doubling, on the stream
-            grown = torch.empty((max(need, 2 * self._records.numel()),), dtype=torch.uint8, device=self.device)
-            used = self._slots * self._record_bytes
-            grown[:used].copy_(self._records[:used])
-            self._records = grown
+        self._reserve(slots)
         engine.map_update(self._cfg, self._records, self._slots, self._gt_hist, det_boxes, det_scores,
                           det_classes, det_counts, gt_boxes, gt_classes, gt_counts)
         if self._recall_limits is not None:
             engine.map_recall_update(self._cfg, self._records, self._slots, int(det_scores.shape[0]),
                                      int(det_scores.shape[1]), self._recall_limits, self._recall_tp)
         self._slots += slots
+
+    def _reserve(self, slots: int) -> None:
+        """Room for ``slots`` more records behind the used ones (grown by doubling, on the stream)."""
+        import torch
+        need = (self._slots + slots) * self._record_bytes
+        if need > self._records.numel():
+            grown = torch.empty((max(need, 2 * self._records.numel()),), dtype=torch.uint8, device=self.device)
+            used = self._slots * self._record_bytes
+            grown[:used].copy_(self._records[:used])
+            self._records = grown
 
     def compute(self, precision_recall: bool = False, confidences=None) -> Dict[str, Any]:
         """``calculate_map``'s result dict over every update since construction or ``reset``.
@@ -596,14 +600,18 @@ class ShardedMapAccumulator(MapAccumulator):
         """Add this rank's shard of a global batch of ``n_total`` images (default: the local batch
         times the world size).  The shard must be the one ``shard_bounds(n_total)`` gives this
         rank, possibly empty (a (0, M) / (0, N) batch), with the same M on every rank."""
+        n_total = self._shard_total(int(det_scores.shape[0]), n_total)
+        super().update(det_boxes, det_scores, det_classes, det_counts, gt_boxes, gt_classes, gt_counts)
+        self._updates.append((n_total, int(det_scores.shape[1])))
+
+    def _shard_total(self, n_local: int, n_total) -> int:
+        """``n_total`` (default: ``n_local`` times the world size), checked against this rank's shard."""
         from ..sharding import shard_bounds
-        n_local = int(det_scores.shape[0])
         n_total = n_local * self.world_size if n_total is None else int(n_total)
         lo, hi = shard_bounds(n_total, self.rank, self.world_size)
         if hi - lo != n_local:
             raise ValueError(f"rank {self.rank} holds {n_local} images, shard_bounds({n_total}) says {hi - lo}")
-        super().update(det_boxes, det_scores, det_classes, det_counts, gt_boxes, gt_classes, gt_counts)
-        self._updates.append((n_total, int(det_scores.shape[1])))
+        return n_total
 
     def _mark(self, phase: str) -> None:
         """Called as each phase of ``compute`` has been enqueued ('check', 'partition', 'exchange',
@@ -617,8 +625,29 @@ class ShardedMapAccumulator(MapAccumulator):
         ``at_confidence`` tables (they join the one all-reduce), while the curves stay on the
         rank that owns the class.  ``owned`` (C,) marks this rank's classes; the other classes
         have empty curve segments here.  The average-recall keys are the same on every rank."""
-        import torch
         _check_pr_args(precision_recall, confidences)
+        host, gt, pr = self._merged_tables(precision_recall, confidences)
+        full = _lib.MAP_VIEW_CORNER if self._args[6] else _lib.MAP_VIEW_CENTRE
+        src = _DeviceSource(host, gt, full)
+        res = self._with_recall(_map_results(src, *self._args), src, gt, host.pop("recall_tp", None))
+        if pr is not None:
+            for k in engine._MAP_PR_TABLES:
+                pr[k] = pr[k].cpu().numpy()
+            owned = (self._owner == self.rank).cpu().numpy()
+            n = int(host["det_hist"][src.matcher_view][owned].sum())     # this rank's records
+            res["precision_recall"] = _precision_recall(pr, src.matcher_view, n, gt, confidences)
+            res["precision_recall"]["owned"] = owned
+        return res
+
+    def _rank_counts(self):
+        """Counts of this rank's own images that the all-reduce sums, by name (int64 CUDA tensors)."""
+        return {} if self._recall_limits is None else {"recall_tp": self._recall_tp}
+
+    def _merged_tables(self, precision_recall: bool = False, confidences=None):
+        """The collective part of ``compute``: the update check, the record exchange, the merged
+        compute and the all-reduce.  Returns the summed tables as NumPy arrays (``det_hist``, ``ap``
+        or ``voc``, and every ``_rank_counts`` entry), the summed ground-truth counts (NumPy) and
+        the curve outputs (or None)."""
         error = None
         try:
             engine.poll_status(self.device.index or 0)
@@ -640,26 +669,14 @@ class ShardedMapAccumulator(MapAccumulator):
                                                _full_views(self._cfg), confidences)
         else:
             out = engine.map_compute_merged(self._cfg, recs, n_recv, gt_hist, self._owner, self.rank)
-        if self._recall_limits is not None:
-            out["recall_tp"] = self._recall_tp
+        out.update(self._rank_counts())
         self._mark("merged")
         if self.world_size > 1:
             out = self._all_reduce(out)
         pr = out.pop("pr", None)
         host = {k: v.cpu().numpy() for k, v in out.items()}
         self._mark("reduce")
-        full = _lib.MAP_VIEW_CORNER if self._args[6] else _lib.MAP_VIEW_CENTRE
-        gt = gt_hist.cpu().numpy()
-        src = _DeviceSource(host, gt, full)
-        res = self._with_recall(_map_results(src, *self._args), src, gt, host.pop("recall_tp", None))
-        if pr is not None:
-            for k in engine._MAP_PR_TABLES:
-                pr[k] = pr[k].cpu().numpy()
-            owned = (self._owner == self.rank).cpu().numpy()
-            n = int(host["det_hist"][src.matcher_view][owned].sum())     # this rank's records
-            res["precision_recall"] = _precision_recall(pr, src.matcher_view, n, gt, confidences)
-            res["precision_recall"]["owned"] = owned
-        return res
+        return host, gt_hist.cpu().numpy(), pr
 
     def _wire(self):
         """Where the collectives' tensors live: the device with NCCL, host memory otherwise."""
@@ -685,15 +702,15 @@ class ShardedMapAccumulator(MapAccumulator):
 
     def _all_reduce(self, out):
         """Sum the ranks' tables: each (view, class) is non-zero on its owner only, so the sums are
-        exact.  One float64 all-reduce; the detection counts, best indices and the average-recall
-        counts of each rank's own images travel as float64 (exact below 2^53).  The curves are not
-        sent."""
+        exact.  One float64 all-reduce; the detection counts, best indices and the counts of each
+        rank's own images (``_rank_counts``) travel as float64 (exact below 2^53).  The curves are
+        not sent."""
         import torch
         from ..sharding import _dist
         key = "ap" if "ap" in out else "voc"
         pr = out.get("pr")
-        recall_tp = out.get("recall_tp")
-        tables = [out[key], out["det_hist"]] + ([recall_tp] if recall_tp is not None else []) + \
+        counts = [k for k in out if k not in (key, "det_hist", "pr")]
+        tables = [out[key], out["det_hist"]] + [out[k] for k in counts] + \
             ([pr[k] for k in engine._MAP_PR_TABLES] if pr else [])
         flat = torch.cat([t.reshape(-1).to(torch.float64) for t in tables]).to(self._wire())
         _dist().all_reduce(flat, group=self.group)
@@ -702,8 +719,8 @@ class ShardedMapAccumulator(MapAccumulator):
             summed.append(flat[lo:lo + t.numel()].to(t.dtype).reshape(t.shape))
             lo += t.numel()
         res = {key: summed.pop(0), "det_hist": summed.pop(0)}
-        if recall_tp is not None:
-            res["recall_tp"] = summed.pop(0)
+        for k in counts:
+            res[k] = summed.pop(0)
         if pr:
             res["pr"] = dict(pr, **dict(zip(engine._MAP_PR_TABLES, summed)))
         return res
@@ -802,3 +819,144 @@ class ShardedConfusionMatrixAccumulator(ConfusionMatrixAccumulator):
         if int(flat[-1]):
             raise AssertionError(error or f"class id outside [0, num_classes) on {int(flat[-1])} other rank(s)")
         return flat[:-1].reshape(self._matrix.shape).numpy()
+
+
+TIDE_FIXES = ("Cls", "Loc", "Both", "Dupe", "Bkg", "Miss", "FP", "FN")     # record sets 1 .. 8
+TIDE_ERRORS = ("Cls", "Loc", "Both", "Dupe", "Bkg", "Miss")
+
+
+def _error_analysis(out, gt_hist, num_classes: int, method: str) -> Dict[str, Any]:
+    """``ErrorAnalysisAccumulator.compute``'s dict from one map compute over the ``TIDE_SETS * C``
+    classes of the record sets (``det_hist``, ``ap`` / ``voc``) plus the ``counts`` (C, 6)."""
+    C, F = num_classes, _lib.TIDE_SETS
+    ap_of = _DeviceSource(out, gt_hist, _lib.MAP_VIEW_CORNER).ap_table([None], "corner", method)
+    ap = np.array([[ap_of(f * C + c, 0) for c in range(C)] for f in range(F)], dtype=np.float64)
+    det, gt = out["det_hist"][_lib.MAP_VIEW_CORNER], gt_hist[_lib.MAP_VIEW_CORNER]
+    active = np.flatnonzero((det[:C] > 0) | (gt[:C] > 0))       # calculate_map's optimize_classes set
+    mean = lambda row: float(np.mean(row[active])) if len(active) else 0.0
+    base = mean(ap[0])
+    counts = np.asarray(out["counts"], dtype=np.int64)
+    return {"AP": base,
+            "dAP": {k: mean(ap[f + 1]) - base for f, k in enumerate(TIDE_FIXES)},
+            "counts": {k: int(counts[:, e].sum()) for e, k in enumerate(TIDE_ERRORS)},
+            "per_class": {"AP": ap[0], "dAP": (ap[1:] - ap[0]).T.copy(), "counts": counts}}
+
+
+class ErrorAnalysisAccumulator(MapAccumulator):
+    """TIDE-style detection error analysis (Bolya et al., ECCV 2020): what each kind of error costs
+    in AP, fed batch by batch with device tensors (``mgd_tide_update``).
+
+    The base is the reference's matcher at ``pos_threshold`` t_f (``iou_mode`` 'corner':
+    ``match_predictions_to_gt_cached``, 'centre': ``match_predictions_to_gt``, as in
+    ``ConfusionMatrixAccumulator``); every detection is used.  Each false positive d gets one type
+    from its best IoU ``s`` with the ground truth of its own class (claimed or not) and ``o`` with
+    that of the other classes, the first that applies: Bkg ``max(s, o) < background_threshold``;
+    Cls ``o >= t_f``; Dupe ``s >= t_f``; Loc ``s >= background_threshold``; Both otherwise.  A Miss is
+    a ground truth the base left unclaimed that no Cls or Loc error targets (the ground truth
+    attaining ``o`` or ``s``; equal IoU: the lowest index).
+
+    Each fix is applied alone to the base, and the AP of the fixed detections is ``calculate_map``'s
+    AP arithmetic at one threshold: Cls gives d its target's class and Loc keeps d's class, and in
+    the visiting order (score descending, equal scores later slot first) d then claims the target
+    as a TP if no one holds it yet, or is dropped; Both / Dupe / Bkg drop those detections; Miss
+    removes the missed ground truth; FP drops every false positive; FN leaves each class only its
+    claimed ground truth.  ``dAP[e]`` is the mean AP over classes with fix e minus the base mean,
+    both over the classes with detections or ground truth (``calculate_map``'s ``optimize_classes``
+    set); the base ``AP`` is ``MapAccumulator``'s mAP at ``iou_thresholds=[pos_threshold]`` with the
+    same matcher.  This is TIDE's definition with this project's matcher and AP arithmetic, with
+    no crowd or ignore regions and these tie rules, so the numbers are not ``tidecv``'s own (which
+    also uses 101-point AP).
+
+    ``update`` takes ``MapAccumulator.update``'s tensors (``det_boxes`` may be the int32
+    ``boxes_xyxy`` of ``engine.decode_nms``) and only enqueues work on the current stream; it keeps
+    ``TIDE_SETS`` (9) records of 40 bytes per padded detection slot.  Scores must be finite;
+    ``compute`` raises AssertionError for a class id outside [0, num_classes).  ``class_names``
+    label the rows of ``per_class`` for the caller; the dict does not use them.
+    """
+
+    def __init__(self, num_classes: int, pos_threshold: float = 0.5, background_threshold: float = 0.1,
+                 iou_mode: str = "corner", method: str = "coco", class_names: List[str] = None, device=None):
+        C, self.pos_threshold, self.background_threshold, _ = engine.tide_config(
+            num_classes, pos_threshold, background_threshold, iou_mode)
+        self.num_classes, self.iou_mode = C, iou_mode
+        self.class_names = [f"class_{i}" for i in range(C)] if class_names is None else list(class_names)
+        self._init_map(method, device)
+
+    def _init_map(self, method, device):
+        # the record sets are blocks of C classes of one map evaluation: one threshold, corner view
+        MapAccumulator.__init__(self, _lib.TIDE_SETS * self.num_classes, [self.pos_threshold], None, method,
+                                use_parallel=False, compute_per_scale=False, device=device)
+
+    def reset(self) -> None:
+        """Forget every update."""
+        import torch
+        super().reset()
+        self._counts = torch.zeros((self.num_classes, _lib.TIDE_ERRORS), dtype=torch.int64, device=self.device)
+
+    def update(self, det_boxes, det_scores, det_classes, det_counts, gt_boxes, gt_classes, gt_counts) -> None:
+        """Add one batch: det_boxes (B, M, 4) xyxy, det_scores (B, M), det_classes (B, M),
+        det_counts (B,), gt_boxes (B, N, 4) xyxy, gt_classes (B, N), gt_counts (B,)."""
+        slots = _lib.TIDE_SETS * int(det_scores.shape[0]) * int(det_scores.shape[1])
+        self._reserve(slots)
+        engine.tide_update(self._records, self._slots, self._gt_hist, self._counts, self.pos_threshold,
+                           self.background_threshold, self.iou_mode, det_boxes, det_scores, det_classes,
+                           det_counts, gt_boxes, gt_classes, gt_counts)
+        self._slots += slots
+
+    def compute(self) -> Dict[str, Any]:
+        """Over every update since construction or ``reset``:
+
+        - ``AP``: the base mAP at ``pos_threshold``;
+        - ``dAP``: ``{"Cls", "Loc", "Both", "Dupe", "Bkg", "Miss", "FP", "FN"}``, the rise of that
+          mAP when only that error is fixed;
+        - ``counts``: ``{"Cls", "Loc", "Both", "Dupe", "Bkg", "Miss"}``, the number of errors;
+        - ``per_class``: ``AP`` (C,) float64, ``dAP`` (C, 8) float64 in the order above, ``counts``
+          (C, 6) int64 (a false positive counts under its detection's class, a Miss under its
+          ground truth's).  A class's AP follows ``calculate_map``: 0.0 with ground truth but no
+          detections or detections but no ground truth, 1.0 with neither.
+        """
+        out, gt = self._tables()
+        return _error_analysis(out, gt, self.num_classes, self._args[3])
+
+    def _tables(self):
+        out = engine.map_compute(self._cfg, self._records, self._slots, self._gt_hist)
+        engine.poll_status(self.device.index or 0)
+        out["counts"] = self._counts.cpu().numpy()
+        return out, self._gt_hist.cpu().numpy()
+
+
+class ShardedErrorAnalysisAccumulator(ErrorAnalysisAccumulator, ShardedMapAccumulator):
+    """``ErrorAnalysisAccumulator`` over a batch sharded across the ranks of ``group``, with
+    ``ShardedMapAccumulator``'s machinery: ``update`` takes this rank's shard (as
+    ``ShardedMapAccumulator.update``, with ``n_total``) and makes no collective call; ``compute`` is
+    collective.  The record sets are exchanged and their APs computed class by class on the rank
+    that owns the class, and the error counts of each rank's images join the one all-reduce.  The
+    update sequences and class-range status of all ranks are compared first, so a class id out of
+    range raises AssertionError on every rank.  Every rank returns the same dict, equal to the
+    single-process one.  Without ``torch.distributed`` or at world size 1 it makes no collective
+    call."""
+
+    def __init__(self, num_classes: int, pos_threshold: float = 0.5, background_threshold: float = 0.1,
+                 iou_mode: str = "corner", method: str = "coco", class_names: List[str] = None, device=None,
+                 group=None):
+        self.group = group
+        super().__init__(num_classes, pos_threshold, background_threshold, iou_mode, method, class_names, device)
+
+    def _init_map(self, method, device):
+        ShardedMapAccumulator.__init__(self, _lib.TIDE_SETS * self.num_classes, [self.pos_threshold], None, method,
+                                       use_parallel=False, compute_per_scale=False, device=device, group=self.group)
+
+    def update(self, det_boxes, det_scores, det_classes, det_counts, gt_boxes, gt_classes, gt_counts,
+               n_total: int = None) -> None:
+        """Add this rank's shard of a global batch of ``n_total`` images (default: the local batch
+        times the world size), as ``ShardedMapAccumulator.update``."""
+        n_total = self._shard_total(int(det_scores.shape[0]), n_total)
+        super().update(det_boxes, det_scores, det_classes, det_counts, gt_boxes, gt_classes, gt_counts)
+        self._updates.append((n_total, _lib.TIDE_SETS * int(det_scores.shape[1])))
+
+    def _rank_counts(self):
+        return {"counts": self._counts}
+
+    def _tables(self):
+        out, gt, _ = self._merged_tables()
+        return out, gt
